@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — shielded agent-steps/s of the batched merge env + CBF shield on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--envs E] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--envs E] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one policy step (3 physics sub-steps, 3 shield solves per CAV, observation, rewards) of every env of
 the workload, with finished envs re-spawned on the device (auto-reset), under i.i.d. uniform meta-actions.
@@ -347,6 +347,35 @@ class Leg(object):
         self.env.close()
 
 
+# What env.step hands its caller (obs, reward, done and the info views), minus the actions it was given.
+DUMP_KEYS = ("obs", "reward", "done", "agents_rewards", "regional_rewards", "agents_dones", "average_speed", "traffic_speed",
+             "min_headway", "merge_percent", "n_agents", "action_mask", "new_actions")
+DUMP_BYTES = 64 * 10 ** 6      # all files of one dump together, .npy headers included
+NPY_HEADER_BYTES = 128         # numpy writes a 128-byte header for arrays of these ranks
+
+
+def dump_sample_size(env):
+    """How many envs a dump keeps: all of them, or as many as fit in DUMP_BYTES at float32 per output value plus the
+    float64 env index."""
+    v = env.buffers()
+    per_env = 8 + sum(4 * (v[k].numel() // env.n_envs) for k in DUMP_KEYS)
+    return min(env.n_envs, (DUMP_BYTES - NPY_HEADER_BYTES * (len(DUMP_KEYS) + 1)) // per_env)
+
+
+def dump_outputs(env, out_dir):
+    """Write the outputs of env's last step as out_dir/<key>.npy (float32) for the envs listed in out_dir/env_index.npy
+    (float64): every env when they fit in DUMP_BYTES, else a sample drawn with a fixed seed."""
+    import torch
+    E, n = env.n_envs, dump_sample_size(env)
+    idx = np.arange(E) if n == E else np.sort(np.random.RandomState(0).choice(E, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    sel = torch.from_numpy(idx).to("cuda:%d" % env.device)
+    v = env.buffers()
+    for k in DUMP_KEYS:
+        np.save(os.path.join(out_dir, k + ".npy"), v[k].index_select(0, sel).cpu().numpy().astype(np.float32))
+
+
 BUILD_NAMES = {3: "generic, 3 CTAs/SM", 4: "generic, 4 CTAs/SM", 31: "all-CAV HSS specialised, 3 CTAs/SM",
                32: "all-CAV MASS specialised, 3 CTAs/SM", 41: "all-CAV HSS specialised, 4 CTAs/SM",
                42: "all-CAV MASS specialised, 4 CTAs/SM", 50: "warp-cooperative, no shield", 51: "warp-cooperative, HSS",
@@ -371,7 +400,15 @@ def main():
     ap.add_argument("--policy", action="store_true",
                     help="BASELINE configs[3]: sample the actions from the MAPPO actor (30-128-128-5) on the device "
                          "inside the timed region instead of reading pre-drawn uniform actions")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0's envs, a "
+                         "seeded sample of them when all would exceed %d MB): the same arguments give the same inputs on "
+                         "every run, so two builds can be compared output for output" % (DUMP_BYTES // 10 ** 6))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     wl = dict(WORKLOADS[args.workload])
     if args.envs:
         wl["envs"] = args.envs
@@ -419,6 +456,8 @@ def main():
     env = leg.env
     sampler.start()
     ms_local, stats, launches = leg.timed(K, W, barrier)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)
     build = env.step_build()
     kms, _ = leg.kernel_times(min(K, 30))
     clocks = sampler.stop()
