@@ -47,7 +47,7 @@ enum { MM_ACT_LEAD = 1, MM_ACT_UPPER = 2, MM_ACT_LOWER = 4, MM_ACT_ADJ = 8, MM_A
  * signature; mm_abi_version() returns the value the library was built with, and mm_create / mm_set_config reject a
  * config whose struct_size field is not sizeof(mm_config) (a binding built against another revision of the header
  * fails loudly instead of handing the library garbage). */
-#define MM_ABI_VERSION 8
+#define MM_ABI_VERSION 9
 int mm_abi_version(void);
 
 typedef struct {
@@ -264,6 +264,44 @@ int mm_set_actor_impl(int impl);
  * [T][n_cols / cols_per_env] u8, DEVICE pointers. */
 int mm_discounted_returns(const float *rewards, const uint8_t *dones, const float *final_value, float gamma, int T,
                           int64_t n_cols, int cols_per_env, float *out, void *stream);
+
+/* On-device PPO learner: the networks of one MAPPO / MAPPO_GI update with the per-sample PPO-clip surrogate and the MSE
+ * value loss (marl/mappo.py:161-206, marl/mappo_gi.py:307-349; rollout.mappo_losses / shared_network_loss with
+ * pairwise=False, critic_loss="mse").  Network kinds, parameters as torch.nn.Linear lays them out (weight [out][in]):
+ *   MM_PPO_ACTOR   ActorNetwork 30-128-128-5, log-softmax: w1..b3 = fc1..fc3
+ *   MM_PPO_CRITIC  CriticNetwork: w1 / b1 = fc1 (30 -> 128), w2 / b2 = fc2 ([h1, one_hot(a)] 133 -> 128), w3 / b3 = fc3 (-> 1)
+ *   MM_PPO_SHARED  ActorCriticNetwork with state_split, hidden 128: w1 [160][30] / b1 [160] = fc11 / fc12 / fc13 as one dense
+ *                  layer, zero outside the blocks (as for mm_actor_sample_mlp), w2 / b2 = fc2, w3 / b3 = actor_linear,
+ *                  w4 [128] / b4 [1] = critic_linear
+ * w4 / b4 are used by MM_PPO_SHARED only.  Rows: states [rows][30] f32, actions [rows] int8 (0..4) and returns [rows] f32
+ * are the rollout buffer as collected; idx [n] int64 lists the rows of the pass in any order.  DEVICE pointers, enqueued on
+ * `stream`, no allocation after the first call on a device and no synchronisation.  Arguments are checked before any
+ * CUDA call (MM_ERR_ARG): kind, required pointers, n >= 1, 0 < clip < 1. */
+enum { MM_PPO_ACTOR = 0, MM_PPO_CRITIC = 1, MM_PPO_SHARED = 2 };
+typedef struct { const float *w1, *b1, *w2, *b2, *w3, *b3, *w4, *b4; } mm_ppo_net;
+typedef struct { float *w1, *b1, *w2, *b2, *w3, *b3, *w4, *b4; } mm_ppo_grads_out;
+
+/* Target pass (forward only), once per update with the TARGET networks: for every listed row, old_logp[row] = log p(a)
+ * (MM_PPO_ACTOR, MM_PPO_SHARED) or q_target[row] = Q(s, one_hot(a)) (MM_PPO_CRITIC); outputs are indexed like states.
+ * Replaces the no-grad half of MAPPO.train (mappo.py:170-183) and MAPPO_GI.train (mappo_gi.py:307-320), which torch
+ * recomputes for every minibatch. */
+int mm_ppo_targets(int kind, const float *states, const int8_t *actions, const int64_t *idx, int64_t n, const mm_ppo_net *net,
+                   float *old_logp, float *q_target, void *stream);
+
+/* Gradient pass, once per minibatch: the gradients of the mean loss over the n listed rows, written (not accumulated) into
+ * `grads` in the parameters' layout (MM_PPO_SHARED: w1 in the dense [160][30] layout), and the mean losses into losses[0]
+ * (PPO surrogate: MM_PPO_ACTOR, MM_PPO_SHARED) / losses[1] (value MSE: MM_PPO_CRITIC, MM_PPO_SHARED); the other slot is
+ * left as it is.  Advantage: returns - q_target (MM_PPO_ACTOR, q_target from the critic's target pass) or returns - V(s)
+ * (MM_PPO_SHARED, V detached).  old_logp from the target pass; ratio r = exp(log p(a) - old_logp), and since both passes
+ * run the same forward arithmetic r == 1 exactly while a network equals its target.  The per-row derivative follows
+ * torch autograd: min splits the gradient half / half at a tie, clamp passes it at its bounds.  Deterministic: each CTA
+ * sums its tiles, a second kernel adds the CTA partials in a fixed order (two calls with equal inputs give bit-identical
+ * gradients); the partials workspace is allocated once per device and shared by the calls on that device, which must
+ * therefore be ordered (one stream).  Replaces actor_loss.backward() / critic_loss.backward() of MAPPO.train and
+ * loss.backward() of MAPPO_GI.train. */
+int mm_ppo_grads(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                 const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
+                 const mm_ppo_grads_out *grads, float *losses, void *stream);
 
 /* The step kernel (the physics of a policy step) exists in several builds of one source: generic for 3 CTAs per SM
  * (6 staged fields, 168 registers; the faster one per unit of work), generic for 4 CTAs per SM (4 staged fields, 128

@@ -28,7 +28,7 @@ _PU8 = C.POINTER(C.c_uint8)
 _PI8 = C.POINTER(C.c_int8)
 
 
-ABI_VERSION = 8           # MM_ABI_VERSION of the header this binding was written against
+ABI_VERSION = 9           # MM_ABI_VERSION of the header this binding was written against
 
 
 class MMConfig(C.Structure):
@@ -77,6 +77,19 @@ class MMStats(C.Structure):
                                           "lane_change_vetoes", "min_headway")]
 
 
+class MMPpoNet(C.Structure):
+    """mm_ppo_net: parameter pointers of one network of the on-device PPO learner"""
+    _fields_ = [(k, C.c_void_p) for k in ("w1", "b1", "w2", "b2", "w3", "b3", "w4", "b4")]
+
+
+class MMPpoGrads(C.Structure):
+    """mm_ppo_grads_out: one gradient buffer per parameter, same layout"""
+    _fields_ = [(k, C.c_void_p) for k in ("w1", "b1", "w2", "b2", "w3", "b3", "w4", "b4")]
+
+
+PPO_ACTOR, PPO_CRITIC, PPO_SHARED = 0, 1, 2     # MM_PPO_ACTOR / _CRITIC / _SHARED
+
+
 class MMError(RuntimeError):
     pass
 
@@ -87,7 +100,7 @@ SUPERVISOR_DRAWS = 32     # MM_SUPERVISOR_DRAWS
 EXPORTS = ("mm_create", "mm_destroy", "mm_set_config", "mm_num_envs", "mm_reset", "mm_step", "mm_step_host",
            "mm_step_host_ragged", "mm_step_host_packed", "mm_expand_obs_rows",
            "mm_buffers_get", "mm_get_state", "mm_set_state", "mm_get_shield_diag", "mm_stats", "mm_shield_qp", "mm_shield_query",
-           "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
+           "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
            "mm_kernel_launches", "mm_last_error", "mm_version")
 
 
@@ -131,6 +144,10 @@ def lib():
     L.mm_step_build.argtypes = [h]
     L.mm_discounted_returns.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int, C.c_int64, C.c_int,
                                         C.c_void_p, C.c_void_p]
+    L.mm_ppo_targets.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(MMPpoNet), C.c_void_p,
+                                 C.c_void_p, C.c_void_p]
+    L.mm_ppo_grads.argtypes = [C.c_int] + [C.c_void_p] * 6 + [C.c_int64, C.c_float, C.POINTER(MMPpoNet), C.POINTER(MMPpoGrads),
+                                                             C.c_void_p, C.c_void_p]
     L.mm_kernel_launches.argtypes = [h]
     L.mm_kernel_launches.restype = C.c_int64
     L.mm_last_error.restype = C.c_char_p

@@ -932,4 +932,42 @@ int mm_discounted_returns(const float *rewards, const uint8_t *dones, const floa
     return 0;
 }
 
+static int check_ppo_net(int kind, const mm_ppo_net *net) {
+    if (kind != MM_PPO_ACTOR && kind != MM_PPO_CRITIC && kind != MM_PPO_SHARED)
+        return fail(MM_ERR_ARG, "kind must be 0 (MAPPO actor), 1 (MAPPO critic) or 2 (MAPPO_GI shared network)");
+    if (!net || !net->w1 || !net->b1 || !net->w2 || !net->b2 || !net->w3 || !net->b3)
+        return fail(MM_ERR_ARG, "net: w1, b1, w2, b2, w3 and b3 are required");
+    if (kind == MM_PPO_SHARED && (!net->w4 || !net->b4)) return fail(MM_ERR_ARG, "net: the shared network needs w4 and b4 (critic_linear)");
+    return 0;
+}
+
+int mm_ppo_targets(int kind, const float *states, const int8_t *actions, const int64_t *idx, int64_t n, const mm_ppo_net *net,
+                   float *old_logp, float *q_target, void *stream) {
+    if (int rc = check_ppo_net(kind, net)) return rc;
+    if (!states || !actions || !idx) return fail(MM_ERR_ARG, "states, actions and idx are required");
+    if (kind == MM_PPO_CRITIC ? !q_target : !old_logp)
+        return fail(MM_ERR_ARG, kind == MM_PPO_CRITIC ? "the critic's target pass writes q_target" : "the target pass writes old_logp");
+    if (n < 1) return fail(MM_ERR_ARG, "n must be >= 1");
+    if (launch_ppo_targets(kind, states, actions, idx, n, net, old_logp, q_target, stream))
+        return fail(MM_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
+    return 0;
+}
+
+int mm_ppo_grads(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                 const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
+                 const mm_ppo_grads_out *grads, float *losses, void *stream) {
+    if (int rc = check_ppo_net(kind, net)) return rc;
+    if (!states || !actions || !returns || !idx || !grads || !losses) return fail(MM_ERR_ARG, "states, actions, returns, idx, grads and losses are required");
+    if (!grads->w1 || !grads->b1 || !grads->w2 || !grads->b2 || !grads->w3 || !grads->b3 ||
+        (kind == MM_PPO_SHARED && (!grads->w4 || !grads->b4)))
+        return fail(MM_ERR_ARG, "grads: one output buffer per parameter is required");
+    if (kind != MM_PPO_CRITIC && !old_logp) return fail(MM_ERR_ARG, "old_logp (from the target pass) is required");
+    if (kind == MM_PPO_ACTOR && !q_target) return fail(MM_ERR_ARG, "q_target (from the critic's target pass) is required");
+    if (n < 1) return fail(MM_ERR_ARG, "n must be >= 1");
+    if (!(clip > 0.f && clip < 1.f)) return fail(MM_ERR_ARG, "clip must be in (0, 1)");
+    if (launch_ppo_grads(kind, states, actions, returns, old_logp, q_target, idx, n, clip, net, grads, losses, stream))
+        return fail(MM_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
+    return 0;
+}
+
 }  // extern "C"

@@ -158,6 +158,13 @@ int launch_actor_mlp(const float *obs, const int32_t *n_agents, int64_t n_rows, 
 int launch_discounted_returns(const float *rewards, const uint8_t *dones, const float *final_value, float gamma, int T,
                               int64_t n_cols, int cols_per_env, float *out, void *stream);
 
+// on-device PPO learner (learner.cu); arguments already checked by the C ABI
+int launch_ppo_targets(int kind, const float *states, const int8_t *actions, const int64_t *idx, int64_t n, const mm_ppo_net *net,
+                       float *old_logp, float *q_target, void *stream);
+int launch_ppo_grads(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                     const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
+                     const mm_ppo_grads_out *grads, float *losses, void *stream);
+
 // envs [env_offset, env_offset + env_count); draws null: Philox draws keyed (seed, env, episode, step); n_used_out
 // (nullable) [n_envs]: how many draws each env's supervisor consumed
 void launch_supervisor(const DevState &st, int env_offset, int env_count, int kind, int8_t *actions, const double *draws,

@@ -9,8 +9,9 @@ Kept from the reference: the networks (marl/single_agent/Model_common.py:5-40: a
 critic on (state, one-hot action)), reward selection `regionalR | global_R` (mappo.py:122-125), reward scaling,
 the discounted return (`_discount_reward`, mappo.py:364-370, final value 0 at episode end, critic bootstrap
 otherwise) and the PPO-clip / critic losses of `MAPPO.train` (mappo.py:161-206) — batched over every live
-(env, agent, t) sample instead of looped per agent.  The learner itself stays out of scope for the hot-path work;
-this module is the caller that lets BASELINE configs[3] (policy + env on device) be measured.
+(env, agent, t) sample instead of looped per agent.  The update runs as torch autograd (the default, and the numerics
+reference) or, with `update(impl="cuda")`, through the learner kernels (mm_ppo_targets / mm_ppo_grads): one target
+pass per update and one fused forward + backward per minibatch.
 """
 import ctypes as C
 
@@ -270,6 +271,127 @@ def actor_sample(actor, obs, n_agents=None, seed=0, step=0, want_logp=False, act
     return (actions, logp) if want_logp else actions
 
 
+# ---- on-device PPO learner (mm_ppo_targets / mm_ppo_grads): the update of `mappo_losses` / `shared_network_loss`
+# (pairwise=False, critic_loss="mse") without autograd
+
+def _ppo_kind(net):
+    """-> (kind, parameters in mm_ppo_net order); asserts the reference's hidden sizes, which the kernels are built for."""
+    if isinstance(net, ActorCriticNetwork):
+        assert net.state_split and net.fc2.in_features == 160 and net.fc2.out_features == 128, \
+            "the learner kernels cover the reference's shared network (hidden size 128, state_split)"
+        w1, b1 = _split_first_layer(net)
+        return _lib.PPO_SHARED, [w1, b1, net.fc2.weight, net.fc2.bias, net.actor_linear.weight, net.actor_linear.bias,
+                                 net.critic_linear.weight, net.critic_linear.bias]
+    shapes = [tuple(net.fc1.weight.shape), tuple(net.fc2.weight.shape), tuple(net.fc3.weight.shape)]
+    if shapes == [(128, NS), (128, 128), (NA, 128)]:
+        kind = _lib.PPO_ACTOR
+    elif shapes == [(128, NS), (128, 128 + NA), (1, 128)]:
+        kind = _lib.PPO_CRITIC
+    else:
+        raise AssertionError("the learner kernels cover the reference's ActorNetwork / CriticNetwork (hidden size 128)")
+    return kind, [net.fc1.weight, net.fc1.bias, net.fc2.weight, net.fc2.bias, net.fc3.weight, net.fc3.bias]
+
+
+def _ppo_net(params):
+    for p in params:
+        assert p.is_cuda and p.dtype == torch.float32 and p.is_contiguous()
+    ptrs = [p.data_ptr() for p in params] + [0] * (8 - len(params))
+    return _lib.MMPpoNet(*ptrs)
+
+
+def _check_rows(S, A8, idx, G=None):
+    rows = S.shape[0]
+    assert S.is_cuda and S.dtype == torch.float32 and S.is_contiguous() and S.dim() == 2 and S.shape[1] == NS
+    assert A8.dtype == torch.int8 and A8.is_contiguous() and A8.numel() == rows
+    assert idx.dtype == torch.int64 and idx.is_contiguous() and idx.dim() == 1 and idx.is_cuda
+    if G is not None:
+        assert G.dtype == torch.float32 and G.is_contiguous() and G.numel() == rows
+    return rows
+
+
+@torch.no_grad()
+def ppo_targets(net, S, A8, idx, out=None):
+    """Target pass of one update (mm_ppo_targets): for the rows listed in idx, the target log-probability of the taken
+    action (`net` an ActorNetwork or the shared ActorCriticNetwork) or Q_target(s, one_hot(a)) (`net` a CriticNetwork).
+    S [rows, 30] f32, A8 [rows] int8 (the rollout buffer as collected), idx int64 [n]; -> out [rows] f32, indexed like
+    S (rows not listed are left as they are)."""
+    rows = _check_rows(S, A8, idx)
+    kind, params = _ppo_kind(net)
+    out = torch.empty(rows, dtype=torch.float32, device=S.device) if out is None else out
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == rows
+    if idx.numel() == 0:
+        return out
+    crit = kind == _lib.PPO_CRITIC
+    _lib.check(_lib.lib().mm_ppo_targets(kind, _ptr(S), _ptr(A8), _ptr(idx), C.c_int64(idx.numel()), C.byref(_ppo_net(params)),
+                                         _ptr(None if crit else out), _ptr(out if crit else None), _stream()))
+    return out
+
+
+def _grad_buffer(p):
+    """p.grad, created if absent; the kernels overwrite it (as backward() after zero_grad(set_to_none=True) would)."""
+    if p.grad is None:
+        p.grad = torch.empty_like(p)
+    return p.grad
+
+
+def _ppo_grads(kind, params, grads, S, A8, G, old_logp, q_target, idx, clip, losses):
+    if idx.numel() == 0:       # an empty shard of a data-parallel update: it contributes nothing to the all-reduce
+        for g in grads:
+            g.zero_()
+        return
+    out = _lib.MMPpoGrads(*([g.data_ptr() for g in grads] + [0] * (8 - len(grads))))
+    _lib.check(_lib.lib().mm_ppo_grads(kind, _ptr(S), _ptr(A8), _ptr(G), _ptr(old_logp), _ptr(q_target), _ptr(idx),
+                                       C.c_int64(idx.numel()), C.c_float(clip), C.byref(_ppo_net(params)), C.byref(out),
+                                       _ptr(losses), _stream()))
+
+
+def mappo_gradients(actor, critic, S, A8, G, old_logp, q_target, idx, clip=0.2, losses=None):
+    """Gradient pass of one MAPPO minibatch (mm_ppo_grads, actor and critic): writes every parameter's .grad as
+    `actor_loss.backward(); critic_loss.backward()` of `mappo_losses` (pairwise=False, critic_loss="mse") would after
+    zero_grad(set_to_none=True), with old_logp / q_target from `ppo_targets` of actor_target / critic_target.  S [rows, 30],
+    A8 [rows] int8, G [rows] f32 (the returns), idx int64 [n] the minibatch's rows in any order.  losses (optional) f32 [2]
+    device buffer.  -> (actor_loss, critic_loss) device scalars, no host synchronisation."""
+    _check_rows(S, A8, idx, G)
+    ka, pa = _ppo_kind(actor)
+    kc, pc = _ppo_kind(critic)
+    assert ka == _lib.PPO_ACTOR and kc == _lib.PPO_CRITIC
+    losses = torch.zeros(2, dtype=torch.float32, device=S.device) if losses is None else losses
+    assert old_logp.numel() == S.shape[0] and q_target.numel() == S.shape[0]
+    _ppo_grads(ka, pa, [_grad_buffer(p) for p in pa], S, A8, G, old_logp, q_target, idx, clip, losses)
+    _ppo_grads(kc, pc, [_grad_buffer(p) for p in pc], S, A8, G, None, None, idx, clip, losses)
+    return losses[0], losses[1]
+
+
+_FOLD_CACHE = {}
+
+
+def shared_network_gradients(policy, S, A8, G, old_logp, idx, clip=0.2, losses=None):
+    """Gradient pass of one MAPPO_GI minibatch (mm_ppo_grads, shared network): writes every parameter's .grad as
+    `loss.backward()` of `shared_network_loss` (pairwise=False, critic_loss="mse") would after zero_grad(set_to_none=True).
+    The kernel differentiates the dense 30 -> 160 first layer; fc11 / fc12 / fc13 receive their own blocks of it.
+    -> (loss, actor_loss, critic_loss) device scalars, no host synchronisation."""
+    _check_rows(S, A8, idx, G)
+    kind, params = _ppo_kind(policy)
+    assert old_logp.numel() == S.shape[0]
+    losses = torch.zeros(2, dtype=torch.float32, device=S.device) if losses is None else losses
+    dev = S.device
+    hit = _FOLD_CACHE.get(id(policy))
+    if hit is None or hit[0].device != dev:
+        dense = (torch.empty((160, NS), device=dev), torch.empty(160, device=dev))
+        cols = [torch.tensor(c, device=dev) for c in (policy.COLS1, policy.COLS2, policy.COLS3)]
+        hit = _FOLD_CACHE[id(policy)] = dense + (cols,)
+    gw1, gb1, cols = hit
+    grads = [gw1, gb1] + [_grad_buffer(p) for p in params[2:]]
+    _ppo_grads(kind, params, grads, S, A8, G, old_logp, None, idx, clip, losses)
+    o = 0
+    for lin, c in zip((policy.fc11, policy.fc12, policy.fc13), cols):
+        k = lin.out_features
+        torch.index_select(gw1[o:o + k], 1, c, out=_grad_buffer(lin.weight))
+        _grad_buffer(lin.bias).copy_(gb1[o:o + k])
+        o += k
+    return losses[0] + losses[1], losses[0], losses[1]
+
+
 def _check_record_slots(rows, obs_copy, live_out):
     if obs_copy is not None:
         assert obs_copy.is_cuda and obs_copy.dtype == torch.float32 and obs_copy.is_contiguous() and obs_copy.numel() == rows * NS
@@ -410,10 +532,14 @@ class BatchedMAPPORollout(object):
             q.grad.copy_(flat[o:o + q.numel()].view_as(q.grad))
             o += q.numel()
 
-    def update(self, minibatch=1 << 18, epochs=1):
+    def update(self, minibatch=1 << 18, epochs=1, impl="torch"):
         """PPO-clip actor update and critic regression on the last rollout (mappo.py:161-206, `mappo_losses`), all
         agents at once, with the per-sample surrogate (the reference's [N] x [N, 1] product is an N x N table).
-        Under torch.distributed every rank runs the same number of minibatches and the gradients are averaged."""
+        Under torch.distributed every rank runs the same number of minibatches and the gradients are averaged.
+        impl: "torch" (autograd) or "cuda" (the learner kernels: `_update_cuda`)."""
+        if impl == "cuda":
+            return self._update_cuda(minibatch, epochs)
+        assert impl == "torch", impl
         b = self.buf
         live = b["live"].reshape(-1)
         idx = live.nonzero(as_tuple=False).squeeze(1)
@@ -446,6 +572,47 @@ class BatchedMAPPORollout(object):
         self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
         self.critic_target.load_state_dict(self.critic.state_dict())
         return stats
+
+    def _learner_batch(self):
+        """(live row list, states [rows, 30], actions int8 [rows], returns [rows], minibatch count) of the last rollout"""
+        b = self.buf
+        idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
+        S = b["states"].reshape(-1, NS)
+        A8 = b["actions"].reshape(-1).to(torch.int8)
+        G = b["returns"].reshape(-1).contiguous()
+        return idx, S, A8, G
+
+    def _minibatch_count(self, idx, minibatch):
+        n_max = torch.tensor([idx.numel()], device=self.dev)
+        if self._world() > 1:
+            import torch.distributed as dist
+            dist.all_reduce(n_max, op=dist.ReduceOp.MAX)
+        return max(1, -(-int(n_max) // int(minibatch)))       # same count on every rank
+
+    def _update_cuda(self, minibatch, epochs):
+        """`update` with the learner kernels: one target pass (old log-probabilities and Q_target of every live sample,
+        the target networks do not change within an update), then per minibatch one gradient pass (mappo_gradients) in
+        place of the two backward passes; all-reduce, gradient clipping and the RMSprop steps are the torch path's.  The
+        losses stay on the device until the one read at the end."""
+        idx, S, A8, G = self._learner_batch()
+        n_mb = self._minibatch_count(idx, minibatch)
+        old_logp = ppo_targets(self.actor_target, S, A8, idx)
+        q_target = ppo_targets(self.critic_target, S, A8, idx)
+        losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
+        for _ in range(epochs):
+            perm = idx[torch.randperm(idx.numel(), device=self.dev)]
+            for j in torch.tensor_split(perm, n_mb):
+                mappo_gradients(self.actor, self.critic, S, A8, G, old_logp, q_target, j, self.clip_param, losses=losses)
+                self._allreduce_grads(list(self.actor.parameters()))
+                nn.utils.clip_grad_norm_(self.actor.parameters(), self.max_grad_norm)
+                self.actor_opt.step()
+                self._allreduce_grads(list(self.critic.parameters()))
+                nn.utils.clip_grad_norm_(self.critic.parameters(), self.max_grad_norm)
+                self.critic_opt.step()
+        a_loss, c_loss = losses.tolist()
+        self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
+        self.critic_target.load_state_dict(self.critic.state_dict())
+        return {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
 
 
 class BatchedMAPPOGIRollout(BatchedMAPPORollout):
@@ -503,9 +670,13 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
             return policy_sample(self.policy, obs.contiguous(), n_agents, seed=seed, step=step)
         return self.act_torch(obs, n_agents)[0]
 
-    def update(self, minibatch=1 << 18, epochs=1):
+    def update(self, minibatch=1 << 18, epochs=1, impl="torch"):
         """One pass of `MAPPO_GI.train` (shared branch, mappo_gi.py:307-349) over the last rollout, all agents at once;
-        under torch.distributed the gradients are averaged over the ranks."""
+        under torch.distributed the gradients are averaged over the ranks.  impl: "torch" (autograd) or "cuda" (the
+        learner kernels)."""
+        if impl == "cuda":
+            return self._update_cuda(minibatch, epochs)
+        assert impl == "torch", impl
         b = self.buf
         idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
         S = b["states"].reshape(-1, NS)
@@ -531,3 +702,22 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
                          "samples": int(idx.numel())}
         self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
         return stats
+
+    def _update_cuda(self, minibatch, epochs):
+        """`update` with the learner kernels: one target pass, one gradient pass per minibatch
+        (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step."""
+        idx, S, A8, G = self._learner_batch()
+        n_mb = self._minibatch_count(idx, minibatch)
+        old_logp = ppo_targets(self.policy_target, S, A8, idx)
+        losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
+        params = list(self.policy.parameters())
+        for _ in range(epochs):
+            perm = idx[torch.randperm(idx.numel(), device=self.dev)]
+            for j in torch.tensor_split(perm, n_mb):
+                shared_network_gradients(self.policy, S, A8, G, old_logp, j, self.clip_param, losses=losses)
+                self._allreduce_grads(params)
+                nn.utils.clip_grad_norm_(params, self.max_grad_norm)
+                self.policy_opt.step()
+        a_loss, c_loss = losses.tolist()
+        self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
+        return {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}

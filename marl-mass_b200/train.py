@@ -50,7 +50,8 @@ def load_ini(path):
     return env_cfg, rollout_kw, train
 
 
-def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print):
+def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch"):
+    """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`)."""
     import torch
     from . import evaluation as ev
     from .env import DEFAULT_CONFIG, MergeEnvBatched
@@ -96,7 +97,7 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
         pol.collect()
         torch.cuda.synchronize(device)
         t1 = time.perf_counter()
-        up = pol.update(minibatch=minibatch)
+        up = pol.update(minibatch=minibatch, impl=update_impl)
         torch.cuda.synchronize(device)
         t2 = time.perf_counter()
         s = mmd.all_reduce_stats(env.stats())
@@ -131,8 +132,10 @@ def main():
     ap.add_argument("--iterations", type=int, default=30)
     ap.add_argument("--eval-interval", type=int, default=10)
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--update-impl", choices=("torch", "cuda"), default="torch",
+                    help="PPO update: torch autograd or the on-device learner kernels")
     a = ap.parse_args()
-    train(a.config, a.envs, a.iterations, a.device, a.eval_interval)
+    train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl)
 
 
 if __name__ == "__main__":
