@@ -254,8 +254,7 @@ int mm_actor_sample_mlp(const float *obs, const int32_t *n_agents, int64_t n_row
 
 /* Implementation switch of mm_actor_sample (process-wide): 0 = tcgen05 with fp16 operands, one warpgroup per 128-row
  * tile and the weights once per SM (default, the kernel of mm_actor_sample_mlp); 1 = the warp-level mma.sync TF32 kernel
- * kept as an independent cross-check; 2 = the first tcgen05 kernel (TF32 operands, one CTA per SM); 3 = tcgen05 with
- * fp16 operands, two CTAs per SM (also reachable through mm_actor_sample_mlp while selected). */
+ * kept as an independent cross-check.  Any other value: MM_ERR_ARG, the switch unchanged. */
 int mm_set_actor_impl(int impl);
 
 /* mm_discounted_returns: MAPPO._discount_reward (marl/mappo.py:364-370) for every (env, agent) column of a rollout at

@@ -5,23 +5,23 @@
 // actor once per agent per step on the CPU; the batched rollout (BASELINE configs[3]) evaluates it for every
 // (env, agent) row of the observation buffer the step kernel has just written, 786 432 rows at 65 536 envs.  As three
 // torch Linear layers that is 1.7 ms per step against 0.9 ms for the env step itself (profiles/README.md): the hidden
-// activations (2 x 400 MB) go through HBM four times.  Here a warp carries 16 rows through all three layers in
-// registers and only the observations (120 B / row) and the actions (1 B / row) touch HBM.
+// activations (2 x 400 MB) go through HBM four times.  Here all three layers stay on chip and only the observations
+// (120 B / row) and the actions (1 B / row) touch HBM.
 //
-// Two implementations, same arithmetic (TF32 operands, fp32 accumulation):
-//   * actor_sample_tcgen05_kernel (default): the two 128-wide layers as tcgen05.mma kind::tf32 with the accumulators in
-//     TMEM, 128 rows per tile, epilogues in the thread that owns the row - see the section further down;
-//   * actor_sample_kernel (mm_set_actor_impl(1)): mma.sync.m16n8k8 per warp, kept as the independent cross-check.  The
-//     accumulator fragment of layer L (thread holds rows g, g+8 and columns 2t, 2t+1 of each 8-wide tile) is reused
+// Two implementations of the same network and draw:
+//   * actor_mlp_wg_kernel<H1> (default; the only kernel of mm_actor_sample_mlp): all three layers as tcgen05.mma with
+//     fp16 operands and the accumulators in TMEM, one warpgroup per 128-row tile - see the section further down;
+//   * actor_sample_kernel (mm_set_actor_impl(1)): TF32 mma.sync.m16n8k8 per warp, kept as the independent cross-check.
+//     The accumulator fragment of layer L (thread holds rows g, g+8 and columns 2t, 2t+1 of each 8-wide tile) is reused
 //     directly as the A fragment of layer L+1 (rows g, g+8, columns t, t+4) by permuting the K index of that layer:
 //     A column t <-> hidden unit 8kk+2t, A column t+4 <-> 8kk+2t+1, and the weights are laid out in shared memory in
 //     fragment order with the same permutation, so no shuffle or shared-memory round trip separates the layers.
-// Measured at 786 432 rows: torch layers 1.89 ms, mma.sync 0.20 ms, tcgen05 0.17 ms (profiles/README.md); this op is
-// ~33 GFLOP per step, so both are bound by their epilogues and staging, not by the tensor pipe.
+// Measured at 786 432 rows on a B200: torch layers 1.89 ms, mma.sync 0.204 ms, tcgen05 warpgroup kernel 0.067 ms
+// (profiles/README.md); this op is ~33 GFLOP per step, so both are bound by their epilogues and staging, not by the
+// tensor pipe.
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <cstdlib>
 #include "mm_internal.h"
 
 namespace mm {
@@ -229,61 +229,19 @@ actor_sample_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
 }
 
 // ------------------------------------------------------------------------------------------------
-// tcgen05 version: the two 128-wide layers on the 5th-generation tensor cores
+// tcgen05 helpers
 // ------------------------------------------------------------------------------------------------
-// One persistent CTA per SM, 512 threads, 128 observation rows per tile (= the 128 TMEM lanes).
-//   layer 1   D1[128x128] = A1[128x32]  * W1^T   4 x tcgen05.mma kind::tf32 (M128 N128 K8), accumulator in TMEM cols 0..127
-//   epilogue  TMEM -> registers (tcgen05.ld 32x32b), + bias, ReLU, TF32 rounding -> A2 in shared memory
-//   layer 2   D2[128x128] = A2[128x128] * W2^T  16 x tcgen05.mma, accumulator in TMEM cols 128..255
-//   epilogue  TMEM -> registers, + bias, ReLU, and the 128 -> 5 output layer as FMAs in the thread that owns the row
-//             (too narrow for an MMA tile), log-softmax, inverse-CDF draw, one action byte per row
-// Operands are K-major, no swizzle: 16-byte rows of 4 TF32 values, core matrices of 8 rows; with the layout
-// [k-chunk][row] (float4) a warp's 32 rows of one chunk are 512 contiguous bytes (conflict-free staging), the stride
-// between 8-row groups is SBO = 128 B and between the two 16-byte k-chunks of one MMA LBO = 2048 B.
-// Warps w, w+4, w+8, w+12 share TMEM lane quarter w%4 (hardware rule) and split the 128 columns four ways; the next
-// tile's observations are requested right after a tile's first MMA is issued, so their latency hides behind the epilogues.
-constexpr int T5_THREADS = 512;
-constexpr int T5_CSPLIT = T5_THREADS / 128;                  // column groups (of 128 / T5_CSPLIT columns) per row
-constexpr int T5_COLS = 128 / T5_CSPLIT;
-constexpr int T5_ROWS = 128;
-constexpr uint32_t T5_CHUNK_BYTES = T5_ROWS * 16;            // one k-chunk (4 values) of all 128 rows
-// shared memory (bytes)
-constexpr uint32_t T5_A1 = 0;                                // [8 chunks][128] float4
-constexpr uint32_t T5_W1 = T5_A1 + 8 * T5_CHUNK_BYTES;       // [8 chunks][128] float4
-constexpr uint32_t T5_A2 = T5_W1 + 8 * T5_CHUNK_BYTES;       // [32 chunks][128] float4
-constexpr uint32_t T5_W2 = T5_A2 + 32 * T5_CHUNK_BYTES;      // [32 chunks][128] float4
-constexpr uint32_t T5_W3 = T5_W2 + 32 * T5_CHUNK_BYTES;      // [128 hidden][8] f32 (5 used)
-constexpr uint32_t T5_B1 = T5_W3 + AC_HID * 8 * 4;
-constexpr uint32_t T5_B2 = T5_B1 + AC_HID * 4;
-constexpr uint32_t T5_B3 = T5_B2 + AC_HID * 4;
-constexpr uint32_t T5_PART = T5_B3 + 8 * 4;                  // [column groups 1..][128 rows][8] f32 partial logits
-constexpr uint32_t T5_BAR = T5_PART + (T5_CSPLIT - 1) * T5_ROWS * 8 * 4;   // 2 mbarriers + the TMEM base address
-constexpr uint32_t T5_SMEM = T5_BAR + 32;
-
-__device__ __forceinline__ uint32_t t5_smem(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ uint64_t t5_desc(uint32_t smem_addr) {
-    // K-major, SWIZZLE_NONE: start address, LBO (between the two k-chunks of an MMA), SBO (between 8-row groups), version 1
-    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | ((uint64_t)(T5_CHUNK_BYTES >> 4) << 16) | ((uint64_t)(128u >> 4) << 32) |
-           (1ull << 46);
-}
-// kind::tf32, F32 accumulate, M = 128, N = 128, A and B K-major (cute/arch/mma_sm100_desc.hpp InstrDescriptor)
-constexpr uint32_t T5_IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-
-__device__ __forceinline__ void t5_mma(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, {%5, %5, %5, %5}, p;\n\t}"
-                 ::"r"(tmem_d), "l"(a_desc), "l"(b_desc), "r"(T5_IDESC), "r"(accumulate), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void t5_commit(uint32_t bar) {
+__device__ __forceinline__ uint32_t tc_smem(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void tc_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void t5_wait(uint32_t bar, uint32_t parity) {
+__device__ __forceinline__ void tc_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0;
     while (!done)
         asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
                      : "=r"(done) : "r"(bar), "r"(parity) : "memory");
 }
-__device__ __forceinline__ void t5_ld32(uint32_t taddr, uint32_t (&v)[32]) {
+__device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
                  "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, %21, %22, "
                  "%23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
@@ -294,247 +252,16 @@ __device__ __forceinline__ void t5_ld32(uint32_t taddr, uint32_t (&v)[32]) {
                  : "r"(taddr) : "memory");
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
-
-__global__ void __launch_bounds__(T5_THREADS, 1)
-actor_sample_tcgen05_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n_agents, int64_t n_rows,
-                            const float *__restrict__ w1, const float *__restrict__ b1, const float *__restrict__ w2,
-                            const float *__restrict__ b2, const float *__restrict__ w3, const float *__restrict__ b3,
-                            uint64_t seed, uint64_t step, const uint8_t *__restrict__ mask_bits,
-                            int8_t *__restrict__ actions, float *__restrict__ logp_all, float *__restrict__ logp_sel) {
-    extern __shared__ __align__(128) uint8_t t5_sm[];
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    float4 *a1 = reinterpret_cast<float4 *>(t5_sm + T5_A1), *w1f = reinterpret_cast<float4 *>(t5_sm + T5_W1);
-    float4 *a2 = reinterpret_cast<float4 *>(t5_sm + T5_A2), *w2f = reinterpret_cast<float4 *>(t5_sm + T5_W2);
-    float *w3s = reinterpret_cast<float *>(t5_sm + T5_W3), *b1s = reinterpret_cast<float *>(t5_sm + T5_B1);
-    float *b2s = reinterpret_cast<float *>(t5_sm + T5_B2), *b3s = reinterpret_cast<float *>(t5_sm + T5_B3);
-    float *part = reinterpret_cast<float *>(t5_sm + T5_PART);
-    uint64_t *bars = reinterpret_cast<uint64_t *>(t5_sm + T5_BAR);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(t5_sm + T5_BAR + 16);
-    const uint32_t bar1 = t5_smem(bars), bar2 = t5_smem(bars + 1);
-
-    // ---- one-time setup: weights in operand layout (TF32-rounded), barriers, TMEM ----
-    auto tf = [](float x) { return __uint_as_float(to_tf32(x)); };
-    for (int idx = tid; idx < 8 * T5_ROWS; idx += T5_THREADS) {          // W1: [out n][in k], k padded 30 -> 32
-        const int c = idx / T5_ROWS, n = idx % T5_ROWS, k = 4 * c;
-        float4 v;
-        v.x = tf(k + 0 < AC_IN ? w1[n * AC_IN + k + 0] : 0.f); v.y = tf(k + 1 < AC_IN ? w1[n * AC_IN + k + 1] : 0.f);
-        v.z = tf(k + 2 < AC_IN ? w1[n * AC_IN + k + 2] : 0.f); v.w = tf(k + 3 < AC_IN ? w1[n * AC_IN + k + 3] : 0.f);
-        w1f[idx] = v;
-    }
-    for (int idx = tid; idx < 32 * T5_ROWS; idx += T5_THREADS) {
-        const int c = idx / T5_ROWS, n = idx % T5_ROWS;
-        const float4 v = *reinterpret_cast<const float4 *>(w2 + n * AC_HID + 4 * c);
-        w2f[idx] = make_float4(tf(v.x), tf(v.y), tf(v.z), tf(v.w));
-    }
-    for (int idx = tid; idx < AC_HID * 8; idx += T5_THREADS) {
-        const int h = idx >> 3, k = idx & 7;
-        w3s[idx] = k < AC_OUT ? w3[k * AC_HID + h] : 0.f;
-    }
-    for (int idx = tid; idx < AC_HID; idx += T5_THREADS) { b1s[idx] = b1[idx]; b2s[idx] = b2[idx]; }
-    if (tid < 8) b3s[tid] = tid < AC_OUT ? b3[tid] : 0.f;
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar1));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar2));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(t5_smem(tmem_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
-    const uint32_t a1_addr = t5_smem(a1), w1_addr = t5_smem(w1f), a2_addr = t5_smem(a2), w2_addr = t5_smem(w2f);
-
-    const int row_in_tile = 32 * (warp & 3) + lane;        // TMEM lane = row of the tile this thread reads
-    const int cgrp = warp >> 2;                            // which T5_COLS of the 128 columns
-    const int col0 = T5_COLS * cgrp;
-    static_assert(T5_COLS == 32, "one tcgen05.ld.32x32b.x32 per thread and epilogue");
-    const uint32_t t_lane = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
-    const int64_t n_tiles = (n_rows + T5_ROWS - 1) / T5_ROWS;
-    // observation staging: thread t handles row t % 128, k-chunks 2 * (t / 128) and + 1
-    const int st_r = tid & (T5_ROWS - 1), st_c0 = 2 * (tid >> 7);
-    float4 pre[2];
-    auto fetch = [&](int64_t tile) {
-        const int64_t row = tile * T5_ROWS + st_r;
-        const float2 *src = reinterpret_cast<const float2 *>(obs + row * AC_IN);   // rows are 120 B: 8-byte aligned
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-            const int c = st_c0 + q;
-            float2 lo = make_float2(0.f, 0.f), hi = lo;
-            if (tile < n_tiles && row < n_rows) {
-                lo = __ldg(src + 2 * c);
-                if (4 * c + 2 < AC_IN) hi = __ldg(src + 2 * c + 1);
-            }
-            pre[q] = make_float4(lo.x, lo.y, hi.x, hi.y);
-        }
-    };
-    fetch(blockIdx.x);
-    uint32_t parity = 0;
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, parity ^= 1) {
-#pragma unroll
-        for (int q = 0; q < 2; ++q)
-            a1[(st_c0 + q) * T5_ROWS + st_r] = make_float4(tf(pre[q].x), tf(pre[q].y), tf(pre[q].z), tf(pre[q].w));
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-                t5_mma(tmem, t5_desc(a1_addr + j * 2 * T5_CHUNK_BYTES), t5_desc(w1_addr + j * 2 * T5_CHUNK_BYTES), j > 0);
-            t5_commit(bar1);
-        }
-        fetch(tile + gridDim.x);                           // next tile's rows: in flight during this tile's epilogues
-        t5_wait(bar1, parity);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        // ---- epilogue 1: h1 = relu(D1 + b1) -> A2 (this thread: its row, 32 columns) ----
-        {
-            uint32_t v[32];
-            t5_ld32(t_lane + (uint32_t)col0, v);
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                float4 o;
-                o.x = tf(fmaxf(__uint_as_float(v[4 * q + 0]) + b1s[col0 + 4 * q + 0], 0.f));
-                o.y = tf(fmaxf(__uint_as_float(v[4 * q + 1]) + b1s[col0 + 4 * q + 1], 0.f));
-                o.z = tf(fmaxf(__uint_as_float(v[4 * q + 2]) + b1s[col0 + 4 * q + 2], 0.f));
-                o.w = tf(fmaxf(__uint_as_float(v[4 * q + 3]) + b1s[col0 + 4 * q + 3], 0.f));
-                a2[(col0 / 4 + q) * T5_ROWS + row_in_tile] = o;
-            }
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-                t5_mma(tmem + 128, t5_desc(a2_addr + j * 2 * T5_CHUNK_BYTES), t5_desc(w2_addr + j * 2 * T5_CHUNK_BYTES), j > 0);
-            t5_commit(bar2);
-        }
-        t5_wait(bar2, parity);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        // ---- epilogue 2: h2 = relu(D2 + b2), output layer as FMAs over this thread's 32 hidden units ----
-        float lg[AC_OUT] = {0.f, 0.f, 0.f, 0.f, 0.f};
-        {
-            uint32_t v[32];
-            t5_ld32(t_lane + 128u + (uint32_t)col0, v);
-#pragma unroll
-            for (int j = 0; j < 32; ++j) {
-                const float h = fmaxf(__uint_as_float(v[j]) + b2s[col0 + j], 0.f);
-                const float4 wa = *reinterpret_cast<const float4 *>(w3s + (col0 + j) * 8);
-                const float wb = w3s[(col0 + j) * 8 + 4];
-                lg[0] = fmaf(h, wa.x, lg[0]); lg[1] = fmaf(h, wa.y, lg[1]); lg[2] = fmaf(h, wa.z, lg[2]);
-                lg[3] = fmaf(h, wa.w, lg[3]); lg[4] = fmaf(h, wb, lg[4]);
-            }
-        }
-        if (cgrp > 0) {
-#pragma unroll
-            for (int k = 0; k < AC_OUT; ++k) part[((cgrp - 1) * T5_ROWS + row_in_tile) * 8 + k] = lg[k];
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        const int64_t row = tile * T5_ROWS + row_in_tile;
-        if (cgrp == 0 && row < n_rows) {
-            float l[AC_OUT];
-#pragma unroll
-            for (int k = 0; k < AC_OUT; ++k) {
-                float acc = lg[k];
-#pragma unroll
-                for (int g2 = 0; g2 < T5_CSPLIT - 1; ++g2) acc += part[(g2 * T5_ROWS + row_in_tile) * 8 + k];
-                l[k] = acc + b3s[k];
-            }
-            apply_action_mask(l, mask_bits, row);
-            float m = l[0];
-#pragma unroll
-            for (int k = 1; k < AC_OUT; ++k) m = fmaxf(m, l[k]);
-            float e[AC_OUT], S = 0.f;
-#pragma unroll
-            for (int k = 0; k < AC_OUT; ++k) { e[k] = __expf(l[k] - m); S += e[k]; }
-            const float logS = __logf(S);
-            const float u = (float)(philox_row(seed, step, (uint64_t)row) >> 8) * (1.0f / 16777216.0f);
-            const float target = u * S;
-            int a = AC_OUT - 1;
-            float c = 0.f;
-            bool found = false;
-#pragma unroll
-            for (int k = 0; k < AC_OUT; ++k) {
-                c += e[k];
-                if (!found && target < c) { a = k; found = true; }
-            }
-            bool live = true;
-            if (n_agents) live = (int)(row % MAXV) < n_agents[row / MAXV];
-            actions[row] = (int8_t)(live ? a : 1);
-            if (logp_sel) logp_sel[row] = l[a] - m - logS;
-            if (logp_all) {
-#pragma unroll
-                for (int k = 0; k < AC_OUT; ++k) logp_all[row * AC_OUT + k] = l[k] - m - logS;
-            }
-        }
-        __syncthreads();   // `part` is reused by the next tile
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
-}
-
-// ------------------------------------------------------------------------------------------------
-// tcgen05, second generation: fp16 operands, two CTAs per SM, any first-layer width, optional value head
-// ------------------------------------------------------------------------------------------------
-// The TF32 kernel above runs one tile at a time per SM: stage -> MMA -> epilogue -> MMA -> epilogue, each phase waiting
-// for the one before (ncu: long-scoreboard stalls on tcgen05.ld / mbarrier polls, tensor pipe 19 % busy).  This one
-// halves every shared-memory operand (kind::f16: fp16 has TF32's 10-bit mantissa; observations live in [-1, 1], the
-// hidden activations of these networks stay far below 65 504) so that TWO CTAs fit an SM (<= 108 KB each, 256 TMEM
-// columns each): while one CTA's threads run an epilogue the other CTA's MMAs and loads proceed - the overlap of a
-// software pipeline without warp specialisation.  MMAs are K = 16 (half as many instructions).  The 128 -> 5 output
-// layer (+ the value column) is a third MMA (N = 16) on h2 staged as fp16: as per-thread FMAs over shared-memory weights
-// it was ~55 % of the kernel's instructions (ncu: 55 M warp-instructions per launch, issue slots 46 % busy).
-// 786 432 rows: TF32 kernel 0.167 ms -> 0.115 (fp16, two CTAs / SM) -> 0.093 (third MMA).
-//   H1 = 128: MAPPO ActorNetwork 30-128-128-5 (Model_common.py:5-23).
-//   H1 = 160: MAPPO_GI ActorCriticNetwork with state_split (Model_gi.py:137-220): its three first-layer blocks
-//             (5 -> 32, 10 -> 64, 10 -> 64 over fixed column lists) are ONE 30 -> 160 layer whose weight matrix is zero
-//             outside the blocks; the host scatters fc11 / fc12 / fc13 into it (rollout.py).  The optional sixth output
-//             column is critic_linear (the state value V(s), mappo_gi.py:396-404).
-// CTA = 256 threads: warp w reads TMEM lane quarter w % 4 (hardware rule) and column half w / 4.  D2 reuses D1's
-// columns (D1 is dead once epilogue 1 has been read and the CTA has synchronised), h2 reuses h1's shared memory, D3 sits
-// in columns 192..207; the final epilogue (log-softmax, draw) runs in the 128 threads of column half 0, one row each.
-template <int H1>
-struct M5 {
-    static constexpr int THREADS = 256;
-    static constexpr int ROWS = 128;
-    static constexpr int CH1 = H1 / 8;                        // k-chunks (8 halves = 16 bytes) of layer 2
-    static constexpr uint32_t A_CHUNK = ROWS * 16;            // one k-chunk of the 128 rows of a tile / of W2's 128 rows
-    static constexpr uint32_t W1_CHUNK = H1 * 16;             // one k-chunk of W1's H1 rows
-    static constexpr uint32_t W3_CHUNK = 16 * 16;             // one k-chunk of the output layer's 16 rows (5 logits, the value, 10 zero)
-    static constexpr uint32_t A1 = 0;                         // [4 chunks][128] 16 B
-    static constexpr uint32_t W1 = A1 + 4 * A_CHUNK;          // [4 chunks][H1]
-    static constexpr uint32_t A2 = W1 + 4 * W1_CHUNK;         // [CH1][128]: h1, then (first 16 chunks) h2
-    static constexpr uint32_t W2 = A2 + CH1 * A_CHUNK;        // [CH1][128]
-    static constexpr uint32_t W3 = W2 + CH1 * A_CHUNK;        // [16 chunks][16]
-    static constexpr uint32_t B1 = W3 + 16 * W3_CHUNK;
-    static constexpr uint32_t B2 = B1 + H1 * 4;
-    static constexpr uint32_t B3 = B2 + AC_HID * 4;
-    static constexpr uint32_t BAR = B3 + 8 * 4;               // 3 mbarriers + the TMEM base address
-    static constexpr uint32_t SMEM = BAR + 32;
-    static constexpr uint32_t D3_COL = 192;                   // TMEM columns: D1 0..H1-1, D2 0..127 (reuses D1's), D3 192..207
-    // instruction descriptors, kind::f16: F32 accumulate, fp16 A / B, K-major, M = 128, N = H1 / 128 / 16
-    static constexpr uint32_t IDESC1 = (1u << 4) | ((uint32_t)(H1 >> 3) << 17) | ((128u >> 4) << 24);
-    static constexpr uint32_t IDESC2 = (1u << 4) | ((uint32_t)(AC_HID >> 3) << 17) | ((128u >> 4) << 24);
-    static constexpr uint32_t IDESC3 = (1u << 4) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
-};
-
-__device__ __forceinline__ uint64_t m5_desc(uint32_t smem_addr, uint32_t lbo_bytes) {
+__device__ __forceinline__ uint64_t tc_desc(uint32_t smem_addr, uint32_t lbo_bytes) {
     // K-major, SWIZZLE_NONE: start address, LBO (between the two 16-byte k-chunks of an MMA), SBO (between 8-row groups)
     return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | ((uint64_t)(lbo_bytes >> 4) << 16) | ((uint64_t)(128u >> 4) << 32) | (1ull << 46);
 }
-__device__ __forceinline__ void m5_mma(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+__device__ __forceinline__ void tc_mma(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
     asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
                  "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %5, %5, %5}, p;\n\t}"
                  ::"r"(tmem_d), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
 }
-__device__ __forceinline__ void m5_ld16(uint32_t taddr, uint32_t (&v)[16]) {
+__device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[16]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
                    "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
@@ -547,222 +274,36 @@ __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
     return r;
 }
 
-template <int H1>
-__global__ void __launch_bounds__(256, 2)
-actor_mlp_tcgen05_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n_agents, int64_t n_rows,
-                         const float *__restrict__ w1, const float *__restrict__ b1, const float *__restrict__ w2,
-                         const float *__restrict__ b2, const float *__restrict__ w3, const float *__restrict__ b3,
-                         const float *__restrict__ wv, const float *__restrict__ bv, uint64_t seed, uint64_t step,
-                         const uint8_t *__restrict__ mask_bits, int8_t *__restrict__ actions, float *__restrict__ logp_all,
-                         float *__restrict__ logp_sel, float *__restrict__ values, float *__restrict__ obs_copy,
-                         uint8_t *__restrict__ live_out) {
-    using L = M5<H1>;
-    extern __shared__ __align__(128) uint8_t m5_sm[];
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    uint4 *a1 = reinterpret_cast<uint4 *>(m5_sm + L::A1), *w1f = reinterpret_cast<uint4 *>(m5_sm + L::W1);
-    uint4 *a2 = reinterpret_cast<uint4 *>(m5_sm + L::A2), *w2f = reinterpret_cast<uint4 *>(m5_sm + L::W2);
-    uint4 *w3f = reinterpret_cast<uint4 *>(m5_sm + L::W3);
-    float *b1s = reinterpret_cast<float *>(m5_sm + L::B1), *b2s = reinterpret_cast<float *>(m5_sm + L::B2);
-    float *b3s = reinterpret_cast<float *>(m5_sm + L::B3);
-    uint64_t *bars = reinterpret_cast<uint64_t *>(m5_sm + L::BAR);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(m5_sm + L::BAR + 24);
-    const uint32_t bar1 = t5_smem(bars), bar2 = t5_smem(bars + 1), bar3 = t5_smem(bars + 2);
-
-    // ---- one-time setup: weights in operand layout (fp16), barriers, TMEM ----
-    for (int idx = tid; idx < 4 * H1; idx += L::THREADS) {           // W1: [out n][in k], k padded 30 -> 32
-        const int c = idx / H1, n = idx % H1, k = 8 * c;
-        float v[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) v[q] = k + q < AC_IN ? w1[n * AC_IN + k + q] : 0.f;
-        w1f[idx] = make_uint4(pack_h2(v[0], v[1]), pack_h2(v[2], v[3]), pack_h2(v[4], v[5]), pack_h2(v[6], v[7]));
-    }
-    for (int idx = tid; idx < L::CH1 * L::ROWS; idx += L::THREADS) {  // W2: [out n = 128][in k = H1]
-        const int c = idx / L::ROWS, n = idx % L::ROWS;
-        const float4 lo = *reinterpret_cast<const float4 *>(w2 + n * H1 + 8 * c), hi = *reinterpret_cast<const float4 *>(w2 + n * H1 + 8 * c + 4);
-        w2f[idx] = make_uint4(pack_h2(lo.x, lo.y), pack_h2(lo.z, lo.w), pack_h2(hi.x, hi.y), pack_h2(hi.z, hi.w));
-    }
-    for (int idx = tid; idx < 16 * 16; idx += L::THREADS) {          // output layer: rows 0..4 logits, 5 the value head, rest zero
-        const int c = idx / 16, n = idx % 16;
-        float v[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) v[q] = n < AC_OUT ? w3[n * AC_HID + 8 * c + q] : (n == AC_OUT && wv ? wv[8 * c + q] : 0.f);
-        w3f[idx] = make_uint4(pack_h2(v[0], v[1]), pack_h2(v[2], v[3]), pack_h2(v[4], v[5]), pack_h2(v[6], v[7]));
-    }
-    for (int idx = tid; idx < H1; idx += L::THREADS) b1s[idx] = b1[idx];
-    for (int idx = tid; idx < AC_HID; idx += L::THREADS) b2s[idx] = b2[idx];
-    if (tid < 8) b3s[tid] = tid < AC_OUT ? b3[tid] : (tid == AC_OUT && bv ? bv[0] : 0.f);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar1));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar2));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar3));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(t5_smem(tmem_slot)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = *tmem_slot;
-    const uint32_t a1_addr = t5_smem(a1), w1_addr = t5_smem(w1f), a2_addr = t5_smem(a2), w2_addr = t5_smem(w2f), w3_addr = t5_smem(w3f);
-
-    const int row_in_tile = 32 * (warp & 3) + lane;        // TMEM lane = row of the tile this thread reads
-    const int hh = warp >> 2;                              // column half
-    const uint32_t t_lane = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
-    const int64_t n_tiles = (n_rows + L::ROWS - 1) / L::ROWS;
-    // observation staging: thread t handles row t % 128, k-chunks 2 * (t / 128) and + 1 (8 floats each)
-    const int st_r = tid & (L::ROWS - 1), st_c0 = 2 * (tid >> 7);
-    float2 pre[8];
-    auto fetch = [&](int64_t tile) {
-        const int64_t row = tile * L::ROWS + st_r;
-        const float2 *src = reinterpret_cast<const float2 *>(obs + row * AC_IN);   // rows are 120 B: 8-byte aligned
-        const bool ok = tile < n_tiles && row < n_rows;
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-            const int f2 = 4 * st_c0 + q;                  // float2 index inside the row: 15 hold data
-            pre[q] = (ok && f2 < AC_IN / 2) ? __ldg(src + f2) : make_float2(0.f, 0.f);
-            // rollout buffer (MAPPO.interact appends the state it acted on, mappo.py:117-131): the rows pass through
-            // this thread anyway
-            if (obs_copy && ok && f2 < AC_IN / 2) __stcs(reinterpret_cast<float2 *>(obs_copy + row * AC_IN) + f2, pre[q]);
-        }
-    };
-    fetch(blockIdx.x);
-    uint32_t parity = 0;
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, parity ^= 1) {
-#pragma unroll
-        for (int q = 0; q < 2; ++q)
-            a1[(st_c0 + q) * L::ROWS + st_r] = make_uint4(pack_h2(pre[4 * q].x, pre[4 * q].y), pack_h2(pre[4 * q + 1].x, pre[4 * q + 1].y),
-                                                         pack_h2(pre[4 * q + 2].x, pre[4 * q + 2].y), pack_h2(pre[4 * q + 3].x, pre[4 * q + 3].y));
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-                m5_mma(tmem, m5_desc(a1_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), m5_desc(w1_addr + j * 2 * L::W1_CHUNK, L::W1_CHUNK),
-                       L::IDESC1, j > 0);
-            t5_commit(bar1);
-        }
-        fetch(tile + gridDim.x);                           // next tile's rows: in flight during this tile's epilogues
-        t5_wait(bar1, parity);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        // ---- epilogue 1: h1 = relu(D1 + b1) -> A2 (this thread: its row, H1 / 2 columns in pieces of 16) ----
-#pragma unroll 1
-        for (int it = 0; it < H1 / 32; ++it) {
-            const int col = hh * (H1 / 2) + 16 * it;
-            uint32_t v[16];
-            m5_ld16(t_lane + (uint32_t)col, v);
-            float h[16];
-#pragma unroll
-            for (int q = 0; q < 16; ++q) h[q] = fmaxf(__uint_as_float(v[q]) + b1s[col + q], 0.f);
-            a2[(col / 8) * L::ROWS + row_in_tile] = make_uint4(pack_h2(h[0], h[1]), pack_h2(h[2], h[3]), pack_h2(h[4], h[5]), pack_h2(h[6], h[7]));
-            a2[(col / 8 + 1) * L::ROWS + row_in_tile] = make_uint4(pack_h2(h[8], h[9]), pack_h2(h[10], h[11]), pack_h2(h[12], h[13]), pack_h2(h[14], h[15]));
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int j = 0; j < H1 / 16; ++j)
-                m5_mma(tmem, m5_desc(a2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), m5_desc(w2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK),
-                       L::IDESC2, j > 0);
-            t5_commit(bar2);
-        }
-        t5_wait(bar2, parity);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        // ---- epilogue 2: h2 = relu(D2 + b2) -> the first 16 chunks of A2 (MMA2 has finished reading h1) ----
-#pragma unroll 1
-        for (int it = 0; it < 4; ++it) {
-            const int col = hh * 64 + 16 * it;
-            uint32_t v[16];
-            m5_ld16(t_lane + (uint32_t)col, v);
-            float h[16];
-#pragma unroll
-            for (int q = 0; q < 16; ++q) h[q] = fmaxf(__uint_as_float(v[q]) + b2s[col + q], 0.f);
-            a2[(col / 8) * L::ROWS + row_in_tile] = make_uint4(pack_h2(h[0], h[1]), pack_h2(h[2], h[3]), pack_h2(h[4], h[5]), pack_h2(h[6], h[7]));
-            a2[(col / 8 + 1) * L::ROWS + row_in_tile] = make_uint4(pack_h2(h[8], h[9]), pack_h2(h[10], h[11]), pack_h2(h[12], h[13]), pack_h2(h[14], h[15]));
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        // ---- output layer 128 -> 5 (+ value) as a third MMA (N = 16): D3 = h2 * W3^T ----
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int j = 0; j < AC_HID / 16; ++j)
-                m5_mma(tmem + L::D3_COL, m5_desc(a2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), m5_desc(w3_addr + j * 2 * L::W3_CHUNK, L::W3_CHUNK),
-                       L::IDESC3, j > 0);
-            t5_commit(bar3);
-        }
-        t5_wait(bar3, parity);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const int64_t row = tile * L::ROWS + row_in_tile;
-        if (hh == 0) {
-            uint32_t v[16];
-            m5_ld16(t_lane + L::D3_COL, v);
-            if (row < n_rows) {
-                float l[AC_OUT];
-#pragma unroll
-                for (int k = 0; k < AC_OUT; ++k) l[k] = __uint_as_float(v[k]) + b3s[k];
-                if (values) values[row] = __uint_as_float(v[AC_OUT]) + b3s[AC_OUT];
-                apply_action_mask(l, mask_bits, row);
-                float m = l[0];
-#pragma unroll
-                for (int k = 1; k < AC_OUT; ++k) m = fmaxf(m, l[k]);
-                float e[AC_OUT], S = 0.f;
-#pragma unroll
-                for (int k = 0; k < AC_OUT; ++k) { e[k] = __expf(l[k] - m); S += e[k]; }
-                const float logS = __logf(S);
-                const float u = (float)(philox_row(seed, step, (uint64_t)row) >> 8) * (1.0f / 16777216.0f);
-                const float target = u * S;
-                int a = AC_OUT - 1;
-                float c = 0.f;
-                bool found = false;
-#pragma unroll
-                for (int k = 0; k < AC_OUT; ++k) {
-                    c += e[k];
-                    if (!found && target < c) { a = k; found = true; }
-                }
-                bool live = true;
-                if (n_agents) live = (int)(row % MAXV) < n_agents[row / MAXV];
-                actions[row] = (int8_t)(live ? a : 1);
-                if (live_out) live_out[row] = live ? 1 : 0;
-                if (logp_sel) logp_sel[row] = l[a] - m - logS;
-                if (logp_all) {
-#pragma unroll
-                    for (int k = 0; k < AC_OUT; ++k) logp_all[row * AC_OUT + k] = l[k] - m - logS;
-                }
-            }
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();   // TMEM columns and A2 are reused by the next tile
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
-}
-
 // ------------------------------------------------------------------------------------------------
-// tcgen05, third generation: one warpgroup per tile, four (H1 = 128) or three (H1 = 160) tiles in flight per SM
+// tcgen05 kernel: fp16 operands, one warpgroup per tile, four (H1 = 128) or three (H1 = 160) tiles in flight per SM
 // ------------------------------------------------------------------------------------------------
-// ncu on the two-CTA kernel above (profiles/r2_w_ncu_summary.txt): issue slots 33 % busy, 47 % of the stall samples on
-// the long scoreboard (mbarrier polls after each of the three MMAs, and the rollout-buffer store of a row right behind
-// its load, which made the prefetch synchronous), 1 400 thread-instructions per row of which the bias add + relu +
-// convert of the 256 hidden activations were two thirds.  Changes:
-//   * the weights sit in shared memory ONCE per SM and every warpgroup (128 threads = the 128 TMEM lanes = the 128 rows of
-//     a tile) runs its own tile pipeline on its own operand buffers, TMEM columns, named barrier and mbarrier: more
-//     tiles in flight per SM, no CTA-wide barrier;
+//   H1 = 128: MAPPO ActorNetwork 30-128-128-5 (Model_common.py:5-23).
+//   H1 = 160: MAPPO_GI ActorCriticNetwork with state_split (Model_gi.py:137-220): its three first-layer blocks
+//             (5 -> 32, 10 -> 64, 10 -> 64 over fixed column lists) are ONE 30 -> 160 layer whose weight matrix is zero
+//             outside the blocks; the host scatters fc11 / fc12 / fc13 into it (rollout.py).  The optional sixth output
+//             column is critic_linear (the state value V(s), mappo_gi.py:396-404).
+// Per 128-row tile (= the 128 TMEM lanes):
+//   layer 1   D1[128 x H1]  = A1[128 x 32] * W1^T    tcgen05.mma kind::f16, K = 16
+//   layer 2   D2[128 x 128] = h1[128 x H1] * W2^T
+//   layer 3   D3[128 x 16]  = h2[128 x 128] * W3^T   5 logits, the value, 10 zero columns: as per-thread FMAs this
+//             output layer was ~55 % of the instructions of an earlier kernel
+//   then log-softmax and the inverse-CDF draw in the thread that owns the row.
+// fp16 operands (kind::f16): fp16 has TF32's 10-bit mantissa, observations live in [-1, 1] and the hidden activations of
+// these networks stay far below 65 504, so half of TF32's shared memory per operand.  Operands are K-major, no swizzle,
+// laid out [k-chunk][row] in 16-byte pieces of 8 halves: core matrices of 8 rows, SBO = 128 B between 8-row groups,
+// LBO = one chunk between the two k-chunks of an MMA.  Design:
+//   * the weights sit in shared memory ONCE per SM and every warpgroup (128 threads = the 128 rows of a tile) runs its
+//     own tile pipeline on its own operand buffers, TMEM columns, named barrier and mbarrier: while one warpgroup runs
+//     an epilogue, the others' MMAs and loads proceed, with no CTA-wide barrier;
+//   * warp w reads TMEM lane quarter w % 4 (hardware rule), i.e. the rows of its own quarter of the tile;
 //   * biases ride in the MMAs: an extra K-step multiplies a constant block (1, 1, 0, ...) by (hi, lo) fp16 halves of the
 //     bias (layer 1 uses its two padding columns k = 30, 31), so the accumulator already holds D + b to ~2^-22;
 //   * the epilogue of a hidden layer is cvt.rn.relu.f16x2.f32 - one instruction per two activations - and a 16-byte
 //     shared store per eight;
-//   * D3 reuses the first 16 columns of the tile's TMEM region (D2 is dead once epilogue 2 has synchronised).
+//   * D2 reuses D1's columns and h2 h1's shared memory; D3 reuses the first 16 columns of the tile's TMEM region (D2 is
+//     dead once epilogue 2 has synchronised).
 template <int H1>
-struct M6 {
+struct WgLayout {
     static constexpr int NWG = H1 == 128 ? 4 : 3;            // tiles in flight: shared memory (H1 = 160) or TMEM (128) bound
     static constexpr int THREADS = 128 * NWG;
     static constexpr int ROWS = 128;
@@ -784,8 +325,8 @@ struct M6 {
     static constexpr uint32_t IDESC2 = (1u << 4) | ((uint32_t)(AC_HID >> 3) << 17) | ((128u >> 4) << 24);
     static constexpr uint32_t IDESC3 = (1u << 4) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
 };
-static_assert(M6<128>::SMEM <= 227 * 1024 && M6<160>::SMEM <= 227 * 1024, "actor kernel shared memory");
-static_assert(M6<128>::NWG * M6<128>::REGION <= 512 && M6<160>::NWG * M6<160>::REGION <= 512, "actor kernel TMEM columns");
+static_assert(WgLayout<128>::SMEM <= 227 * 1024 && WgLayout<160>::SMEM <= 227 * 1024, "actor kernel shared memory");
+static_assert(WgLayout<128>::NWG * WgLayout<128>::REGION <= 512 && WgLayout<160>::NWG * WgLayout<160>::REGION <= 512, "actor kernel TMEM columns");
 
 __device__ __forceinline__ uint32_t pack_relu_h2(uint32_t a_bits, uint32_t b_bits) {
     uint32_t r;
@@ -799,7 +340,7 @@ __device__ __forceinline__ uint32_t hi_lo_h2(float b) {          // fp16 halves 
 __device__ __forceinline__ void wg_sync(int wg) { asm volatile("bar.sync %0, 128;" ::"r"(wg + 1) : "memory"); }
 
 template <int H1>
-__global__ void __launch_bounds__(M6<H1>::THREADS, 1)
+__global__ void __launch_bounds__(WgLayout<H1>::THREADS, 1)
 actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n_agents, int64_t n_rows,
                     const float *__restrict__ w1, const float *__restrict__ b1, const float *__restrict__ w2,
                     const float *__restrict__ b2, const float *__restrict__ w3, const float *__restrict__ b3,
@@ -807,15 +348,15 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
                     const uint8_t *__restrict__ mask_bits, int8_t *__restrict__ actions, float *__restrict__ logp_all,
                     float *__restrict__ logp_sel, float *__restrict__ values, float *__restrict__ obs_copy,
                     uint8_t *__restrict__ live_out) {
-    using L = M6<H1>;
-    extern __shared__ __align__(128) uint8_t m6_sm[];
+    using L = WgLayout<H1>;
+    extern __shared__ __align__(128) uint8_t wg_sm[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, wg = warp >> 2;
-    uint4 *w1f = reinterpret_cast<uint4 *>(m6_sm + L::W1), *w2f = reinterpret_cast<uint4 *>(m6_sm + L::W2);
-    uint4 *w3f = reinterpret_cast<uint4 *>(m6_sm + L::W3), *ones = reinterpret_cast<uint4 *>(m6_sm + L::ONES);
-    uint4 *a1 = reinterpret_cast<uint4 *>(m6_sm + L::TILE0 + wg * L::TILE_BYTES), *a2 = a1 + 4 * L::ROWS;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(m6_sm + L::BAR);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(m6_sm + L::BAR + 8 * L::NWG);
-    const uint32_t bar = t5_smem(bars + wg);
+    uint4 *w1f = reinterpret_cast<uint4 *>(wg_sm + L::W1), *w2f = reinterpret_cast<uint4 *>(wg_sm + L::W2);
+    uint4 *w3f = reinterpret_cast<uint4 *>(wg_sm + L::W3), *ones = reinterpret_cast<uint4 *>(wg_sm + L::ONES);
+    uint4 *a1 = reinterpret_cast<uint4 *>(wg_sm + L::TILE0 + wg * L::TILE_BYTES), *a2 = a1 + 4 * L::ROWS;
+    uint64_t *bars = reinterpret_cast<uint64_t *>(wg_sm + L::BAR);
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(wg_sm + L::BAR + 8 * L::NWG);
+    const uint32_t bar = tc_smem(bars + wg);
 
     // ---- one-time setup: weights and biases in operand layout (fp16), the constant block, barriers, TMEM ----
     for (int idx = tid; idx < 4 * H1; idx += L::THREADS) {
@@ -849,10 +390,10 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
         }
     }
     for (int idx = tid; idx < 2 * L::ROWS; idx += L::THREADS) ones[idx] = make_uint4(idx < L::ROWS ? 0x3C003C00u : 0u, 0u, 0u, 0u);
-    if (tid < L::NWG) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(t5_smem(bars + tid)));
+    if (tid < L::NWG) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(tc_smem(bars + tid)));
     if (tid == 0) asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(t5_smem(tmem_slot)) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(tc_smem(tmem_slot)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -860,8 +401,8 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = *tmem_slot + (uint32_t)wg * L::REGION;          // this warpgroup's columns
-    const uint32_t a1_addr = t5_smem(a1), a2_addr = t5_smem(a2), w1_addr = t5_smem(w1f), w2_addr = t5_smem(w2f);
-    const uint32_t w3_addr = t5_smem(w3f), ones_addr = t5_smem(ones);
+    const uint32_t a1_addr = tc_smem(a1), a2_addr = tc_smem(a2), w1_addr = tc_smem(w1f), w2_addr = tc_smem(w2f);
+    const uint32_t w3_addr = tc_smem(w3f), ones_addr = tc_smem(ones);
 
     const int r = tid & 127;                                              // row of the tile = TMEM lane
     const uint32_t t_lane = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
@@ -919,18 +460,18 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #pragma unroll
             for (int j = 0; j < 2; ++j)
-                m5_mma(tmem, m5_desc(a1_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), m5_desc(w1_addr + j * 2 * L::W1_CHUNK, L::W1_CHUNK),
+                tc_mma(tmem, tc_desc(a1_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), tc_desc(w1_addr + j * 2 * L::W1_CHUNK, L::W1_CHUNK),
                        L::IDESC1, j > 0);
-            t5_commit(bar);
+            tc_commit(bar);
         }
         fetch(tile + stride);                                  // next tile's rows: in flight during this tile's MMAs and epilogues
-        t5_wait(bar, parity); parity ^= 1;
+        tc_wait(bar, parity); parity ^= 1;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         // ---- epilogue 1: h1 = relu(D1) -> A2 ----
 #pragma unroll 1
         for (int col = 0; col < H1; col += 32) {
             uint32_t v[32];
-            t5_ld32(t_lane + (uint32_t)col, v);
+            tc_ld32(t_lane + (uint32_t)col, v);
 #pragma unroll
             for (int g = 0; g < 4; ++g)
                 a2[(col / 8 + g) * L::ROWS + r] = make_uint4(pack_relu_h2(v[8 * g], v[8 * g + 1]), pack_relu_h2(v[8 * g + 2], v[8 * g + 3]),
@@ -943,18 +484,18 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #pragma unroll
             for (int j = 0; j < H1 / 16; ++j)
-                m5_mma(tmem, m5_desc(a2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), m5_desc(w2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK),
+                tc_mma(tmem, tc_desc(a2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), tc_desc(w2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK),
                        L::IDESC2, j > 0);
-            m5_mma(tmem, m5_desc(ones_addr, L::A_CHUNK), m5_desc(w2_addr + (H1 / 16) * 2 * L::A_CHUNK, L::A_CHUNK), L::IDESC2, 1);
-            t5_commit(bar);
+            tc_mma(tmem, tc_desc(ones_addr, L::A_CHUNK), tc_desc(w2_addr + (H1 / 16) * 2 * L::A_CHUNK, L::A_CHUNK), L::IDESC2, 1);
+            tc_commit(bar);
         }
-        t5_wait(bar, parity); parity ^= 1;
+        tc_wait(bar, parity); parity ^= 1;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         // ---- epilogue 2: h2 = relu(D2) -> the first 16 chunks of A2 (MMA2 has finished reading h1) ----
 #pragma unroll 1
         for (int col = 0; col < AC_HID; col += 32) {
             uint32_t v[32];
-            t5_ld32(t_lane + (uint32_t)col, v);
+            tc_ld32(t_lane + (uint32_t)col, v);
 #pragma unroll
             for (int g = 0; g < 4; ++g)
                 a2[(col / 8 + g) * L::ROWS + r] = make_uint4(pack_relu_h2(v[8 * g], v[8 * g + 1]), pack_relu_h2(v[8 * g + 2], v[8 * g + 3]),
@@ -968,17 +509,17 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #pragma unroll
             for (int j = 0; j < AC_HID / 16; ++j)
-                m5_mma(tmem, m5_desc(a2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), m5_desc(w3_addr + j * 2 * L::W3_CHUNK, L::W3_CHUNK),
+                tc_mma(tmem, tc_desc(a2_addr + j * 2 * L::A_CHUNK, L::A_CHUNK), tc_desc(w3_addr + j * 2 * L::W3_CHUNK, L::W3_CHUNK),
                        L::IDESC3, j > 0);
-            m5_mma(tmem, m5_desc(ones_addr, L::A_CHUNK), m5_desc(w3_addr + 16 * L::W3_CHUNK, L::W3_CHUNK), L::IDESC3, 1);
-            t5_commit(bar);
+            tc_mma(tmem, tc_desc(ones_addr, L::A_CHUNK), tc_desc(w3_addr + 16 * L::W3_CHUNK, L::W3_CHUNK), L::IDESC3, 1);
+            tc_commit(bar);
         }
-        t5_wait(bar, parity); parity ^= 1;
+        tc_wait(bar, parity); parity ^= 1;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         {
             const int64_t row = tile * L::ROWS + r;
             uint32_t v[16];
-            m5_ld16(t_lane, v);
+            tc_ld16(t_lane, v);
             if (row < n_rows) {
                 float l[AC_OUT];
 #pragma unroll
@@ -1020,14 +561,10 @@ actor_mlp_wg_kernel(const float *__restrict__ obs, const int32_t *__restrict__ n
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(*tmem_slot) : "memory");
 }
 
-// -1: not chosen yet; 0: tcgen05 fp16, a warpgroup per tile; 1: mma.sync TF32; 2: tcgen05 TF32, one CTA per SM; 3: tcgen05 fp16, two CTAs per SM
-int g_actor_impl = -1;
-void set_actor_impl(int impl) { g_actor_impl = (impl >= 1 && impl <= 3) ? impl : 0; }
-static void resolve_actor_impl() {
-    if (g_actor_impl >= 0) return;
-    const char *e = getenv("MM_ACTOR_IMPL");
-    g_actor_impl = !e ? 0 : (e[0] == 'm' ? 1 : (e[0] == 't' ? 2 : (e[0] == 'c' ? 3 : 0)));
-}
+// Implementation of mm_actor_sample, chosen by mm_set_actor_impl: the tcgen05 kernel (default) or, when set, the
+// mma.sync kernel as the independent cross-check.  mm_actor_sample_mlp always runs the tcgen05 kernel.
+static bool g_actor_mma = false;
+void set_actor_impl(int impl) { g_actor_mma = impl == 1; }
 
 template <int H1>
 static int launch_actor_mlp_t(const float *obs, const int32_t *n_agents, int64_t n_rows, const float *w1, const float *b1,
@@ -1038,26 +575,13 @@ static int launch_actor_mlp_t(const float *obs, const int32_t *n_agents, int64_t
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= MM_MAX_DEVICES) return 1;
     if (!ready[dev]) {
-        if (cudaFuncSetAttribute(actor_mlp_tcgen05_kernel<H1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)M5<H1>::SMEM) != cudaSuccess)
+        if (cudaFuncSetAttribute(actor_mlp_wg_kernel<H1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WgLayout<H1>::SMEM) != cudaSuccess)
             return 1;
         ready[dev] = true;
     }
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (g_actor_impl != 3) {                                       // default: one warpgroup per tile, one CTA per SM
-        static bool wg_ready[MM_MAX_DEVICES] = {};
-        if (!wg_ready[dev]) {
-            if (cudaFuncSetAttribute(actor_mlp_wg_kernel<H1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)M6<H1>::SMEM) != cudaSuccess)
-                return 1;
-            wg_ready[dev] = true;
-        }
-        const int64_t n_tiles = (n_rows + 127) / 128, grid = n_tiles < sms ? n_tiles : sms;
-        actor_mlp_wg_kernel<H1><<<(unsigned)grid, M6<H1>::THREADS, M6<H1>::SMEM, (cudaStream_t)stream>>>(
-            obs, n_agents, n_rows, w1, b1, w2, b2, w3, b3, wv, bv, seed, step, mask_bits, actions, logp_all, logp_sel, values, obs_copy,
-            live_out);
-        return cudaGetLastError() == cudaSuccess ? 0 : 1;
-    }
-    const int64_t tiles = (n_rows + 127) / 128, ctas = tiles < 2 * sms ? tiles : 2 * sms;   // persistent: two CTAs per SM
-    actor_mlp_tcgen05_kernel<H1><<<(unsigned)ctas, 256, M5<H1>::SMEM, (cudaStream_t)stream>>>(
+    const int64_t n_tiles = (n_rows + 127) / 128, grid = n_tiles < sms ? n_tiles : sms;   // persistent: one CTA per SM
+    actor_mlp_wg_kernel<H1><<<(unsigned)grid, WgLayout<H1>::THREADS, WgLayout<H1>::SMEM, (cudaStream_t)stream>>>(
         obs, n_agents, n_rows, w1, b1, w2, b2, w3, b3, wv, bv, seed, step, mask_bits, actions, logp_all, logp_sel, values, obs_copy,
         live_out);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
@@ -1068,7 +592,6 @@ int launch_actor_mlp(const float *obs, const int32_t *n_agents, int64_t n_rows, 
                      uint64_t seed, uint64_t step, const uint8_t *mask_bits, int8_t *actions, float *logp_all, float *logp_sel,
                      float *values, float *obs_copy, uint8_t *live_out, void *stream) {
     if (n_rows <= 0) return 0;
-    resolve_actor_impl();
     if (h1 == 128)
         return launch_actor_mlp_t<128>(obs, n_agents, n_rows, w1, b1, w2, b2, w3, b3, wv, bv, seed, step, mask_bits, actions, logp_all,
                                        logp_sel, values, obs_copy, live_out, stream);
@@ -1107,38 +630,22 @@ int launch_discounted_returns(const float *rewards, const uint8_t *dones, const 
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
-
 int launch_actor_sample(const float *obs, const int32_t *n_agents, int64_t n_rows, const float *w1, const float *b1,
                         const float *w2, const float *b2, const float *w3, const float *b3, uint64_t seed, uint64_t step,
                         const uint8_t *mask_bits, int8_t *actions, float *logp_all, float *logp_sel, void *stream) {
     if (n_rows <= 0) return 0;
-    static bool attr_set = false;
-    const int smem = AC_SMEM_WORDS * (int)sizeof(uint32_t);
-    if (!attr_set) {
-        if (cudaFuncSetAttribute(actor_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
-        attr_set = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    // g_actor_impl (mm_set_actor_impl; initial value from MM_ACTOR_IMPL=mma): 1 selects the warp-level mma.sync kernel
-    // above, kept as the independent cross-check of the tcgen05 one
-    resolve_actor_impl();
-    if (g_actor_impl == 0 || g_actor_impl == 3)
+    if (!g_actor_mma)
         return launch_actor_mlp(obs, n_agents, n_rows, 128, w1, b1, w2, b2, w3, b3, nullptr, nullptr, seed, step, mask_bits, actions,
                                 logp_all, logp_sel, nullptr, nullptr, nullptr, stream);
-    if (g_actor_impl == 2) {
-        static bool t5_attr = false;
-        if (!t5_attr) {
-            if (cudaFuncSetAttribute(actor_sample_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T5_SMEM) != cudaSuccess)
-                return 1;
-            t5_attr = true;
-        }
-        int64_t t5_tiles = (n_rows + T5_ROWS - 1) / T5_ROWS, t5_ctas = t5_tiles < sms ? t5_tiles : sms;
-        actor_sample_tcgen05_kernel<<<(unsigned)t5_ctas, T5_THREADS, T5_SMEM, (cudaStream_t)stream>>>(
-            obs, n_agents, n_rows, w1, b1, w2, b2, w3, b3, seed, step, mask_bits, actions, logp_all, logp_sel);
-        return cudaGetLastError() == cudaSuccess ? 0 : 1;
+    static bool ready[MM_MAX_DEVICES] = {};
+    const int smem = AC_SMEM_WORDS * (int)sizeof(uint32_t);
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= MM_MAX_DEVICES) return 1;
+    if (!ready[dev]) {
+        if (cudaFuncSetAttribute(actor_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
+        ready[dev] = true;
     }
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     int64_t tiles = (n_rows + 15) / 16, ctas = (tiles + AC_THREADS / 32 - 1) / (AC_THREADS / 32);
     if (ctas > sms) ctas = sms;   // persistent: one CTA per SM, warps stride over the 16-row tiles
     actor_sample_kernel<<<(unsigned)ctas, AC_THREADS, smem, (cudaStream_t)stream>>>(obs, n_agents, n_rows, w1, b1, w2, b2, w3,

@@ -894,8 +894,7 @@ int mm_actor_sample_mlp(const float *obs, const int32_t *n_agents, int64_t n_row
 }
 
 int mm_set_actor_impl(int impl) {
-    if (impl < 0 || impl > 3)
-        return fail(MM_ERR_ARG, "impl must be 0 (tcgen05 fp16, warpgroup per tile), 1 (mma.sync TF32), 2 (tcgen05 TF32) or 3 (tcgen05 fp16, two CTAs per SM)");
+    if (impl != 0 && impl != 1) return fail(MM_ERR_ARG, "impl must be 0 (tcgen05 fp16, default) or 1 (mma.sync TF32 cross-check)");
     set_actor_impl(impl);
     return 0;
 }

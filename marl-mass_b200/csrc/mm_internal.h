@@ -149,7 +149,7 @@ void launch_packed_pack(const uint32_t *einfo, const int32_t *n_agents, const fl
 int launch_actor_sample(const float *obs, const int32_t *n_agents, int64_t n_rows, const float *w1, const float *b1,
                         const float *w2, const float *b2, const float *w3, const float *b3, uint64_t seed, uint64_t step,
                         const uint8_t *mask_bits, int8_t *actions, float *logp_all, float *logp_sel, void *stream);
-void set_actor_impl(int impl);
+void set_actor_impl(int impl);   // 0: the fp16 tcgen05 kernel (default), 1: the mma.sync cross-check (checked by the C ABI)
 // the fp16 tcgen05 kernel for a 30 - h1 - 128 - 5 network (h1 = 128 or 160), optional value head (wv [128], bv [1] -> values)
 int launch_actor_mlp(const float *obs, const int32_t *n_agents, int64_t n_rows, int h1, const float *w1, const float *b1,
                      const float *w2, const float *b2, const float *w3, const float *b3, const float *wv, const float *bv,

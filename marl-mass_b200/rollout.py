@@ -172,11 +172,17 @@ def discounted_returns(rewards, dones, final_value, gamma):
     return out
 
 
+_ACTOR_IMPLS = {"tcgen05": 0, "mma": 1}
+
+
 def set_actor_impl(name):
-    """'tcgen05' (default: fp16 operands, a warpgroup per 128-row tile, weights once per SM), 'mma' (the warp-level
-    mma.sync TF32 kernel, kept as an independent cross-check), 'tcgen05_tf32' (the first tcgen05 kernel: TF32 operands,
-    one CTA per SM) or 'tcgen05_cta' (fp16 operands, two CTAs per SM: the default of the first half of round 2)."""
-    _lib.check(_lib.lib().mm_set_actor_impl({"tcgen05": 0, "mma": 1, "tcgen05_tf32": 2, "tcgen05_cta": 3}[name]))
+    """Kernel of mm_actor_sample (actor_sample without obs_copy / live_out), process-wide: 'tcgen05' (default: fp16
+    operands, a warpgroup per 128-row tile, weights once per SM) or 'mma' (the warp-level mma.sync TF32 kernel, kept as
+    an independent cross-check).  The appending actor_sample calls and policy_sample always run the tcgen05 kernel.
+    Any other name raises ValueError."""
+    if name not in _ACTOR_IMPLS:
+        raise ValueError("actor impl must be one of %s, got %r" % (", ".join(map(repr, _ACTOR_IMPLS)), name))
+    _lib.check(_lib.lib().mm_set_actor_impl(_ACTOR_IMPLS[name]))
 
 
 _DENSE_CACHE = {}

@@ -41,9 +41,9 @@ lp = mm.rollout.actor_sample(pol.actor, obs, v["n_agents"], seed=1, step=1, want
 with torch.no_grad():
     logp = pol.actor(obs.view(-1, mm.NS))          # the env has stepped since the first evaluation: same rows again
 print("max |logp_fused - logp_torch| = %.3e" % float((lp.view(-1, 5) - logp).abs().max()))
-# round 2: the three actor kernels and the MAPPO_GI shared network on the same rows
+# the two actor kernels and the MAPPO_GI shared network on the same rows
 from marl_mass_b200 import rollout
-for name in ("tcgen05", "tcgen05_cta", "tcgen05_tf32", "mma"):
+for name in ("tcgen05", "mma"):
     rollout.set_actor_impl(name)
     print("actor_sample %-13s %.4f ms" % (name, timed(lambda: rollout.actor_sample(pol.actor, obs, v["n_agents"], seed=1, step=1), n=50)))
 rollout.set_actor_impl("tcgen05")

@@ -2,8 +2,9 @@
 kernel, through the C ABI, against the reference vectors (tests/golden/mappo_caller.npz), the numpy restatements in
 oracle/ and a plain torch fp32 evaluation of the same network.
 
-Tolerances: the actor runs on TF32 tensor cores (10-bit mantissa, fp32 accumulate): log-probabilities within 2e-2
-absolute of the fp32 network on O(1) inputs (observed ~3e-3); returns are fp32 sums: 1e-5 relative.
+Tolerances: the actor runs on tensor cores with fp16 operands (the mma.sync cross-check with TF32 ones: both have a
+10-bit mantissa) and fp32 accumulation: log-probabilities within 2e-2 absolute of the fp32 network on O(1) inputs
+(observed ~3e-3); returns are fp32 sums: 1e-5 relative.
 """
 import os
 
@@ -85,53 +86,35 @@ def test_actor_matches_torch_fp32_on_env_observations_and_masks_absent_agents(mm
 
 
 def test_tcgen05_and_mma_sync_actor_kernels_agree(mm):
-    """The tcgen05 kernel (TMEM accumulators, row-per-thread epilogue) against the independent mma.sync kernel (register
-    fragments): same TF32 inputs for the two hidden layers, different accumulation order, and the output layer in fp32
-    FMAs (tcgen05 kernel) vs a TF32 MMA (mma.sync kernel) -> log-probabilities within 1e-2 (observed 3.5e-3 with 3x
-    the default weight scale); the same uniform per row -> the same action except where the draw falls within that
-    distance of a CDF step."""
+    """The default tcgen05 kernel (fp16 operands, biases inside the MMAs, TMEM accumulators) against the independent
+    mma.sync kernel (TF32 register fragments) and torch fp32, with the default weights and with 3x their scale (a sharper
+    policy): fp16 and TF32 share the 10-bit mantissa and both accumulate in fp32 -> log-probabilities within 1e-2 of
+    torch and of each other (observed at 3x scale: 5.7e-3 and 3.0e-3); the same uniform per row -> the same
+    action except where the draw falls within that distance of a CDF step.  Neither row count is a multiple of the
+    128-row tile."""
     import torch
     from marl_mass_b200 import rollout
-    torch.manual_seed(3)
-    actor = rollout.ActorNetwork().cuda()
-    for p in actor.parameters():
-        p.data.mul_(3.0)
-    obs = (torch.rand(100003, mm.NS, device="cuda") * 2.4 - 1.2).contiguous()      # not a multiple of the 128-row tile
-    try:
-        rollout.set_actor_impl("mma")
-        a_m, lp_m = rollout.actor_sample(actor, obs, None, seed=5, step=2, want_logp=True)
-        rollout.set_actor_impl("tcgen05")
-        a_t, lp_t = rollout.actor_sample(actor, obs, None, seed=5, step=2, want_logp=True)
-        torch.cuda.synchronize()
-    finally:
-        rollout.set_actor_impl("tcgen05")
-    assert float((lp_m - lp_t).abs().max()) < 1e-2
-    assert float((a_m != a_t).float().mean()) < 5e-3
-
-
-def test_all_four_actor_kernels_agree(mm):
-    """fp16 tcgen05 (default: a warpgroup per tile, biases inside the MMAs; and the two-CTA build with fp32 bias adds) vs
-    TF32 tcgen05 vs TF32 mma.sync on the same network and rows: fp16 and TF32 operands share the 10-bit mantissa,
-    accumulation is fp32 everywhere -> log-probabilities within 1e-2, the same draw except next to a CDF step."""
-    import torch
-    from marl_mass_b200 import rollout
-    torch.manual_seed(4)
-    actor = rollout.ActorNetwork().cuda()
-    obs = (torch.rand(70001, mm.NS, device="cuda") * 2.2 - 1.1).contiguous()
-    out = {}
-    try:
-        for name in ("tcgen05", "tcgen05_cta", "tcgen05_tf32", "mma"):
-            rollout.set_actor_impl(name)
-            out[name] = rollout.actor_sample(actor, obs, None, seed=9, step=1, want_logp=True)
-            torch.cuda.synchronize()
-    finally:
-        rollout.set_actor_impl("tcgen05")
-    ref = torch.log_softmax(actor.fc3(torch.relu(actor.fc2(torch.relu(actor.fc1(obs))))), dim=1)
-    for name, (a, lp) in out.items():
-        assert float((lp - ref).abs().max()) < 1e-2, name
-        assert float((a != out["tcgen05"][0]).float().mean()) < 5e-3, name
-    # the two fp16 builds round the same operands: only the bias path differs (hi + lo fp16 halves inside the MMA vs fp32 add)
-    assert float((out["tcgen05"][1] - out["tcgen05_cta"][1]).abs().max()) < 2e-3
+    for torch_seed, scale, rows, span, seed in ((3, 3.0, 100003, 1.2, 5), (4, 1.0, 70001, 1.1, 9)):
+        torch.manual_seed(torch_seed)
+        actor = rollout.ActorNetwork().cuda()
+        for p in actor.parameters():
+            p.data.mul_(scale)
+        obs = (torch.rand(rows, mm.NS, device="cuda") * 2 * span - span).contiguous()
+        out = {}
+        try:
+            for name in ("mma", "tcgen05"):
+                rollout.set_actor_impl(name)
+                out[name] = rollout.actor_sample(actor, obs, None, seed=seed, step=2, want_logp=True)
+                torch.cuda.synchronize()
+        finally:
+            rollout.set_actor_impl("tcgen05")
+        with torch.no_grad():
+            ref = torch.log_softmax(actor.fc3(torch.relu(actor.fc2(torch.relu(actor.fc1(obs))))), dim=1)
+        (a_m, lp_m), (a_t, lp_t) = out["mma"], out["tcgen05"]
+        for name, (_, lp) in out.items():
+            assert float((lp - ref).abs().max()) < 1e-2, (name, scale)
+        assert float((lp_m - lp_t).abs().max()) < 1e-2, scale
+        assert float((a_m != a_t).float().mean()) < 5e-3, scale
 
 
 def test_fused_shared_network_of_mappo_gi(mm):

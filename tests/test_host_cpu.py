@@ -61,6 +61,25 @@ def test_mm_config_layout_agrees_between_header_binding_and_integration_stub():
     assert b"struct_size" in L.mm_last_error()
 
 
+def test_actor_impl_switch_accepts_only_the_two_kernels():
+    """mm_set_actor_impl selects 0 (tcgen05, default) or 1 (the mma.sync cross-check) and refuses anything else with a
+    message naming the two; the Python wrapper refuses unknown names.  The switch makes no CUDA call, so this runs
+    without a GPU."""
+    import marl_mass_b200 as mm
+    from marl_mass_b200 import rollout
+    L = mm.lib()
+    try:
+        for impl in (0, 1):
+            assert L.mm_set_actor_impl(impl) == 0
+        for impl in (-1, 2, 3, 4):
+            assert L.mm_set_actor_impl(impl) == -1
+            assert b"0 (tcgen05" in L.mm_last_error() and b"1 (mma.sync" in L.mm_last_error()
+        with pytest.raises(ValueError, match="'tcgen05', 'mma'"):
+            rollout.set_actor_impl("torch")
+    finally:
+        assert L.mm_set_actor_impl(0) == 0
+
+
 def test_shared_object_is_sm100a_only():
     from marl_mass_b200 import _lib
     out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
