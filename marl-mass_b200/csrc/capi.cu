@@ -34,7 +34,8 @@ int fail(mm_status code, const char *what, cudaError_t ce = cudaSuccess) {
         if (_ce != cudaSuccess) return fail(MM_ERR_CUDA, #expr, _ce);        \
     } while (0)
 
-constexpr int MAX_CHUNKS = 16;
+constexpr int HOST_STREAMS = 4;      // compute streams of the *_host entry points (DESIGN.md §6: four beat two and eight)
+constexpr int N_STREAMS = 2 * HOST_STREAMS;   // mm_step_host_packed adds one copy stream per compute stream
 constexpr int GRAPH_MAX_ENVS = 131072;   // mm_step replays a CUDA graph up to this batch size (above, launch overhead is noise)
 constexpr int MM_SUP_TASKS_PER_ENV = 2;   // predicted collisions per env and step the dmc task list holds (more: evaluated in place)
 constexpr int MAX_HOST_CHUNKS = 64;   // chunks of one mm_step_host_ragged / _packed call
@@ -53,14 +54,13 @@ struct mm_env {
     int8_t *new_actions = nullptr;
     const double *sup_draws = nullptr;
     int32_t *sup_used = nullptr;
-    void *sup_tasks = nullptr;          // dmc pass 2: MM_SUP_TASKS_PER_ENV task records per env (allocated with the first dmc use)
+    char *sup_tasks = nullptr;          // dmc pass 2: MM_SUP_TASKS_PER_ENV task records per env (allocated with the first dmc use)
     int *sup_task_count = nullptr;      // one counter per call (calls start on distinct tiles)
     // mm_step_host_ragged, allocated on first use: first packed row of every env, packed-row staging, per-chunk counts
     int64_t *row_offset = nullptr;
     float *rows_stage = nullptr;
     int64_t *chunk_rows_dev = nullptr, *chunk_rows_host = nullptr;
     cudaEvent_t chunk_done[MAX_HOST_CHUNKS]{};
-    bool ragged_ready = false;
     // mm_step_host_packed, allocated on first use: packed vehicle rows / neighbour words, per-env offsets inside a chunk,
     // count bytes, running totals chained chunk to chunk (device + pinned host mirror), one event per chunk's scan
     float *veh_packed = nullptr;
@@ -69,7 +69,6 @@ struct mm_env {
     uint8_t *n_veh_u8 = nullptr, *n_agents_u8 = nullptr;
     int64_t *chunk_base_dev = nullptr, *chunk_base_host = nullptr, *chunk_base_host_dev = nullptr;
     cudaEvent_t scan_done[MAX_HOST_CHUNKS]{};
-    bool packed_ready = false;
     size_t stats_rows = 0;
     uint64_t seed = 0;
     int64_t launches = 0;
@@ -90,20 +89,41 @@ struct mm_env {
     };
     std::vector<StepGraph> graphs;
     uint64_t epoch = 0;
-    cudaStream_t streams[MAX_CHUNKS]{};
-    int n_streams = 0;
+    cudaStream_t streams[N_STREAMS]{};
     std::vector<void *> allocs;
 };
 
 namespace {
 
+// The allocation helpers do nothing when *ptr is already set, so lazily allocated buffers are requested piece by piece on
+// every call: a failure half-way leaves a handle that retries the missing pieces instead of using null pointers.
 template <typename T>
 int dev_alloc(mm_env *env, T **ptr, size_t count, bool zero = true) {
+    if (*ptr) return 0;
     void *p = nullptr;
     CUDA_OK(cudaMalloc(&p, count * sizeof(T)));
-    if (zero) CUDA_OK(cudaMemset(p, 0, count * sizeof(T)));
     env->allocs.push_back(p);
+    if (zero) CUDA_OK(cudaMemset(p, 0, count * sizeof(T)));
     *ptr = static_cast<T *>(p);
+    return 0;
+}
+
+// Pinned host memory, freed by mm_destroy.  With `dev` the block is mapped and *dev receives its device address.
+template <typename T>
+int host_alloc(T **ptr, size_t count, bool zero, T **dev = nullptr) {
+    if (!*ptr) {
+        void *p = nullptr;
+        CUDA_OK(cudaHostAlloc(&p, count * sizeof(T), dev ? cudaHostAllocMapped : cudaHostAllocDefault));
+        if (zero) memset(p, 0, count * sizeof(T));
+        *ptr = static_cast<T *>(p);
+    }
+    if (dev && !*dev) CUDA_OK(cudaHostGetDevicePointer((void **)dev, *ptr, 0));
+    return 0;
+}
+
+int event_alloc(cudaEvent_t *events, int n) {
+    for (int i = 0; i < n; ++i)
+        if (!events[i]) CUDA_OK(cudaEventCreateWithFlags(&events[i], cudaEventDisableTiming));
     return 0;
 }
 
@@ -157,12 +177,6 @@ int reset_stats(mm_env *env) {
 // un-chunked device-resident step.  A mid-size batch is still cut in 4 chunks (>= 16 Ki envs), one per stream, so that
 // its device-to-host copies overlap the compute of the following chunks instead of trailing a single launch.
 int host_chunk_target(int n_envs) {
-    static const int forced = [] {
-        const char *s = getenv("MM_HOST_CHUNK");
-        int v = s ? atoi(s) : 0;
-        return v > 0 ? v : 0;
-    }();
-    if (forced) return forced;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -171,6 +185,24 @@ int host_chunk_target(int n_envs) {
     if (t < 16384) t = 16384;
     if (t > half_wave) t = half_wave;
     return t;
+}
+
+// The chunks of one host-path call: `used` <= `max_chunks` chunks of `chunk` envs each, the last one shorter.  `chunk` is
+// a multiple of 768 envs, which every supported tile size (32..384) divides; this also keeps the per-warp statistics
+// rows of different chunks disjoint.
+struct ChunkPlan {
+    int n_envs, chunk, used;
+    int off(int c) const { return c * chunk; }
+    int count(int c) const { return n_envs - c * chunk < chunk ? n_envs - c * chunk : chunk; }
+};
+
+ChunkPlan plan_chunks(int n_envs, int max_chunks) {
+    const int target = host_chunk_target(n_envs);
+    int n_chunks = (n_envs + target - 1) / target;
+    if (n_chunks < 1) n_chunks = 1;
+    if (n_chunks > max_chunks) n_chunks = max_chunks;
+    const int chunk = ((n_envs + n_chunks - 1) / n_chunks + 767) / 768 * 768;
+    return {n_envs, chunk, (n_envs + chunk - 1) / chunk};
 }
 
 // The *_host entry points run on the handle's own non-blocking streams.  Work the caller enqueued earlier (mm_reset,
@@ -192,7 +224,7 @@ void enqueue_step(mm_env *env, const int8_t *actions_dev, int auto_reset, int of
         const bool dmc = env->cfg.supervisor != MM_SUPERVISOR_PRIORITY;
         launch_supervisor(env->st, off, count, dmc ? 1 : 0, env->new_actions, env->sup_draws, MM_SUPERVISOR_DRAWS,
                           env->cfg.headway_time, env->seed, env->sup_used,
-                          static_cast<char *>(env->sup_tasks) + (size_t)off * MM_SUP_TASKS_PER_ENV * supervisor_task_bytes(),
+                          env->sup_tasks + (size_t)off * MM_SUP_TASKS_PER_ENV * supervisor_task_bytes(),
                           env->sup_task_count + off / TILE, count * MM_SUP_TASKS_PER_ENV, stream);
         env->launches += dmc ? 2 : 1;
         actions_dev = env->new_actions;
@@ -213,27 +245,42 @@ void enqueue_step(mm_env *env, const int8_t *actions_dev, int auto_reset, int of
     }
 }
 
-}  // namespace
+// host-buffer step of envs [off, off+count) on `stream`: their actions from the caller's host buffer, then the step
+int enqueue_host_step(mm_env *env, const int8_t *actions, int auto_reset, int off, int count, cudaStream_t stream) {
+    CUDA_OK(cudaMemcpyAsync(env->actions + (size_t)off * MAXV, actions + (size_t)off * MAXV, (size_t)count * MAXV,
+                            cudaMemcpyHostToDevice, stream));
+    enqueue_step(env, env->actions, auto_reset, off, count, stream);
+    return 0;
+}
 
-namespace {
+// the per-env outputs of envs [off, off+count) to the caller's host buffers; a null buffer is not copied
+int copy_env_outputs(mm_env *env, int off, int count, cudaStream_t stream, float *reward, uint8_t *done,
+                     float *regional_rewards, int32_t *n_agents_i32) {
+    if (reward)
+        CUDA_OK(cudaMemcpyAsync(reward + off, env->out.reward + off, (size_t)count * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    if (done)
+        CUDA_OK(cudaMemcpyAsync(done + off, env->out.done + off, (size_t)count, cudaMemcpyDeviceToHost, stream));
+    if (regional_rewards)
+        CUDA_OK(cudaMemcpyAsync(regional_rewards + (size_t)off * MAXV, env->out.regional_rewards + (size_t)off * MAXV,
+                                (size_t)count * MAXV * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    if (n_agents_i32)
+        CUDA_OK(cudaMemcpyAsync(n_agents_i32 + off, env->out.n_agents + off, (size_t)count * sizeof(int32_t),
+                                cudaMemcpyDeviceToHost, stream));
+    return 0;
+}
+
 int ensure_supervisor_stack(mm_env *env) {
     // the supervisors keep 2 x 12 vehicles x 18-point trajectories per thread: a 17 KB frame
     CUDA_OK(cudaSetDevice(env->device));
     size_t stack = 0;
     CUDA_OK(cudaDeviceGetLimit(&stack, cudaLimitStackSize));
     if (stack < 32768) CUDA_OK(cudaDeviceSetLimit(cudaLimitStackSize, 32768));
-    if (!env->sup_tasks) {
-        const size_t E_pad = ((size_t)env->n_envs + TILE - 1) / TILE * TILE;
-        void *p = nullptr;
-        CUDA_OK(cudaMalloc(&p, E_pad * MM_SUP_TASKS_PER_ENV * supervisor_task_bytes()));
-        env->allocs.push_back(p);
-        env->sup_tasks = p;
-        CUDA_OK(cudaMalloc(&p, (E_pad / TILE + 1) * sizeof(int)));
-        env->allocs.push_back(p);
-        env->sup_task_count = static_cast<int *>(p);
-    }
-    return 0;
+    const size_t E_pad = ((size_t)env->n_envs + TILE - 1) / TILE * TILE;
+    int rc = dev_alloc(env, &env->sup_tasks, E_pad * MM_SUP_TASKS_PER_ENV * supervisor_task_bytes(), false);
+    rc |= dev_alloc(env, &env->sup_task_count, E_pad / TILE + 1, false);
+    return rc;
 }
+
 }  // namespace
 
 extern "C" {
@@ -280,8 +327,7 @@ int mm_create(const mm_config *cfg, int n_envs, int device, int record_diag, mm_
     }
     if (rc) { mm_destroy(env); return rc; }
     if ((rc = reset_stats(env))) { mm_destroy(env); return rc; }
-    env->n_streams = MAX_CHUNKS;
-    for (int i = 0; i < env->n_streams; ++i) {
+    for (int i = 0; i < N_STREAMS; ++i) {
         cudaError_t ce = cudaStreamCreateWithFlags(&env->streams[i], cudaStreamNonBlocking);
         if (ce != cudaSuccess) { mm_destroy(env); return fail(MM_ERR_CUDA, "cudaStreamCreate", ce); }
     }
@@ -299,7 +345,7 @@ int mm_destroy(mm_env *env) {
     if (!env) return 0;
     cudaSetDevice(env->device);
     cudaDeviceSynchronize();
-    for (int i = 0; i < MAX_CHUNKS; ++i)
+    for (int i = 0; i < N_STREAMS; ++i)
         if (env->streams[i]) cudaStreamDestroy(env->streams[i]);
     for (int i = 0; i < MAX_HOST_CHUNKS; ++i)
         if (env->chunk_done[i]) cudaEventDestroy(env->chunk_done[i]);
@@ -371,8 +417,7 @@ int mm_step(mm_env *env, const int8_t *actions_dev, int auto_reset, void *stream
     CUDA_OK(cudaSetDevice(env->device));
     env->last_stream = (cudaStream_t)stream;
     const int8_t *actions = actions_dev ? actions_dev : env->actions;
-    static const bool no_graph = getenv("MM_NO_GRAPH") != nullptr;
-    if (no_graph || env->n_envs > GRAPH_MAX_ENVS) {
+    if (env->n_envs > GRAPH_MAX_ENVS) {
         enqueue_step(env, actions, auto_reset, 0, env->n_envs, (cudaStream_t)stream);
         CUDA_OK(cudaGetLastError());
         return 0;
@@ -423,37 +468,19 @@ int mm_step_host(mm_env *env, const int8_t *actions, int auto_reset, float *obs,
     if (!env) return fail(MM_ERR_ARG, "env is null");
     if (!actions) return fail(MM_ERR_ARG, "actions is null");
     CUDA_OK(cudaSetDevice(env->device));
-    const int E = env->n_envs;
-    // Chunks of ~64 Ki envs (a multiple of the 128-env tile, which also keeps the per-warp statistics rows
-    // disjoint) issued round-robin on 4 streams: chunk k's device-to-host copies run while chunks k+1.. compute.
-    const int chunk_target = host_chunk_target(E);
-    const int n_str = 4;
-    int n_chunks = (E + chunk_target - 1) / chunk_target;
-    if (n_chunks < 1) n_chunks = 1;
-    int chunk = ((E + n_chunks - 1) / n_chunks + 767) / 768 * 768;   // multiple of every supported tile size (32..384)
-    if (int rc = order_after_caller(env, n_str)) return rc;
-    for (int c = 0; c < n_chunks; ++c) {
-        int off = c * chunk;
-        if (off >= E) break;
-        int count = E - off < chunk ? E - off : chunk;
-        cudaStream_t s = env->streams[c % n_str];
-        CUDA_OK(cudaMemcpyAsync(env->actions + (size_t)off * MAXV, actions + (size_t)off * MAXV, (size_t)count * MAXV,
-                                cudaMemcpyHostToDevice, s));
-        enqueue_step(env, env->actions, auto_reset, off, count, s);
+    // Chunks issued round-robin on the compute streams: chunk k's device-to-host copies run while chunks k+1.. compute.
+    const ChunkPlan plan = plan_chunks(env->n_envs, std::numeric_limits<int>::max());
+    if (int rc = order_after_caller(env, HOST_STREAMS)) return rc;
+    for (int c = 0; c < plan.used; ++c) {
+        const int off = plan.off(c), count = plan.count(c);
+        cudaStream_t s = env->streams[c % HOST_STREAMS];
+        if (int rc = enqueue_host_step(env, actions, auto_reset, off, count, s)) return rc;
         if (obs)
             CUDA_OK(cudaMemcpyAsync(obs + (size_t)off * MAXV * NS, env->out.obs + (size_t)off * MAXV * NS,
                                     (size_t)count * MAXV * NS * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (reward)
-            CUDA_OK(cudaMemcpyAsync(reward + off, env->out.reward + off, (size_t)count * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (done)
-            CUDA_OK(cudaMemcpyAsync(done + off, env->out.done + off, (size_t)count, cudaMemcpyDeviceToHost, s));
-        if (regional_rewards)
-            CUDA_OK(cudaMemcpyAsync(regional_rewards + (size_t)off * MAXV, env->out.regional_rewards + (size_t)off * MAXV,
-                                    (size_t)count * MAXV * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (n_agents)
-            CUDA_OK(cudaMemcpyAsync(n_agents + off, env->out.n_agents + off, (size_t)count * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        if (int rc = copy_env_outputs(env, off, count, s, reward, done, regional_rewards, n_agents)) return rc;
     }
-    for (int c = 0; c < n_str; ++c) CUDA_OK(cudaStreamSynchronize(env->streams[c]));
+    for (int c = 0; c < HOST_STREAMS; ++c) CUDA_OK(cudaStreamSynchronize(env->streams[c]));
     CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -464,49 +491,21 @@ int mm_step_host_ragged(mm_env *env, const int8_t *actions, int auto_reset, floa
     if (!actions || !obs_rows || !row_offset) return fail(MM_ERR_ARG, "actions, obs_rows and row_offset are required");
     CUDA_OK(cudaSetDevice(env->device));
     const int E = env->n_envs;
-    if (!env->ragged_ready) {   // first use: staging for the packed rows, offsets, per-chunk counts, events
-        // every piece is kept as soon as it exists, and the block is marked done only when all of them do: a failure
-        // half-way leaves a handle that retries the missing pieces on the next call instead of using null pointers
-        void *p = nullptr;
-        if (!env->row_offset) {
-            CUDA_OK(cudaMalloc(&p, ((size_t)E + 1) * sizeof(int64_t)));
-            env->allocs.push_back(p);
-            env->row_offset = static_cast<int64_t *>(p);
-        }
-        if (!env->rows_stage) {
-            CUDA_OK(cudaMalloc(&p, (size_t)E * MAXV * NS * sizeof(float)));
-            env->allocs.push_back(p);
-            env->rows_stage = static_cast<float *>(p);
-        }
-        if (!env->chunk_rows_dev) {
-            CUDA_OK(cudaMalloc(&p, MAX_HOST_CHUNKS * sizeof(int64_t)));
-            env->allocs.push_back(p);
-            env->chunk_rows_dev = static_cast<int64_t *>(p);
-        }
-        if (!env->chunk_rows_host) {
-            CUDA_OK(cudaHostAlloc(&p, MAX_HOST_CHUNKS * sizeof(int64_t), cudaHostAllocDefault));
-            env->chunk_rows_host = static_cast<int64_t *>(p);
-        }
-        for (int c = 0; c < MAX_HOST_CHUNKS; ++c)
-            if (!env->chunk_done[c]) CUDA_OK(cudaEventCreateWithFlags(&env->chunk_done[c], cudaEventDisableTiming));
-        env->ragged_ready = true;
-    }
-    const int chunk_target = host_chunk_target(E);
-    const int n_str = 4;
-    int n_chunks = (E + chunk_target - 1) / chunk_target;
-    if (n_chunks < 1) n_chunks = 1;
-    if (n_chunks > MAX_HOST_CHUNKS) n_chunks = MAX_HOST_CHUNKS;
-    int chunk = ((E + n_chunks - 1) / n_chunks + 767) / 768 * 768;
-    // Software pipeline over the chunks, n_str deep: a chunk's compute + packing is enqueued on its stream; when its row
-    // count has arrived (one event wait on the host) its packed rows follow on the same stream - exactly that many
+    // staging for the packed rows, offsets, per-chunk counts, events: allocated on first use
+    int err = dev_alloc(env, &env->row_offset, (size_t)E + 1, false);
+    err |= dev_alloc(env, &env->rows_stage, (size_t)E * MAXV * NS, false);
+    err |= dev_alloc(env, &env->chunk_rows_dev, MAX_HOST_CHUNKS, false);
+    err |= host_alloc(&env->chunk_rows_host, MAX_HOST_CHUNKS, false);
+    err |= event_alloc(env->chunk_done, MAX_HOST_CHUNKS);
+    if (err) return err;
+    const ChunkPlan plan = plan_chunks(E, MAX_HOST_CHUNKS);
+    // Software pipeline over the chunks, HOST_STREAMS deep: a chunk's compute + packing is enqueued on its stream; when
+    // its row count has arrived (one event wait on the host) its packed rows follow on the same stream - exactly that many
     // bytes - and only then the stream's next chunk.  The copies of chunk c overlap the compute of chunks c+1..c+3.
     auto enqueue_compute = [&](int c) -> int {
-        const int off = c * chunk;
-        const int count = E - off < chunk ? E - off : chunk;
-        cudaStream_t s = env->streams[c % n_str];
-        CUDA_OK(cudaMemcpyAsync(env->actions + (size_t)off * MAXV, actions + (size_t)off * MAXV, (size_t)count * MAXV,
-                                cudaMemcpyHostToDevice, s));
-        enqueue_step(env, env->actions, auto_reset, off, count, s);
+        const int off = plan.off(c), count = plan.count(c);
+        cudaStream_t s = env->streams[c % HOST_STREAMS];
+        if (int rc = enqueue_host_step(env, actions, auto_reset, off, count, s)) return rc;
         // chunk c packs its rows from row off * MAXV on: offsets are absolute and increasing, dense inside a chunk
         launch_ragged_pack(env->out.obs + (size_t)off * MAXV * NS, env->out.n_agents + off, count, (int64_t)off * MAXV,
                            env->row_offset + off, env->chunk_rows_dev + c, env->rows_stage, s);
@@ -516,9 +515,8 @@ int mm_step_host_ragged(mm_env *env, const int8_t *actions, int auto_reset, floa
         return 0;
     };
     auto enqueue_copies = [&](int c) -> int {
-        const int off = c * chunk;
-        const int count = E - off < chunk ? E - off : chunk;
-        cudaStream_t s = env->streams[c % n_str];
+        const int off = plan.off(c), count = plan.count(c);
+        cudaStream_t s = env->streams[c % HOST_STREAMS];
         CUDA_OK(cudaEventSynchronize(env->chunk_done[c]));
         const int64_t rows = env->chunk_rows_host[c];
         const size_t first = (size_t)off * MAXV * NS;
@@ -526,28 +524,17 @@ int mm_step_host_ragged(mm_env *env, const int8_t *actions, int auto_reset, floa
             CUDA_OK(cudaMemcpyAsync(obs_rows + first, env->rows_stage + first, (size_t)rows * NS * sizeof(float),
                                     cudaMemcpyDeviceToHost, s));
         CUDA_OK(cudaMemcpyAsync(row_offset + off, env->row_offset + off, (size_t)count * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-        if (reward)
-            CUDA_OK(cudaMemcpyAsync(reward + off, env->out.reward + off, (size_t)count * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (done)
-            CUDA_OK(cudaMemcpyAsync(done + off, env->out.done + off, (size_t)count, cudaMemcpyDeviceToHost, s));
-        if (regional_rewards)
-            CUDA_OK(cudaMemcpyAsync(regional_rewards + (size_t)off * MAXV, env->out.regional_rewards + (size_t)off * MAXV,
-                                    (size_t)count * MAXV * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (n_agents)
-            CUDA_OK(cudaMemcpyAsync(n_agents + off, env->out.n_agents + off, (size_t)count * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        return 0;
+        return copy_env_outputs(env, off, count, s, reward, done, regional_rewards, n_agents);
     };
-    int used = 0;
-    while (used < n_chunks && used * chunk < E) ++used;
-    if (int rc = order_after_caller(env, n_str)) return rc;
-    for (int c = 0; c < used && c < n_str; ++c)
+    if (int rc = order_after_caller(env, HOST_STREAMS)) return rc;
+    for (int c = 0; c < plan.used && c < HOST_STREAMS; ++c)
         if (int rc = enqueue_compute(c)) return rc;
-    for (int c = 0; c < used; ++c) {
+    for (int c = 0; c < plan.used; ++c) {
         if (int rc = enqueue_copies(c)) return rc;
-        if (c + n_str < used)
-            if (int rc = enqueue_compute(c + n_str)) return rc;
+        if (c + HOST_STREAMS < plan.used)
+            if (int rc = enqueue_compute(c + HOST_STREAMS)) return rc;
     }
-    for (int c = 0; c < n_str; ++c) CUDA_OK(cudaStreamSynchronize(env->streams[c]));
+    for (int c = 0; c < HOST_STREAMS; ++c) CUDA_OK(cudaStreamSynchronize(env->streams[c]));
     row_offset[E] = (int64_t)E * MAXV;
     CUDA_OK(cudaGetLastError());
     return 0;
@@ -559,62 +546,35 @@ int mm_step_host_packed(mm_env *env, const int8_t *actions, int auto_reset, cons
         return fail(MM_ERR_ARG, "actions, out->veh, out->nbr, out->n_veh and out->n_agents are required");
     CUDA_OK(cudaSetDevice(env->device));
     const int E = env->n_envs;
-    if (!env->packed_ready) {   // first use; pieces are kept as they come, the block completes only when all exist
-        auto grab = [&](void **dst, size_t bytes) -> int {
-            if (*dst) return 0;
-            void *p = nullptr;
-            CUDA_OK(cudaMalloc(&p, bytes));
-            CUDA_OK(cudaMemset(p, 0, bytes));
-            env->allocs.push_back(p);
-            *dst = p;
-            return 0;
-        };
-        int rc = 0;
-        rc |= grab((void **)&env->out.veh, (size_t)E * MAXV * MM_VEH_F32 * sizeof(float));
-        rc |= grab((void **)&env->out.nbr, (size_t)E * MAXV * sizeof(uint16_t));
-        rc |= grab((void **)&env->veh_packed, (size_t)E * MAXV * MM_VEH_F32 * sizeof(float));
-        rc |= grab((void **)&env->nbr_packed, (size_t)E * MAXV * sizeof(uint16_t));
-        rc |= grab((void **)&env->voff, (size_t)E * sizeof(int32_t));
-        rc |= grab((void **)&env->aoff, (size_t)E * sizeof(int32_t));
-        rc |= grab((void **)&env->n_veh_u8, (size_t)E);
-        rc |= grab((void **)&env->n_agents_u8, (size_t)E);
-        rc |= grab((void **)&env->chunk_base_dev, (size_t)(MAX_HOST_CHUNKS + 1) * 2 * sizeof(int64_t));
-        if (rc) return rc;
-        if (!env->chunk_base_host) {
-            void *p = nullptr;
-            // mapped: the scan kernel writes a chunk's totals here itself.  (A small device-to-host memcpy per chunk on
-            // the compute streams sits in the copy engine's queue until its chunk has run - and every data copy issued
-            // later queues behind it: measured, the packed rows then left only after ALL compute had finished.)
-            CUDA_OK(cudaHostAlloc(&p, (size_t)(MAX_HOST_CHUNKS + 1) * 2 * sizeof(int64_t), cudaHostAllocMapped));
-            env->chunk_base_host = static_cast<int64_t *>(p);
-            CUDA_OK(cudaHostGetDevicePointer((void **)&env->chunk_base_host_dev, p, 0));
-            env->chunk_base_host[0] = env->chunk_base_host[1] = 0;
-        }
-        for (int c = 0; c < MAX_HOST_CHUNKS; ++c) {
-            if (!env->chunk_done[c]) CUDA_OK(cudaEventCreateWithFlags(&env->chunk_done[c], cudaEventDisableTiming));
-            if (!env->scan_done[c]) CUDA_OK(cudaEventCreateWithFlags(&env->scan_done[c], cudaEventDisableTiming));
-        }
-        env->packed_ready = true;
-    }
-    const int chunk_target = host_chunk_target(E);
-    static const int n_str = [] { const char *e = getenv("MM_HOST_STREAMS"); int v = e ? atoi(e) : 0; return (v >= 1 && v <= 8) ? v : 4; }();
-    int n_chunks = (E + chunk_target - 1) / chunk_target;
-    if (n_chunks < 1) n_chunks = 1;
-    if (n_chunks > MAX_HOST_CHUNKS) n_chunks = MAX_HOST_CHUNKS;
-    const int chunk = ((E + n_chunks - 1) / n_chunks + 767) / 768 * 768;
-    // Chunks of ~64 Ki envs round-robin on four compute streams; ALL of a step's compute is enqueued up front (a chunk
-    // touches only its own envs and its own range of the packed buffers), so the GPU never waits for the host.  The
-    // packed rows of the batch are dense from the first env to the last: a chunk's scan starts from the totals of the
-    // chunk before it (a device-side chain base[c] -> base[c+1], one event wait between neighbouring chunks' scans).
-    // The host learns a chunk's totals with the chunk's event and then issues exactly-sized copies on a copy stream, in
-    // chunk order, while later chunks compute.
+    // allocated on first use, zero-filled
+    int err = dev_alloc(env, &env->out.veh, (size_t)E * MAXV * MM_VEH_F32);
+    err |= dev_alloc(env, &env->out.nbr, (size_t)E * MAXV);
+    err |= dev_alloc(env, &env->veh_packed, (size_t)E * MAXV * MM_VEH_F32);
+    err |= dev_alloc(env, &env->nbr_packed, (size_t)E * MAXV);
+    err |= dev_alloc(env, &env->voff, (size_t)E);
+    err |= dev_alloc(env, &env->aoff, (size_t)E);
+    err |= dev_alloc(env, &env->n_veh_u8, (size_t)E);
+    err |= dev_alloc(env, &env->n_agents_u8, (size_t)E);
+    err |= dev_alloc(env, &env->chunk_base_dev, (size_t)(MAX_HOST_CHUNKS + 1) * 2);
+    // mapped: the scan kernel writes a chunk's totals here itself.  (A small device-to-host memcpy per chunk on the
+    // compute streams sits in the copy engine's queue until its chunk has run - and every data copy issued later queues
+    // behind it: measured, the packed rows then left only after ALL compute had finished.)  Zero-filled: the chain of
+    // totals starts from chunk_base_host[0..1] = 0.
+    err |= host_alloc(&env->chunk_base_host, (size_t)(MAX_HOST_CHUNKS + 1) * 2, true, &env->chunk_base_host_dev);
+    err |= event_alloc(env->chunk_done, MAX_HOST_CHUNKS);
+    err |= event_alloc(env->scan_done, MAX_HOST_CHUNKS);
+    if (err) return err;
+    const ChunkPlan plan = plan_chunks(E, MAX_HOST_CHUNKS);
+    // Chunks round-robin on the compute streams; ALL of a step's compute is enqueued up front (a chunk touches only its
+    // own envs and its own range of the packed buffers), so the GPU never waits for the host.  The packed rows of the
+    // batch are dense from the first env to the last: a chunk's scan starts from the totals of the chunk before it (a
+    // device-side chain base[c] -> base[c+1], one event wait between neighbouring chunks' scans).  The host learns a
+    // chunk's totals with the chunk's event and then issues exactly-sized copies on a copy stream, in chunk order, while
+    // later chunks compute.
     auto enqueue_compute = [&](int c) -> int {
-        const int off = c * chunk;
-        const int count = E - off < chunk ? E - off : chunk;
-        cudaStream_t s = env->streams[c % n_str];
-        CUDA_OK(cudaMemcpyAsync(env->actions + (size_t)off * MAXV, actions + (size_t)off * MAXV, (size_t)count * MAXV,
-                                cudaMemcpyHostToDevice, s));
-        enqueue_step(env, env->actions, auto_reset, off, count, s);
+        const int off = plan.off(c), count = plan.count(c);
+        cudaStream_t s = env->streams[c % HOST_STREAMS];
+        if (int rc = enqueue_host_step(env, actions, auto_reset, off, count, s)) return rc;
         if (c > 0) CUDA_OK(cudaStreamWaitEvent(s, env->scan_done[c - 1], 0));
         launch_packed_pack(env->st.einfo + off, env->out.n_agents + off, env->out.veh + (size_t)off * MAXV * MM_VEH_F32,
                            env->out.nbr + (size_t)off * MAXV, count, env->chunk_base_dev + 2 * c, env->chunk_base_dev + 2 * (c + 1),
@@ -626,12 +586,9 @@ int mm_step_host_packed(mm_env *env, const int8_t *actions, int auto_reset, cons
         return 0;
     };
     auto enqueue_copies = [&](int c) -> int {
-        const int off = c * chunk;
-        const int count = E - off < chunk ? E - off : chunk;
-        cudaStream_t s = env->streams[n_str + c % n_str];      // copy streams: the compute streams stay busy
+        const int off = plan.off(c), count = plan.count(c);
+        cudaStream_t s = env->streams[HOST_STREAMS + c % HOST_STREAMS];      // copy streams: the compute streams stay busy
         CUDA_OK(cudaEventSynchronize(env->chunk_done[c]));
-        static const bool nocopy = getenv("MM_PACKED_NOCOPY") != nullptr;     // timing experiment: compute + packing only
-        if (nocopy) return 0;
         const int64_t v0 = env->chunk_base_host[2 * c], v1 = env->chunk_base_host[2 * (c + 1)];
         const int64_t a0 = env->chunk_base_host[2 * c + 1], a1 = env->chunk_base_host[2 * (c + 1) + 1];
         if (v1 > v0)
@@ -641,23 +598,14 @@ int mm_step_host_packed(mm_env *env, const int8_t *actions, int auto_reset, cons
             CUDA_OK(cudaMemcpyAsync(out->nbr + a0, env->nbr_packed + a0, (size_t)(a1 - a0) * sizeof(uint16_t), cudaMemcpyDeviceToHost, s));
         CUDA_OK(cudaMemcpyAsync(out->n_veh + off, env->n_veh_u8 + off, (size_t)count, cudaMemcpyDeviceToHost, s));
         CUDA_OK(cudaMemcpyAsync(out->n_agents + off, env->n_agents_u8 + off, (size_t)count, cudaMemcpyDeviceToHost, s));
-        if (out->reward)
-            CUDA_OK(cudaMemcpyAsync(out->reward + off, env->out.reward + off, (size_t)count * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (out->done)
-            CUDA_OK(cudaMemcpyAsync(out->done + off, env->out.done + off, (size_t)count, cudaMemcpyDeviceToHost, s));
-        if (out->regional_rewards)
-            CUDA_OK(cudaMemcpyAsync(out->regional_rewards + (size_t)off * MAXV, env->out.regional_rewards + (size_t)off * MAXV,
-                                    (size_t)count * MAXV * sizeof(float), cudaMemcpyDeviceToHost, s));
-        return 0;
+        return copy_env_outputs(env, off, count, s, out->reward, out->done, out->regional_rewards, nullptr);
     };
-    int used = 0;
-    while (used < n_chunks && used * chunk < E) ++used;
-    if (int rc = order_after_caller(env, 2 * n_str)) return rc;
-    for (int c = 0; c < used; ++c)
+    if (int rc = order_after_caller(env, N_STREAMS)) return rc;
+    for (int c = 0; c < plan.used; ++c)
         if (int rc = enqueue_compute(c)) return rc;
-    for (int c = 0; c < used; ++c)
+    for (int c = 0; c < plan.used; ++c)
         if (int rc = enqueue_copies(c)) return rc;
-    for (int c = 0; c < 2 * n_str; ++c) CUDA_OK(cudaStreamSynchronize(env->streams[c]));
+    for (int c = 0; c < N_STREAMS; ++c) CUDA_OK(cudaStreamSynchronize(env->streams[c]));
     CUDA_OK(cudaGetLastError());
     return 0;
 }

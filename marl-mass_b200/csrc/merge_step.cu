@@ -743,14 +743,12 @@ static bool step_attrs_ready(size_t smem) {
 }
 
 void launch_step_impl(const StepParams &p, bool diag, void *stream) {
-    // MM_EXTRA_SMEM (bytes): occupancy experiment knob - pads the CTA's shared memory to lower the CTAs/SM
-    static const size_t extra = [] { const char *e = getenv("MM_EXTRA_SMEM"); return e ? (size_t)atol(e) : (size_t)0; }();
-    if (!step_attrs_ready(STEP_SMEM + extra)) return;
+    if (!step_attrs_ready(STEP_SMEM)) return;
     int grid = (p.env_count + BLOCK - 1) / BLOCK;
     if (grid <= 0) return;
-    if (diag) step_kernel<true, false><<<grid, BLOCK, STEP_SMEM + extra, (cudaStream_t)stream>>>(p);
-    else if (p.cfg.couple_counts) step_kernel<false, true><<<grid, BLOCK, STEP_SMEM + extra, (cudaStream_t)stream>>>(p);
-    else step_kernel<false, false><<<grid, BLOCK, STEP_SMEM + extra, (cudaStream_t)stream>>>(p);
+    if (diag) step_kernel<true, false><<<grid, BLOCK, STEP_SMEM, (cudaStream_t)stream>>>(p);
+    else if (p.cfg.couple_counts) step_kernel<false, true><<<grid, BLOCK, STEP_SMEM, (cudaStream_t)stream>>>(p);
+    else step_kernel<false, false><<<grid, BLOCK, STEP_SMEM, (cudaStream_t)stream>>>(p);
 }
 
 #ifndef MM_VARIANT_TU

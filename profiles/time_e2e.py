@@ -1,4 +1,4 @@
-"""Host-path timing: python profiles/time_e2e.py [envs] [steps]  (MM_HOST_CHUNK=<envs per chunk> to override the chunking)"""
+"""Host-path timing: python profiles/time_e2e.py [envs] [steps]"""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -32,7 +32,7 @@ for name, call, out in (("packed", env.step_host_packed, env.alloc_host_out(pinn
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     s = env.stats(reset=True)
-    print("%s chunk=%s: %.3f ms/step, %.3e agent-steps/s" % (name, os.environ.get("MM_HOST_CHUNK", "auto"), dt / K * 1e3, s["agent_steps"] / dt))
+    print("%s: %.3f ms/step, %.3e agent-steps/s" % (name, dt / K * 1e3, s["agent_steps"] / dt))
     if name == "packed":
         t0 = time.perf_counter()
         rows, off = env.expand_obs_rows(out)
