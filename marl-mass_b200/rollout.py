@@ -185,16 +185,17 @@ def set_actor_impl(name):
     _lib.check(_lib.lib().mm_set_actor_impl(_ACTOR_IMPLS[name]))
 
 
-_DENSE_CACHE = {}
-
-
 def _split_first_layer(policy):
     """The three first-layer blocks of the state_split network (Model_gi.py:137-176: fc11 over the presence columns,
     fc12 over x / y, fc13 over vx / vy) as ONE 30 -> 160 layer: weight [160][30], zero outside the blocks, bias [160].
-    Cached per module until a parameter changes (torch bumps `_version` on every in-place update)."""
+
+    Kept on the module itself (so it dies with it: a later module that reuses its id and memory starts empty) until a
+    parameter is replaced or changed in place by a torch op (optimizer steps, load_state_dict: torch bumps `_version`).
+    Writes through `.data` and collective writes (dist.broadcast) do not bump `_version`; after such writes call
+    `first_layer_changed(policy)`, as `BatchedMAPPORollout.sync_parameters` does."""
     ps = (policy.fc11.weight, policy.fc11.bias, policy.fc12.weight, policy.fc12.bias, policy.fc13.weight, policy.fc13.bias)
     key = tuple((p.data_ptr(), p._version) for p in ps)
-    hit = _DENSE_CACHE.get(id(policy))
+    hit = policy.__dict__.get("_mm_first_layer")
     if hit is not None and hit[0] == key:
         return hit[1], hit[2]
     h4, h2 = policy.fc11.out_features, policy.fc12.out_features
@@ -203,8 +204,14 @@ def _split_first_layer(policy):
     w[h4:h4 + h2, list(policy.COLS2)] = ps[2].detach().float()
     w[h4 + h2:, list(policy.COLS3)] = ps[4].detach().float()
     b = torch.cat([ps[1].detach().float(), ps[3].detach().float(), ps[5].detach().float()]).contiguous()
-    _DENSE_CACHE[id(policy)] = (key, w, b)
+    policy.__dict__["_mm_first_layer"] = (key, w, b)
     return w, b
+
+
+def first_layer_changed(policy):
+    """Drop the dense first layer `_split_first_layer` keeps on a shared network: required after its parameters were
+    written in a way torch does not count (through `.data`, by a collective); any module is accepted."""
+    policy.__dict__.pop("_mm_first_layer", None)
 
 
 def policy_sample(policy, obs, n_agents=None, seed=0, step=0, want_logp=False, action_mask=None, want_value=False,
@@ -368,9 +375,6 @@ def mappo_gradients(actor, critic, S, A8, G, old_logp, q_target, idx, clip=0.2, 
     return losses[0], losses[1]
 
 
-_FOLD_CACHE = {}
-
-
 def shared_network_gradients(policy, S, A8, G, old_logp, idx, clip=0.2, losses=None):
     """Gradient pass of one MAPPO_GI minibatch (mm_ppo_grads, shared network): writes every parameter's .grad as
     `loss.backward()` of `shared_network_loss` (pairwise=False, critic_loss="mse") would after zero_grad(set_to_none=True).
@@ -381,11 +385,11 @@ def shared_network_gradients(policy, S, A8, G, old_logp, idx, clip=0.2, losses=N
     assert old_logp.numel() == S.shape[0]
     losses = torch.zeros(2, dtype=torch.float32, device=S.device) if losses is None else losses
     dev = S.device
-    hit = _FOLD_CACHE.get(id(policy))
+    hit = policy.__dict__.get("_mm_fold")       # scratch for the dense first layer's gradient, kept on the module
     if hit is None or hit[0].device != dev:
         dense = (torch.empty((160, NS), device=dev), torch.empty(160, device=dev))
         cols = [torch.tensor(c, device=dev) for c in (policy.COLS1, policy.COLS2, policy.COLS3)]
-        hit = _FOLD_CACHE[id(policy)] = dense + (cols,)
+        hit = policy.__dict__["_mm_fold"] = dense + (cols,)
     gw1, gb1, cols = hit
     grads = [gw1, gb1] + [_grad_buffer(p) for p in params[2:]]
     _ppo_grads(kind, params, grads, S, A8, G, old_logp, None, idx, clip, losses)
@@ -517,12 +521,16 @@ class BatchedMAPPORollout(object):
         return dist.get_world_size() if (dist.is_available() and dist.is_initialized()) else 1
 
     def sync_parameters(self, src=0):
-        """Broadcast rank `src`'s networks (call once after construction under torchrun)."""
+        """Broadcast rank `src`'s networks (call once after construction under torchrun).  The broadcast writes the
+        parameters behind torch's back, so the dense first layer kept on a shared network is dropped afterwards; call
+        this also after writing the networks' parameters through `.data` yourself."""
         import torch.distributed as dist
         if self._world() > 1:
             for m in self.networks():
                 for t in list(m.parameters()) + list(m.buffers()):
                     dist.broadcast(t.data, src)
+        for m in self.networks():
+            first_layer_changed(m)
 
     def _allreduce_grads(self, params):
         import torch.distributed as dist

@@ -13,7 +13,10 @@ forward: the fp16 rounding of the backward's dZ operands and the accumulation or
 
 Tolerances: per parameter tensor ||g_cuda - g_ref|| / ||g_ref|| <= 1e-2 against the fp16-operand reference on every
 case and against the fp32 reference on rows from collect(); losses within 1e-3 relative; log-probabilities / Q values of
-the target pass within 2e-2 absolute of the fp32 network.
+the target pass within 2e-2 absolute of the fp32 network.  Against fp32 on returns of reward_scale = 1 and in the later
+minibatches of a real update, 3e-2 per tensor and 1e-2 on the losses: there the kernels stay within 3.4e-3 of the
+fp16-operand reference while the fp32 gap reaches 1.3e-2, so the gap is the fp16 rounding of the forward, which that
+reference models; which part of it is not isolated (leaving out the rows within 1e-2 of a clip bound did not shrink it).  test_gpu_learner_exact.py checks the kernels bit for bit on exactly representable data.
 """
 import copy
 import glob
@@ -28,6 +31,7 @@ from conftest import ROOT
 pytestmark = pytest.mark.gpu
 
 GRAD_TOL = 1e-2
+FP32_WIDE_TOL = 3e-2     # against fp32 after the first minibatch of an update and on large returns (module docstring)
 LOSS_TOL = 1e-3
 FWD_TOL = 2e-2
 CLIP = 0.2
@@ -150,7 +154,7 @@ def _random_rows(rows, seed):
     return S, A8, G
 
 
-def _collected_rows(shared, envs=1024, steps=100):
+def _collected_rows(shared, envs=1024, steps=100, reward_scale=None):
     import torch
     from marl_mass_b200.env import DEFAULT_CONFIG, MergeEnvBatched
     from marl_mass_b200.rollout import BatchedMAPPOGIRollout, BatchedMAPPORollout
@@ -158,6 +162,8 @@ def _collected_rows(shared, envs=1024, steps=100):
     ini = "mass_td3_mixed_srew_shared.ini" if shared else "mass_td3_srew.ini"
     env_cfg, kw, _ = load_ini(os.path.join(ROOT, "examples", ini))
     kw["roll_out_n_steps"] = steps
+    if reward_scale is not None:
+        kw["reward_scale"] = reward_scale
     env = MergeEnvBatched(envs, dict(DEFAULT_CONFIG, **env_cfg), device=0)
     torch.manual_seed(11)
     pol = (BatchedMAPPOGIRollout if shared else BatchedMAPPORollout)(env, seed=5, **kw)
@@ -175,12 +181,12 @@ def _rel(a, b):
     return float((a - b).norm() / max(float(b.norm()), 1e-30))
 
 
-def _check_grads(gc, gt, lc, lt, tag):
+def _check_grads(gc, gt, lc, lt, tag, tol=GRAD_TOL):
     worst = 0.0
     for n in gt:
         e = _rel(gc[n], gt[n])
         worst = max(worst, e)
-        assert e <= GRAD_TOL, (tag, n, e)
+        assert e <= tol, (tag, n, e)
     for x, y in zip(lc, lt):
         assert abs(x - y) <= LOSS_TOL * max(abs(y), 1e-3), (tag, x, y)
     return worst
@@ -202,12 +208,15 @@ def _constants(kind, nets, S, A8, live, seed):
 
 
 @pytest.mark.parametrize("kind", ["mappo", "shared"])
-@pytest.mark.parametrize("source", ["random", "collected"])
+@pytest.mark.parametrize("source", ["random", "collected", "collected_unscaled"])
 @pytest.mark.parametrize("n", [100003, 127, 1])
 def test_gradients_match_torch_autograd(mm, kind, source, n):
     """All parameter tensors (MAPPO actor + critic; the shared network with fc11 / fc12 / fc13 folded back from the dense
     first layer and the value head critic_linear), rows in random order, n not a multiple of 128.
-    Against the fp16-operand reference on every case, against the fp32 reference on rows from collect()."""
+    Against the fp16-operand reference on every case, against the fp32 reference on rows from collect().
+    "collected_unscaled": collect() with reward_scale = 1, returns up to a few hundred (2 (Q - G) and the advantages
+    enter fp16 that large); there the fp32 comparison is held to FP32_WIDE_TOL (on a B200, 1.1e-2 on fc1.weight at
+    n = 100 003), the fp16-operand one to GRAD_TOL."""
     import torch
     if source == "random":
         rows = 200000
@@ -215,8 +224,10 @@ def test_gradients_match_torch_autograd(mm, kind, source, n):
         live = torch.arange(rows, device="cuda")
         nets = _nets(kind, 7)
     else:
-        pol, S, A8, G, live = _collected_rows(kind == "shared")
+        pol, S, A8, G, live = _collected_rows(kind == "shared", reward_scale=1.0 if source == "collected_unscaled" else None)
         nets = (pol.actor, pol.critic) if kind == "mappo" else (pol.policy,)
+        if source == "collected_unscaled":
+            assert float(G[live].abs().max()) > 100.0
     old, q = _constants(kind, nets, S, A8, live, 3)
     torch.manual_seed(n)
     j = live[torch.randperm(live.numel(), device="cuda")[:n]]
@@ -225,9 +236,10 @@ def test_gradients_match_torch_autograd(mm, kind, source, n):
         assert {"net0.fc11.weight", "net0.fc12.weight", "net0.fc13.weight", "net0.critic_linear.weight"} <= set(gc)
     gt, at, ct = _torch_grads(kind, nets, S, A8, G, old, q, j, "fp16")
     _check_grads(gc, gt, (ac, cc), (at, ct), (kind, source, n, "fp16 operands"))
-    if source == "collected":
+    if source != "random":
         gt, at, ct = _torch_grads(kind, nets, S, A8, G, old, q, j)
-        _check_grads(gc, gt, (ac, cc), (at, ct), (kind, source, n, "fp32"))
+        _check_grads(gc, gt, (ac, cc), (at, ct), (kind, source, n, "fp32"),
+                     GRAD_TOL if source == "collected" else FP32_WIDE_TOL)
 
 
 def test_shared_first_layer_gradient_lands_on_the_blocks_only(mm):
@@ -328,7 +340,61 @@ def test_target_pass_matches_the_target_networks_and_gives_ratio_one(mm):
     a_loss, _ = rollout.mappo_gradients(actor, critic, S, A8, G, old, q0, live, CLIP)
     assert float(a_loss) == -1.0
     _, a_loss, _ = rollout.shared_network_gradients(pol, S, A8, G, oldp, live, CLIP)
-    assert math.isfinite(float(a_loss))
+    # r == 1: the surrogate is -mean(G - V), V the value head; against the float64 restatement (fp16 rounding apart)
+    import learner_ref
+    params = {n: p.detach().double().cpu().numpy() for n, p in pol.named_parameters()}
+    S64, A64, G64, live64 = S.cpu().numpy(), A8.cpu().numpy(), G.cpu().numpy(), live.cpu().numpy()
+    t = learner_ref.learner_pass("shared", params, S64, A64, None, None, None, np.arange(rows), CLIP)
+    want = learner_ref.learner_pass("shared", params, S64, A64, G64, t["logp"], None, live64, CLIP)["loss_a"]
+    assert want == pytest.approx(-float(np.mean(G64[live64] - t["v"][live64])), rel=1e-12)
+    assert abs(float(a_loss) - want) <= LOSS_TOL * max(abs(want), 1e-3), (float(a_loss), want)
+
+
+@pytest.mark.parametrize("write", ["torch_op", "data_then_sync"])
+def test_shared_first_layer_follows_parameter_writes(mm, write):
+    """policy_sample, ppo_targets and shared_network_gradients run the shared network's first layer as it is at the
+    call, although the dense 30 -> 160 layer is kept on the module between calls.  "torch_op": the parameters
+    overwritten by an in-place torch op (as optimizer steps and load_state_dict write; torch bumps _version).
+    "data_then_sync": overwritten through .data, which bumps no _version (sync_parameters' broadcast writes this way),
+    then sync_parameters, which drops the kept layer."""
+    import torch
+    from torch import nn
+    from marl_mass_b200 import rollout
+    rows = 5000
+    S, A8, G = _random_rows(rows, 51)
+    live = torch.arange(rows, device="cuda")
+    (pol,), (other,) = _nets("shared", 21), _nets("shared", 22)
+    with torch.no_grad():
+        for p in other.parameters():
+            p.mul_(3.0)                     # log-probabilities far from pol's
+    ro = rollout.BatchedMAPPOGIRollout.__new__(rollout.BatchedMAPPOGIRollout)     # only its networks are used
+    ro.policy, ro.policy_target = pol, _nets("shared", 23)[0]
+    old = rollout.ppo_targets(pol, S, A8, live)
+    rollout.shared_network_gradients(pol, S, A8, G, old, live, CLIP)
+    rollout.policy_sample(pol, S, want_logp=True)
+    if write == "torch_op":
+        with torch.no_grad():
+            for p, q in zip(pol.parameters(), other.parameters()):
+                p.copy_(q)
+    else:
+        versions = [p._version for p in pol.parameters()]
+        for p, q in zip(pol.parameters(), other.parameters()):
+            p.data.copy_(q.data)
+        assert [p._version for p in pol.parameters()] == versions
+        ro.sync_parameters()
+    onehot = nn.functional.one_hot(A8.long(), 5).float()
+    with torch.no_grad():
+        want_all = other(S)
+        want = (want_all * onehot).sum(1)
+    assert float((want - old).abs().max()) > 10 * FWD_TOL      # a stale first layer would show
+    got = rollout.ppo_targets(pol, S, A8, live)
+    assert float((got - want).abs().max()) < FWD_TOL
+    _, logp = rollout.policy_sample(pol, S, want_logp=True)
+    assert float((logp - want_all).abs().max()) < FWD_TOL
+    gc, _, _ = _cuda_grads("shared", (pol,), S, A8, G, got, None, live)
+    gt, _, _ = _torch_grads("shared", (pol,), S, A8, G, got, None, live, "fp16")
+    for n in gt:
+        assert _rel(gc[n], gt[n]) <= GRAD_TOL, (n, _rel(gc[n], gt[n]))
 
 
 @pytest.mark.parametrize("shared", [False, True])
@@ -368,6 +434,68 @@ def test_whole_update_cuda_against_torch(mm, shared):
             continue
         cos = float(torch.dot(dt, dc) / (dt.norm() * dc.norm()))
         assert cos >= 0.99, cos
+
+
+@pytest.mark.parametrize("shared", [False, True])
+def test_every_minibatch_of_a_real_update_matches_autograd(mm, monkeypatch, shared):
+    """update(impl="cuda") on a collect() buffer of the shipped ini, 8 minibatches x 2 epochs: after every gradient pass
+    the kernel's gradients and losses are held against torch autograd on the same rows with the networks as they are at
+    that moment, old_logp / Q_target from the target networks as torch computes them.  From the second minibatch on the
+    networks have left their targets, so ratios leave 1 and clipping acts.
+
+    Against the fp16-operand reference every minibatch meets the collected-rows standard (GRAD_TOL, LOSS_TOL).  Against
+    the fp32 reference, once the networks have left their targets, the fp16 rounding of the forward moves some
+    minibatches past it: on a B200 the worst reached 1.3e-2 on a weight tensor and 5.6e-3 on a loss (not explained by
+    clip decisions: leaving out the rows within 1e-2 of a bound did not shrink it), so that comparison is held to
+    FP32_WIDE_TOL and 10 LOSS_TOL, and its worst values are printed."""
+    import torch
+    from torch import nn
+    from marl_mass_b200 import rollout
+    pol, S, A8, G, live = _collected_rows(shared)
+    kind = "shared" if shared else "mappo"
+    nets = (pol.policy,) if shared else (pol.actor, pol.critic)
+    with torch.no_grad():
+        onehot = nn.functional.one_hot(A8.long(), 5).float()
+        tgt = pol.policy_target if shared else pol.actor_target
+        old = (tgt(S) * onehot).sum(1)
+        q = None if shared else pol.critic_target(S, onehot).squeeze(1)
+    name = "shared_network_gradients" if shared else "mappo_gradients"
+    kernel = getattr(rollout, name)
+    seen = []
+
+    def checked(*args, **kw):
+        out = kernel(*args, **kw)
+        j = args[5 if shared else 7]
+        gc = {n: p.grad.clone() for n, p in _params(nets)}
+        lc = (float(out[1]), float(out[2])) if shared else (float(out[0]), float(out[1]))
+        gt, at, ct = _torch_grads(kind, nets, S, A8, G, old, q, j, "fp16")
+        worst = _check_grads(gc, gt, lc, (at, ct), (kind, len(seen), "fp16"))
+        gt, at, ct = _torch_grads(kind, nets, S, A8, G, old, q, j)
+        worst32 = max(_rel(gc[n], gt[n]) for n in gt)
+        loss32 = max(abs(x - y) / max(abs(y), 1e-3) for x, y in zip(lc, (at, ct)))
+        assert worst32 <= FP32_WIDE_TOL and loss32 <= 10 * LOSS_TOL, (kind, len(seen), worst32, loss32)
+        with torch.no_grad():
+            s, a = S[j], A8[j].long()
+            head = pol.policy(s) if shared else pol.actor(s)
+            r = torch.exp(head.gather(1, a[:, None]).squeeze(1) - old[j])
+            adv = G[j] - (pol.policy(s, out_type="v").squeeze(1) if shared else q[j])
+            clipped = ((r > 1 + CLIP) & (adv > 0)) | ((r < 1 - CLIP) & (adv < 0))
+            seen.append((worst, worst32, loss32, float(((r - 1).abs() > 1e-3).float().mean()), float(clipped.float().mean())))
+        for n, p in _params(nets):
+            p.grad = gc[n]
+        return out
+
+    monkeypatch.setattr(rollout, name, checked)
+    minibatch = live.numel() // 8 + 1
+    torch.manual_seed(17)
+    pol.update(minibatch=minibatch, epochs=2, impl="cuda")
+    assert len(seen) == 16
+    for k, (worst, worst32, loss32, off_one, clipped) in enumerate(seen):
+        print("%s minibatch %2d: worst rel err %.2e (fp16 operands) %.2e (fp32), loss %.1e (fp32); r != 1 on %.4f of rows, "
+              "clipped %.4f" % (kind, k, worst, worst32, loss32, off_one, clipped))
+    assert seen[0][3] == 0.0                                       # the first minibatch runs at the target networks
+    assert all(s[3] > 0.0 for s in seen[1:])                       # afterwards the ratios really left 1
+    assert max(s[4] for s in seen) > 0.0
 
 
 @pytest.mark.parametrize("ini", sorted(glob.glob(os.path.join(ROOT, "examples", "*.ini"))))

@@ -211,11 +211,19 @@ from marl_mass_b200.rollout import ActorCriticNetwork, BatchedMAPPOGIRollout
 torch.manual_seed(100 + rank)
 ro = BatchedMAPPOGIRollout.__new__(BatchedMAPPOGIRollout)
 ro.policy, ro.policy_target = ActorCriticNetwork(), ActorCriticNetwork()
+from marl_mass_b200.rollout import _split_first_layer
+before = _split_first_layer(ro.policy)[0].clone()      # the dense first layer of this rank's own weights, kept
 ro.sync_parameters()
 flat = torch.cat([q.detach().reshape(-1) for m in ro.networks() for q in m.parameters()])
 both = [torch.zeros_like(flat) for _ in range(2)]
 dist.all_gather(both, flat)
 assert torch.equal(both[0], both[1])
+# the broadcast writes behind torch's back (no _version bump): the dense layer must follow rank 0's weights
+w, b = _split_first_layer(ro.policy)
+pol = ro.policy
+for (lo, hi), lin, cols in (((0, 32), pol.fc11, pol.COLS1), ((32, 96), pol.fc12, pol.COLS2), ((96, 160), pol.fc13, pol.COLS3)):
+    assert torch.equal(w[lo:hi][:, list(cols)], lin.weight.detach()) and torch.equal(b[lo:hi], lin.bias.detach())
+assert rank == 0 or not torch.equal(before, w)
 x = torch.randn(16, 30)
 ro.policy(x).sum().backward()
 params = [q for q in ro.policy.parameters() if q.grad is not None]
@@ -233,7 +241,8 @@ print("ok", rank)
 
 def test_stats_all_reduce_world_size_2_gloo(tmp_path):
     """The only collective on the path (SURVEY.md §8e): SUM of the counters, MIN of min_headway; and the learner's
-    parameter broadcast + gradient averaging over the ranks."""
+    parameter broadcast (after which the shared network's dense first layer follows the broadcast weights) + gradient
+    averaging over the ranks."""
     script = tmp_path / "worker.py"
     script.write_text(_WORKER)
     port = str(29500 + os.getpid() % 2000)
