@@ -302,6 +302,43 @@ int mm_ppo_grads(int kind, const float *states, const int8_t *actions, const flo
                  const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
                  const mm_ppo_grads_out *grads, float *losses, void *stream);
 
+/* Optimiser step of the learner on the device: for each group (one network), torch.nn.utils.clip_grad_norm_(params,
+ * max_norm) followed by torch.optim.RMSprop(lr, alpha, eps).step() without momentum, centring or weight decay
+ * (marl/mappo.py:88-90, marl/mappo_gi.py:150-156), in one launch with one CTA per group.  Per group:
+ *   g = grad * grad_scale                      (the data-parallel average: grad_scale = 1.0f / world, the float reciprocal
+ *                                               that torch multiplies by for `grad /= world` on a CUDA tensor)
+ *   total = ||g||_2 over every tensor of the group, summed in a fixed order (optim.cu; deterministic)
+ *   coef = min(1, (1 / (total + 1e-6)) * max_norm), or 1 when max_norm <= 0 (no clipping); g *= coef, written to grad
+ *   square_avg = square_avg * alpha; square_avg = square_avg + (one_minus_alpha * g) * g
+ *   param = param + (-lr) * (g / (sqrt(square_avg) + eps))
+ * each operation rounded on its own, as torch's single-tensor and foreach RMSprop order them.  total (before clipping,
+ * what clip_grad_norm_ returns) goes to total_norm when it is not null.  param, grad, square_avg [numel] f32 and
+ * total_norm, mirror are DEVICE pointers; the tables and mirror_cols are HOST memory, read before the call returns.
+ * Mirror (nullable): the kernel also stores every updated param element i, as (r, c) = (i / mirror_ncols,
+ * i % mirror_ncols), at mirror[r * mirror_ld + mirror_cols[c]]: the dense 30 -> 160 first layer of the shared network
+ * (fc11 / fc12 / fc13 at their rows and columns) stays equal to its blocks without a rebuild.  Arguments are checked
+ * before any CUDA call (MM_ERR_ARG): null pointers, 1 <= n_groups <= MM_OPT_MAX_GROUPS, 1 <= n_tensors <=
+ * MM_OPT_MAX_TENSORS, numel >= 0, and a mirror needs mirror_cols with 1..MM_OPT_MAX_MIRROR_COLS entries in
+ * [0, min(mirror_ld, 256)) and a numel that is a multiple of mirror_ncols. */
+#define MM_OPT_MAX_GROUPS 8
+#define MM_OPT_MAX_TENSORS 16
+#define MM_OPT_MAX_MIRROR_COLS 16
+typedef struct {
+    float *param, *grad, *square_avg;
+    int64_t numel;
+    float *mirror;
+    const int32_t *mirror_cols;
+    int32_t mirror_ncols;
+    int64_t mirror_ld;
+} mm_opt_tensor;
+typedef struct {
+    const mm_opt_tensor *tensors;
+    int32_t n_tensors;
+    float lr, alpha, one_minus_alpha, eps, max_norm, grad_scale;
+    float *total_norm;
+} mm_opt_group;
+int mm_rmsprop_step(const mm_opt_group *groups, int n_groups, void *stream);
+
 /* The step kernel (the physics of a policy step) exists in several builds of one source: generic for 3 CTAs per SM
  * (6 staged fields, 168 registers; the faster one per unit of work), generic for 4 CTAs per SM (4 staged fields, 128
  * registers), and two builds specialised at compile time for all-CAV envs of env id merge-multi-agent-v1 with

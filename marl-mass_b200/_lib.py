@@ -90,6 +90,22 @@ class MMPpoGrads(C.Structure):
 PPO_ACTOR, PPO_CRITIC, PPO_SHARED = 0, 1, 2     # MM_PPO_ACTOR / _CRITIC / _SHARED
 
 
+class MMOptTensor(C.Structure):
+    """mm_opt_tensor: one parameter of an optimiser group (device pointers; mirror_cols is host memory)"""
+    _fields_ = [("param", C.c_void_p), ("grad", C.c_void_p), ("square_avg", C.c_void_p), ("numel", C.c_int64),
+                ("mirror", C.c_void_p), ("mirror_cols", _PI), ("mirror_ncols", C.c_int32), ("mirror_ld", C.c_int64)]
+
+
+class MMOptGroup(C.Structure):
+    """mm_opt_group: one network stepped by mm_rmsprop_step"""
+    _fields_ = [("tensors", C.POINTER(MMOptTensor)), ("n_tensors", C.c_int32)] + \
+               [(k, C.c_float) for k in ("lr", "alpha", "one_minus_alpha", "eps", "max_norm", "grad_scale")] + \
+               [("total_norm", C.c_void_p)]
+
+
+OPT_MAX_GROUPS, OPT_MAX_TENSORS = 8, 16     # MM_OPT_MAX_GROUPS / MM_OPT_MAX_TENSORS
+
+
 class MMError(RuntimeError):
     pass
 
@@ -100,7 +116,7 @@ SUPERVISOR_DRAWS = 32     # MM_SUPERVISOR_DRAWS
 EXPORTS = ("mm_create", "mm_destroy", "mm_set_config", "mm_num_envs", "mm_reset", "mm_step", "mm_step_host",
            "mm_step_host_ragged", "mm_step_host_packed", "mm_expand_obs_rows",
            "mm_buffers_get", "mm_get_state", "mm_set_state", "mm_get_shield_diag", "mm_stats", "mm_shield_qp", "mm_shield_query",
-           "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
+           "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_rmsprop_step", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
            "mm_kernel_launches", "mm_last_error", "mm_version")
 
 
@@ -148,6 +164,7 @@ def lib():
                                  C.c_void_p, C.c_void_p]
     L.mm_ppo_grads.argtypes = [C.c_int] + [C.c_void_p] * 6 + [C.c_int64, C.c_float, C.POINTER(MMPpoNet), C.POINTER(MMPpoGrads),
                                                              C.c_void_p, C.c_void_p]
+    L.mm_rmsprop_step.argtypes = [C.POINTER(MMOptGroup), C.c_int, C.c_void_p]
     L.mm_kernel_launches.argtypes = [h]
     L.mm_kernel_launches.restype = C.c_int64
     L.mm_last_error.restype = C.c_char_p

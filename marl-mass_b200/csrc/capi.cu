@@ -917,4 +917,30 @@ int mm_ppo_grads(int kind, const float *states, const int8_t *actions, const flo
     return 0;
 }
 
+int mm_rmsprop_step(const mm_opt_group *groups, int n_groups, void *stream) {
+    if (!groups) return fail(MM_ERR_ARG, "groups is null");
+    if (n_groups < 1 || n_groups > MM_OPT_MAX_GROUPS) return fail(MM_ERR_ARG, "n_groups must be in 1..MM_OPT_MAX_GROUPS (8)");
+    for (int gi = 0; gi < n_groups; ++gi) {
+        const mm_opt_group &g = groups[gi];
+        if (!g.tensors) return fail(MM_ERR_ARG, "group tensors is null");
+        if (g.n_tensors < 1 || g.n_tensors > MM_OPT_MAX_TENSORS)
+            return fail(MM_ERR_ARG, "n_tensors must be in 1..MM_OPT_MAX_TENSORS (16)");
+        for (int k = 0; k < g.n_tensors; ++k) {
+            const mm_opt_tensor &t = g.tensors[k];
+            if (!t.param || !t.grad || !t.square_avg) return fail(MM_ERR_ARG, "param, grad and square_avg are required");
+            if (t.numel < 0) return fail(MM_ERR_ARG, "numel must be >= 0");
+            if (!t.mirror) continue;
+            if (!t.mirror_cols || t.mirror_ncols < 1 || t.mirror_ncols > MM_OPT_MAX_MIRROR_COLS)
+                return fail(MM_ERR_ARG, "a mirror needs a column map (mirror_cols, 1..16 entries)");
+            if (t.mirror_ld < 1) return fail(MM_ERR_ARG, "mirror_ld must be >= 1");
+            if (t.numel % t.mirror_ncols != 0) return fail(MM_ERR_ARG, "numel must be a multiple of mirror_ncols");
+            for (int c = 0; c < t.mirror_ncols; ++c)
+                if (t.mirror_cols[c] < 0 || t.mirror_cols[c] >= t.mirror_ld || t.mirror_cols[c] > 255)
+                    return fail(MM_ERR_ARG, "mirror_cols must lie in [0, min(mirror_ld, 256))");
+        }
+    }
+    if (launch_rmsprop_step(groups, n_groups, stream)) return fail(MM_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
+    return 0;
+}
+
 }  // extern "C"

@@ -164,6 +164,8 @@ int launch_ppo_targets(int kind, const float *states, const int8_t *actions, con
 int launch_ppo_grads(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
                      const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
                      const mm_ppo_grads_out *grads, float *losses, void *stream);
+// clip_grad_norm_ + RMSprop, one CTA per group (optim.cu); arguments already checked by the C ABI
+int launch_rmsprop_step(const mm_opt_group *groups, int n_groups, void *stream);
 
 // envs [env_offset, env_offset + env_count); draws null: Philox draws keyed (seed, env, episode, step); n_used_out
 // (nullable) [n_envs]: how many draws each env's supervisor consumed

@@ -15,6 +15,7 @@ pass per update and one fused forward + backward per minibatch.
 """
 import ctypes as C
 
+import numpy as np
 import torch
 from torch import nn
 
@@ -185,6 +186,11 @@ def set_actor_impl(name):
     _lib.check(_lib.lib().mm_set_actor_impl(_ACTOR_IMPLS[name]))
 
 
+def _first_layer_key(policy):
+    return tuple((p.data_ptr(), p._version) for p in (policy.fc11.weight, policy.fc11.bias, policy.fc12.weight,
+                                                      policy.fc12.bias, policy.fc13.weight, policy.fc13.bias))
+
+
 def _split_first_layer(policy):
     """The three first-layer blocks of the state_split network (Model_gi.py:137-176: fc11 over the presence columns,
     fc12 over x / y, fc13 over vx / vy) as ONE 30 -> 160 layer: weight [160][30], zero outside the blocks, bias [160].
@@ -192,9 +198,10 @@ def _split_first_layer(policy):
     Kept on the module itself (so it dies with it: a later module that reuses its id and memory starts empty) until a
     parameter is replaced or changed in place by a torch op (optimizer steps, load_state_dict: torch bumps `_version`).
     Writes through `.data` and collective writes (dist.broadcast) do not bump `_version`; after such writes call
-    `first_layer_changed(policy)`, as `BatchedMAPPORollout.sync_parameters` does."""
+    `first_layer_changed(policy)`, as `BatchedMAPPORollout.sync_parameters` does.  A `DeviceRMSprop` given the module
+    as `shared_network` writes the layer it keeps along with the parameters, so it stays valid across device steps."""
     ps = (policy.fc11.weight, policy.fc11.bias, policy.fc12.weight, policy.fc12.bias, policy.fc13.weight, policy.fc13.bias)
-    key = tuple((p.data_ptr(), p._version) for p in ps)
+    key = _first_layer_key(policy)
     hit = policy.__dict__.get("_mm_first_layer")
     if hit is not None and hit[0] == key:
         return hit[1], hit[2]
@@ -402,6 +409,146 @@ def shared_network_gradients(policy, S, A8, G, old_logp, idx, clip=0.2, losses=N
     return losses[0] + losses[1], losses[0], losses[1]
 
 
+# ---- the optimiser step on the device (mm_rmsprop_step): clip_grad_norm_ + RMSprop, one launch for whole networks
+
+_MIRROR_COLS = {}
+
+
+def _mirror_cols(cols):
+    """host int32 column map of a mirror entry (kept alive here: the table points at it)"""
+    if cols not in _MIRROR_COLS:
+        _MIRROR_COLS[cols] = (C.c_int32 * len(cols))(*cols)
+    return _MIRROR_COLS[cols]
+
+
+class DeviceRMSprop(torch.optim.Optimizer):
+    """`torch.nn.utils.clip_grad_norm_(params, max_grad_norm)` followed by `torch.optim.RMSprop(params, lr, alpha, eps)`
+    (no momentum, not centred, no weight decay: the reference's optimiser, mappo.py:88-90, mappo_gi.py:150-156) in one
+    kernel launch (mm_rmsprop_step); `rmsprop_step` steps several of them in one launch.  max_grad_norm None or <= 0:
+    no clipping.  The parameters (one group, at most 16 float32 CUDA tensors on one device) are one network.
+
+    - State: torch.optim.RMSprop's (`step`, `square_avg` per parameter), so the state_dict of either class loads into
+      the other.
+    - Gradients: every `.grad` is a view of one flat buffer, `flat_grad`.  `zero_grad()` zeros it in place and keeps the
+      views (`set_to_none` is ignored); autograd accumulates into them and the learner kernels overwrite them.  A `.grad`
+      replaced from outside is copied back into its view at the next step.
+    - Unlike torch, every parameter is stepped on every call: a parameter whose `.grad` is None counts as a zero gradient
+      (its square_avg decays) where torch would skip it.  Every learner parameter receives a gradient on every minibatch.
+    - After a step, `.grad` holds the clipped gradients (as clip_grad_norm_ leaves them) and `total_norm` [1] the norm
+      before clipping (what clip_grad_norm_ returns), on the device.
+    - shared_network: the ActorCriticNetwork these parameters belong to, if any.  The kernel writes its fc11 / fc12 /
+      fc13 updates into the dense first layer `_split_first_layer` keeps for it as well: device writes do not bump
+      torch's `_version`, so without that the kept layer would go stale."""
+
+    def __init__(self, params, lr, alpha=0.99, eps=1e-8, max_grad_norm=None, momentum=0, centered=False, weight_decay=0,
+                 shared_network=None):
+        if momentum != 0 or centered or weight_decay != 0:
+            raise ValueError("DeviceRMSprop is the reference's RMSprop: momentum, centered and weight_decay are not supported")
+        if not lr >= 0.0 or not eps >= 0.0 or not 0.0 <= alpha <= 1.0:
+            raise ValueError("invalid lr, alpha or eps: %r, %r, %r" % (lr, alpha, eps))
+        super().__init__(params, dict(lr=lr, alpha=alpha, eps=eps, momentum=0, centered=False, weight_decay=0))
+        ps = self.param_groups[0]["params"]
+        if not 1 <= len(ps) <= _lib.OPT_MAX_TENSORS:
+            raise ValueError("DeviceRMSprop steps 1..%d parameter tensors, got %d" % (_lib.OPT_MAX_TENSORS, len(ps)))
+        for p in ps:
+            if not (p.is_cuda and p.dtype == torch.float32 and p.is_contiguous() and p.device == ps[0].device):
+                raise ValueError("DeviceRMSprop needs contiguous float32 CUDA parameters on one device")
+        self.max_grad_norm = 0.0 if max_grad_norm is None else float(max_grad_norm)
+        self.shared_network = shared_network
+        self.flat_grad = torch.zeros(sum(p.numel() for p in ps), device=ps[0].device)
+        self.total_norm = torch.zeros(1, device=ps[0].device)
+        self._views, o = [], 0
+        for p in ps:
+            v = self.flat_grad[o:o + p.numel()].view_as(p)
+            if p.grad is not None:
+                v.copy_(p.grad)
+            p.grad = v
+            self._views.append(v)
+            o += p.numel()
+
+    def add_param_group(self, param_group):
+        if self.param_groups:
+            raise ValueError("DeviceRMSprop holds one parameter group (one network, clipped as a whole)")
+        super().add_param_group(param_group)
+
+    def zero_grad(self, set_to_none=True):
+        """Zero the flat gradient buffer in place; the `.grad` views stay (set_to_none is ignored)."""
+        self.flat_grad.zero_()
+        for p, v in zip(self.param_groups[0]["params"], self._views):
+            p.grad = v
+
+    @torch.no_grad()
+    def step(self, closure=None, grad_divisor=1):
+        """One clip + RMSprop step; grad_divisor: divide the gradients first (the world size after an all-reduce sum of
+        `flat_grad`), rounded as torch's `grad /= grad_divisor` on a CUDA tensor."""
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        rmsprop_step([self], grad_divisor)
+        return loss
+
+    def _mirrors(self):
+        """{param index: (dest pointer, column map, row stride)} of the dense first layer kept for shared_network, when it
+        is current (a stale one is rebuilt from the parameters at its next use)"""
+        net = self.shared_network
+        hit = None if net is None else net.__dict__.get("_mm_first_layer")
+        if hit is None or hit[0] != _first_layer_key(net):
+            return {}
+        w, b = hit[1], hit[2]
+        index = {id(p): k for k, p in enumerate(self.param_groups[0]["params"])}
+        out, row = {}, 0
+        for lin, cols in ((net.fc11, net.COLS1), (net.fc12, net.COLS2), (net.fc13, net.COLS3)):
+            if id(lin.weight) in index:
+                out[index[id(lin.weight)]] = (w.data_ptr() + 4 * row * NS, cols, NS)
+            if id(lin.bias) in index:
+                out[index[id(lin.bias)]] = (b.data_ptr() + 4 * row, (0,), 1)
+            row += lin.out_features
+        return out
+
+    def _table(self, grad_scale):
+        g = self.param_groups[0]
+        if g.get("momentum", 0) != 0 or g.get("centered", False) or g.get("weight_decay", 0) != 0:
+            raise ValueError("DeviceRMSprop is the reference's RMSprop: momentum, centered and weight_decay are not supported")
+        ps = g["params"]
+        mirrors = self._mirrors()
+        tensors = (_lib.MMOptTensor * len(ps))()
+        steps = []
+        for k, (p, v) in enumerate(zip(ps, self._views)):
+            if p.grad is not v:
+                v.copy_(p.grad) if p.grad is not None else v.zero_()
+                p.grad = v
+            st = self.state[p]
+            if "square_avg" not in st:
+                st["step"] = torch.tensor(0.0)
+                st["square_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+            sq = st["square_avg"]
+            assert sq.is_contiguous() and sq.device == p.device and sq.dtype == torch.float32
+            steps.append(st["step"])
+            t = tensors[k]
+            t.param, t.grad, t.square_avg, t.numel = p.data_ptr(), v.data_ptr(), sq.data_ptr(), p.numel()
+            if k in mirrors:
+                dst, cols, ld = mirrors[k]
+                t.mirror, t.mirror_cols, t.mirror_ncols, t.mirror_ld = dst, _mirror_cols(cols), len(cols), ld
+        torch._foreach_add_(steps, 1)
+        # alpha, 1 - alpha (in double, as torch forms it), eps, lr: rounded to float32 as torch rounds these scalars
+        grp = _lib.MMOptGroup(tensors, len(ps), g["lr"], g["alpha"], 1.0 - g["alpha"], g["eps"], self.max_grad_norm,
+                              grad_scale, self.total_norm.data_ptr())
+        return grp, tensors
+
+
+def rmsprop_step(optimizers, grad_divisor=1):
+    """Step several DeviceRMSprop (one network each, on one device) in ONE launch of mm_rmsprop_step on the current
+    stream.  grad_divisor > 1: the gradients are first multiplied by float32(1 / grad_divisor), which is what torch's
+    `grad /= grad_divisor` computes on a CUDA tensor (a division by a CPU scalar runs as a product with its reciprocal)."""
+    if not 1 <= len(optimizers) <= _lib.OPT_MAX_GROUPS:
+        raise ValueError("rmsprop_step steps 1..%d optimisers in one launch" % _lib.OPT_MAX_GROUPS)
+    scale = float(np.float32(1.0) / np.float32(grad_divisor))
+    tables = [o._table(scale) for o in optimizers]
+    groups = (_lib.MMOptGroup * len(tables))(*[t[0] for t in tables])
+    _lib.check(_lib.lib().mm_rmsprop_step(groups, len(tables), _stream()))
+
+
 def _check_record_slots(rows, obs_copy, live_out):
     if obs_copy is not None:
         assert obs_copy.is_cuda and obs_copy.dtype == torch.float32 and obs_copy.is_contiguous() and obs_copy.numel() == rows * NS
@@ -412,11 +559,15 @@ def _check_record_slots(rows, obs_copy, live_out):
 class BatchedMAPPORollout(object):
     def __init__(self, env, actor=None, critic=None, roll_out_n_steps=100, reward_gamma=0.99, reward_scale=20.0,
                  reward_type="regionalR", clip_param=0.2, actor_lr=5e-4, critic_lr=5e-4, max_grad_norm=5.0, seed=0,
-                 fused=True, obs=None, reset_seed=None):
+                 fused=True, obs=None, reset_seed=None, optimizer="torch"):
         """obs: the observation of an env the caller has already reset (train.py resets with a rank-distinct spawn
         seed and hands its first observation over).  Without it the first collect() spawns the scenes itself with
         `reset_seed` (default: derived from `seed`, which the data-parallel driver makes rank-distinct) - never with the
-        env's config seed, which is the same on every rank and would make the shards replicas of one another."""
+        env's config seed, which is the same on every rank and would make the shards replicas of one another.
+        optimizer: "torch" (torch.optim.RMSprop after clip_grad_norm_, the default) or "cuda" (`DeviceRMSprop`: the same
+        step as one launch per minibatch, with either update impl)."""
+        if optimizer not in ("torch", "cuda"):
+            raise ValueError("optimizer must be 'torch' or 'cuda', got %r" % (optimizer,))
         self.env = env
         dev = torch.device("cuda", env.device)
         self.actor = (actor or ActorNetwork()).to(dev)
@@ -428,8 +579,9 @@ class BatchedMAPPORollout(object):
         self.T = int(roll_out_n_steps)
         self.gamma, self.reward_scale, self.reward_type = float(reward_gamma), float(reward_scale), reward_type
         self.clip_param, self.max_grad_norm = clip_param, max_grad_norm
-        self.actor_opt = torch.optim.RMSprop(self.actor.parameters(), lr=actor_lr)   # mappo.py:88-90
-        self.critic_opt = torch.optim.RMSprop(self.critic.parameters(), lr=critic_lr)
+        self.optimizer = optimizer
+        self.actor_opt = self._make_optimizer(self.actor, actor_lr)    # mappo.py:88-90
+        self.critic_opt = self._make_optimizer(self.critic, critic_lr)
         self.dev = dev
         self.obs = obs
         self.reset_seed = (0x5EED0000 + int(seed)) if reset_seed is None else int(reset_seed)
@@ -532,6 +684,29 @@ class BatchedMAPPORollout(object):
         for m in self.networks():
             first_layer_changed(m)
 
+    def _make_optimizer(self, net, lr, shared_network=None):
+        if self.optimizer == "cuda":
+            return DeviceRMSprop(net.parameters(), lr=lr, max_grad_norm=self.max_grad_norm, shared_network=shared_network)
+        return torch.optim.RMSprop(net.parameters(), lr=lr)
+
+    def _optimizer_step(self, opts, nets):
+        """all-reduce (data parallel), clip_grad_norm_ and the RMSprop step of each optimiser in `opts` (nets: their
+        networks): torch ops per network, or with optimizer="cuda" one in-place all-reduce of each flat gradient buffer
+        and ONE mm_rmsprop_step launch for all of them (the division by the world size happens in the kernel)."""
+        if self.optimizer == "cuda":
+            w = self._world()
+            if w > 1:
+                import torch.distributed as dist
+                for o in opts:
+                    dist.all_reduce(o.flat_grad)
+            rmsprop_step(opts, w)
+            return
+        for o, net in zip(opts, nets):
+            params = list(net.parameters())
+            self._allreduce_grads(params)
+            nn.utils.clip_grad_norm_(params, self.max_grad_norm)
+            o.step()
+
     def _allreduce_grads(self, params):
         import torch.distributed as dist
         w = self._world()
@@ -573,14 +748,10 @@ class BatchedMAPPORollout(object):
                                                        S[j], A[j], G[j], self.clip_param)
                 self.actor_opt.zero_grad(set_to_none=True)
                 actor_loss.backward()
-                self._allreduce_grads(list(self.actor.parameters()))
-                nn.utils.clip_grad_norm_(self.actor.parameters(), self.max_grad_norm)
-                self.actor_opt.step()
+                self._optimizer_step([self.actor_opt], [self.actor])
                 self.critic_opt.zero_grad(set_to_none=True)
                 critic_loss.backward()
-                self._allreduce_grads(list(self.critic.parameters()))
-                nn.utils.clip_grad_norm_(self.critic.parameters(), self.max_grad_norm)
-                self.critic_opt.step()
+                self._optimizer_step([self.critic_opt], [self.critic])
                 stats = {"actor_loss": float(actor_loss.detach()), "critic_loss": float(critic_loss.detach()),
                          "samples": int(idx.numel())}
         self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
@@ -606,8 +777,9 @@ class BatchedMAPPORollout(object):
     def _update_cuda(self, minibatch, epochs):
         """`update` with the learner kernels: one target pass (old log-probabilities and Q_target of every live sample,
         the target networks do not change within an update), then per minibatch one gradient pass (mappo_gradients) in
-        place of the two backward passes; all-reduce, gradient clipping and the RMSprop steps are the torch path's.  The
-        losses stay on the device until the one read at the end."""
+        place of the two backward passes; then all-reduce, gradient clipping and the RMSprop steps as in the torch path
+        (with optimizer="cuda" one launch steps both networks).  The losses stay on the device until the one read at the
+        end."""
         idx, S, A8, G = self._learner_batch()
         n_mb = self._minibatch_count(idx, minibatch)
         old_logp = ppo_targets(self.actor_target, S, A8, idx)
@@ -617,12 +789,7 @@ class BatchedMAPPORollout(object):
             perm = idx[torch.randperm(idx.numel(), device=self.dev)]
             for j in torch.tensor_split(perm, n_mb):
                 mappo_gradients(self.actor, self.critic, S, A8, G, old_logp, q_target, j, self.clip_param, losses=losses)
-                self._allreduce_grads(list(self.actor.parameters()))
-                nn.utils.clip_grad_norm_(self.actor.parameters(), self.max_grad_norm)
-                self.actor_opt.step()
-                self._allreduce_grads(list(self.critic.parameters()))
-                nn.utils.clip_grad_norm_(self.critic.parameters(), self.max_grad_norm)
-                self.critic_opt.step()
+                self._optimizer_step([self.actor_opt, self.critic_opt], [self.actor, self.critic])
         a_loss, c_loss = losses.tolist()
         self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
         self.critic_target.load_state_dict(self.critic.state_dict())
@@ -648,7 +815,7 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
         self.policy = net.to(dev)
         self.policy_target = ActorCriticNetwork(NS, NA, hidden_size, 1, state_split=self.policy.state_split).to(dev)
         self.policy_target.load_state_dict(self.policy.state_dict())
-        self.policy_opt = torch.optim.RMSprop(self.policy.parameters(), lr=self.actor_opt.param_groups[0]["lr"])
+        self.policy_opt = self._make_optimizer(self.policy, self.actor_opt.param_groups[0]["lr"], shared_network=self.policy)
         self.actor = self.critic = self.actor_target = self.critic_target = None     # not part of this learner
         self.actor_opt = self.critic_opt = None
 
@@ -702,16 +869,13 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
             import torch.distributed as dist
             dist.all_reduce(n_max, op=dist.ReduceOp.MAX)
         n_mb = max(1, -(-int(n_max) // int(minibatch)))       # same count on every rank
-        params = list(self.policy.parameters())
         for _ in range(epochs):
             perm = idx[torch.randperm(idx.numel(), device=self.dev)]
             for j in torch.tensor_split(perm, n_mb):
                 loss, a_loss, c_loss = shared_network_loss(self.policy, self.policy_target, S[j], A[j], G[j], self.clip_param)
                 self.policy_opt.zero_grad(set_to_none=True)
                 loss.backward()
-                self._allreduce_grads(params)
-                nn.utils.clip_grad_norm_(params, self.max_grad_norm)
-                self.policy_opt.step()
+                self._optimizer_step([self.policy_opt], [self.policy])
                 stats = {"actor_loss": float(a_loss.detach()), "critic_loss": float(c_loss.detach()),
                          "samples": int(idx.numel())}
         self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
@@ -719,19 +883,16 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
 
     def _update_cuda(self, minibatch, epochs):
         """`update` with the learner kernels: one target pass, one gradient pass per minibatch
-        (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step."""
+        (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step (optimizer="cuda": one launch)."""
         idx, S, A8, G = self._learner_batch()
         n_mb = self._minibatch_count(idx, minibatch)
         old_logp = ppo_targets(self.policy_target, S, A8, idx)
         losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
-        params = list(self.policy.parameters())
         for _ in range(epochs):
             perm = idx[torch.randperm(idx.numel(), device=self.dev)]
             for j in torch.tensor_split(perm, n_mb):
                 shared_network_gradients(self.policy, S, A8, G, old_logp, j, self.clip_param, losses=losses)
-                self._allreduce_grads(params)
-                nn.utils.clip_grad_norm_(params, self.max_grad_norm)
-                self.policy_opt.step()
+                self._optimizer_step([self.policy_opt], [self.policy])
         a_loss, c_loss = losses.tolist()
         self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
         return {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}

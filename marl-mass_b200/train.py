@@ -50,8 +50,11 @@ def load_ini(path):
     return env_cfg, rollout_kw, train
 
 
-def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch"):
-    """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`)."""
+def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch",
+          optimizer="torch"):
+    """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`).
+    optimizer: "torch" (clip_grad_norm_ + torch.optim.RMSprop, the default) or "cuda" (`rollout.DeviceRMSprop`: the same
+    step in one launch per minibatch)."""
     import torch
     from . import evaluation as ev
     from .env import DEFAULT_CONFIG, MergeEnvBatched
@@ -78,9 +81,9 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
     obs0, _ = env.reset(seed=mmd.rank_seed(env_cfg["seed"], rank) if world > 1 else env_cfg["seed"])
     if tr.get("shared_network"):
         pol = BatchedMAPPOGIRollout(env, hidden_size=tr.get("critic_hidden_size", 128),
-                                    seed=tr["torch_seed"] + 104729 * rank, obs=obs0, **rollout_kw)
+                                    seed=tr["torch_seed"] + 104729 * rank, obs=obs0, optimizer=optimizer, **rollout_kw)
     else:
-        pol = BatchedMAPPORollout(env, seed=tr["torch_seed"] + 104729 * rank, obs=obs0, **rollout_kw)
+        pol = BatchedMAPPORollout(env, seed=tr["torch_seed"] + 104729 * rank, obs=obs0, optimizer=optimizer, **rollout_kw)
     pol.sync_parameters()
     if rank != 0:
         log = lambda *_: None
@@ -134,8 +137,10 @@ def main():
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--update-impl", choices=("torch", "cuda"), default="torch",
                     help="PPO update: torch autograd or the on-device learner kernels")
+    ap.add_argument("--optimizer", choices=("torch", "cuda"), default="torch",
+                    help="gradient clipping + RMSprop step: torch ops or one device launch per minibatch")
     a = ap.parse_args()
-    train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl)
+    train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl, optimizer=a.optimizer)
 
 
 if __name__ == "__main__":

@@ -1,10 +1,14 @@
 """PPO update time, torch autograd against the learner kernels, on the workload of the recorded training logs:
 python profiles/time_update.py [envs] [repeats]
+python profiles/time_update.py [envs] launches
 
-Per example ini (mass_td3_srew, mass_td3_mixed_srew_shared): one 100-step collect() at 4096 envs, then update() with
-impl="torch" and impl="cuda" alternately from the same saved networks / optimiser state (warm-up first, the device
-synchronised around every timed call), and the gradient pass alone per 2^18-row minibatch with CUDA events.  Prints one
-JSON line per ini with the GPU name and power limit (nvidia-smi, read-only query)."""
+Per example ini (mass_td3_srew, mass_td3_mixed_srew_shared): one 100-step collect() at 4096 envs, then three arms
+alternately from the same saved networks / optimiser state (warm-up first, the device synchronised around every timed
+call): update(impl="torch"), update(impl="cuda") with the torch optimiser, and update(impl="cuda") with the device
+optimiser (optimizer="cuda": clip_grad_norm_ + RMSprop in one launch per minibatch); and the gradient pass alone per
+2^18-row minibatch with CUDA events.  Prints one JSON line per ini with the GPU name and power limit (nvidia-smi,
+read-only query).  With "launches" instead of a repeat count: one update per arm under torch.profiler (a separate run:
+tracing slows the host), and the device activities (kernels, memsets, copies) per update and per minibatch."""
 import copy
 import json
 import os
@@ -22,7 +26,8 @@ from marl_mass_b200.rollout import BatchedMAPPOGIRollout, BatchedMAPPORollout  #
 from marl_mass_b200.train import load_ini  # noqa: E402
 
 E = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
-REPEATS = int(sys.argv[2]) if len(sys.argv) > 2 else 10
+LAUNCHES = len(sys.argv) > 2 and sys.argv[2] == "launches"
+REPEATS = int(sys.argv[2]) if len(sys.argv) > 2 and not LAUNCHES else 10
 MB = 1 << 18
 
 
@@ -42,30 +47,55 @@ def run(ini):
     obs0, _ = env.reset(seed=env_cfg["seed"])
     torch.manual_seed(0)
     shared = tr["shared_network"]
-    pol = BatchedMAPPOGIRollout(env, obs=obs0, **kw) if shared else BatchedMAPPORollout(env, obs=obs0, **kw)
+    cls = BatchedMAPPOGIRollout if shared else BatchedMAPPORollout
+    pol = cls(env, obs=obs0, **kw)
     pol.collect()
     torch.cuda.synchronize()
-    mods = pol.networks()
-    opts = [pol.policy_opt] if shared else [pol.actor_opt, pol.critic_opt]
-    saved = [copy.deepcopy(m.state_dict()) for m in mods], [copy.deepcopy(o.state_dict()) for o in opts]
+    nets = {"policy": copy.deepcopy(pol.policy)} if shared else {"actor": copy.deepcopy(pol.actor),
+                                                                  "critic": copy.deepcopy(pol.critic)}
+    pol_dev = cls(env, obs=obs0, optimizer="cuda", **nets, **kw)     # the same networks, the device optimiser
+    pol_dev.buf = pol.buf
+    arms = {"torch": (pol, "torch"), "cuda": (pol, "cuda"), "cuda_devopt": (pol_dev, "cuda")}
+    saved = {}
+    for p in (pol, pol_dev):
+        opts = [p.policy_opt] if shared else [p.actor_opt, p.critic_opt]
+        saved[id(p)] = (p.networks(), opts, [copy.deepcopy(m.state_dict()) for m in pol.networks()],
+                        [copy.deepcopy(o.state_dict()) for o in opts])
 
-    def timed_update(impl):
-        for m, sd in zip(mods, saved[0]):
+    def timed_update(arm):
+        p, impl = arms[arm]
+        mods, opts, sd_m, sd_o = saved[id(p)]
+        for m, sd in zip(mods, sd_m):
             m.load_state_dict(sd)
-        for o, sd in zip(opts, saved[1]):
-            o.load_state_dict(sd)
+        for o, sd in zip(opts, sd_o):
+            o.load_state_dict(copy.deepcopy(sd))
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        st = pol.update(minibatch=MB, impl=impl)
+        st = p.update(minibatch=MB, impl=impl)
         torch.cuda.synchronize()
         return time.perf_counter() - t0, st
 
-    times = {"torch": [], "cuda": []}
-    for impl in ("torch", "cuda"):
-        timed_update(impl)                       # warm-up
+    n_mb = -(-int(pol.buf["live"].sum()) // MB)
+    if LAUNCHES:
+        from torch.profiler import ProfilerActivity, profile
+        counts = {}
+        for arm in arms:
+            timed_update(arm)                    # warm-up
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                timed_update(arm)
+            n = sum(1 for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA)
+            counts[arm] = {"device_activities": n, "per_minibatch": n / n_mb}
+        name, power = gpu_info()
+        print(json.dumps({"ini": ini, "gpu": name, "power_limit": power, "minibatches": n_mb, "launches": counts}), flush=True)
+        env.close()
+        return
+
+    times = {arm: [] for arm in arms}
+    for arm in arms:
+        timed_update(arm)                        # warm-up
     for _ in range(REPEATS):
-        for impl in ("torch", "cuda"):
-            times[impl].append(timed_update(impl)[0])
+        for arm in arms:
+            times[arm].append(timed_update(arm)[0])
 
     # the gradient pass alone, per 2^18-row minibatch
     b = pol.buf
@@ -97,13 +127,14 @@ def run(ini):
         torch.cuda.synchronize()
         return a.elapsed_time(e) / n
 
-    n_mb = -(-idx.numel() // MB)
     name, power = gpu_info()
     rec = {"ini": ini, "gpu": name, "power_limit": power, "envs": E, "rollout_steps": pol.T, "samples": int(idx.numel()),
            "minibatch": MB, "minibatches": n_mb, "repeats": REPEATS,
            "update_torch_s_median": statistics.median(times["torch"]), "update_cuda_s_median": statistics.median(times["cuda"]),
-           "update_torch_s": times["torch"], "update_cuda_s": times["cuda"],
+           "update_cuda_devopt_s_median": statistics.median(times["cuda_devopt"]),
+           "update_torch_s": times["torch"], "update_cuda_s": times["cuda"], "update_cuda_devopt_s": times["cuda_devopt"],
            "speedup": statistics.median(times["torch"]) / statistics.median(times["cuda"]),
+           "speedup_devopt": statistics.median(times["torch"]) / statistics.median(times["cuda_devopt"]),
            "grad_pass_ms_per_minibatch": events(grad_pass), "target_pass_ms": events(target_pass, 5)}
     env.close()
     print(json.dumps(rec), flush=True)
