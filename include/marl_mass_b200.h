@@ -149,6 +149,42 @@ int mm_num_envs(const mm_env *env);
  * num_cav > 0 pins the CAV count (reset(num_CAV=...)).  mask is a DEVICE pointer.  Writes the first obs. */
 int mm_reset(mm_env *env, uint64_t seed, const uint8_t *mask_dev, int num_cav, void *stream);
 
+/* AbstractEnv.reset(is_training=False, testing_seeds=seeds[e], num_CAV=num_cav[e]) for every env at once: exactly the
+ * reference's scene for each seed, built on the device from its MT19937 draws (numpy's legacy RandomState(seed), as
+ * spawn.py replays it on the host).  The state is what mm_set_state leaves for that scene - every field, einfo, the
+ * episode counters and the spawn seed untouched - and obs / n_agents / action_mask are refreshed as mm_set_state does.
+ * seeds [n_envs] int64 and num_cav [n_envs] int32 (NULL: 0, the count is drawn) are HOST arrays, copied before the call
+ * returns; the work is enqueued on `stream` without synchronisation.  Arguments are checked before any CUDA call
+ * (MM_ERR_ARG): a seed outside [0, 2^32) (where numpy raises ValueError), a num_cav outside 0..11, and a num_cav for
+ * which the reference's spawn would raise or build more than 11 vehicles (that depends on the seed's HDV-count draw). */
+int mm_reset_seeded(mm_env *env, const int64_t *seeds, const int32_t *num_cav, void *stream);
+/* The checks of mm_reset_seeded for n_envs envs of a handle with config cfg, alone: pure host code, no device. */
+int mm_check_seeds(const mm_config *cfg, int n_envs, const int64_t *seeds, const int32_t *num_cav);
+
+/* Episode records of the reference's evaluation protocol (MAPPO.evaluation, marl/mappo.py:255-361; evaluation.evaluation)
+ * kept on the device.  mm_eval_record(env, rec, t) runs after the t-th mm_step(auto_reset = 0) of an evaluation and, for
+ * every env whose active byte is still set: stores the global reward at rewards[e][t]; adds info["average_speed"] and
+ * info["traffic_speed"] (as float64, in step order) to avg_speed_sum / traffic_speed_sum; keeps the minimum of
+ * info["min_headway"] in min_headway (a value replaces it only when smaller); counts steps; with vehicle_speed /
+ * vehicle_position set, stores speed and x of slots 0..n_agents[e]-1 at [e][t][slot] (float64); and when done is set,
+ * records merge_percent and crashed (any of the first n_agents[e] vehicles crashed) and clears active.  n_agents is the
+ * agent count at reset (the caller copies mm_buffers.n_agents after the reset).  The caller initialises the records:
+ * active 1, sums and steps 0, min_headway +inf.  All pointers are DEVICE pointers, enqueued on `stream`.  Checked before
+ * any CUDA call (MM_ERR_ARG): null env / records / required pointers, T >= 1, 0 <= t < T. */
+typedef struct {
+    int32_t T;                          /* step capacity of rewards / vehicle_speed / vehicle_position */
+    const int32_t *n_agents;            /* [n_envs] agents at reset */
+    uint8_t *active;                    /* [n_envs] 1 until the episode's first done */
+    float *rewards;                     /* [n_envs][T] */
+    int32_t *steps;                     /* [n_envs] */
+    double *avg_speed_sum, *traffic_speed_sum;   /* [n_envs] */
+    float *min_headway;                 /* [n_envs] */
+    float *merge_percent;               /* [n_envs] written at done */
+    uint8_t *crashed;                   /* [n_envs] written at done */
+    double *vehicle_speed, *vehicle_position;    /* nullable, [n_envs][T][MM_MAXV] */
+} mm_eval_records;
+int mm_eval_record(mm_env *env, const mm_eval_records *rec, int t, void *stream);
+
 /* MergeEnv.step (merge_env_v1.py:126-166): actions_dev is [n_envs][MM_MAXV] int8 on the device
  * (NULL: use mm_buffers.actions).  auto_reset != 0 re-spawns finished envs after their outputs are written
  * (the obs of a finished env is then the first obs of its next episode, as MAPPO.interact does, mappo.py:133-135). */

@@ -106,6 +106,13 @@ class MMOptGroup(C.Structure):
 OPT_MAX_GROUPS, OPT_MAX_TENSORS = 8, 16     # MM_OPT_MAX_GROUPS / MM_OPT_MAX_TENSORS
 
 
+class MMEvalRecords(C.Structure):
+    """mm_eval_records: the evaluation's per-episode records (device pointers) and their step capacity T"""
+    _fields_ = [("T", C.c_int32)] + [(k, C.c_void_p) for k in ("n_agents", "active", "rewards", "steps", "avg_speed_sum",
+                                                              "traffic_speed_sum", "min_headway", "merge_percent", "crashed",
+                                                              "vehicle_speed", "vehicle_position")]
+
+
 class MMError(RuntimeError):
     pass
 
@@ -117,7 +124,7 @@ EXPORTS = ("mm_create", "mm_destroy", "mm_set_config", "mm_num_envs", "mm_reset"
            "mm_step_host_ragged", "mm_step_host_packed", "mm_expand_obs_rows",
            "mm_buffers_get", "mm_get_state", "mm_set_state", "mm_get_shield_diag", "mm_stats", "mm_shield_qp", "mm_shield_query",
            "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_rmsprop_step", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
-           "mm_kernel_launches", "mm_last_error", "mm_version")
+           "mm_reset_seeded", "mm_check_seeds", "mm_eval_record", "mm_kernel_launches", "mm_last_error", "mm_version")
 
 
 def lib():
@@ -140,6 +147,9 @@ def lib():
     L.mm_num_envs.argtypes = [h]
     L.mm_reset.argtypes = [h, C.c_uint64, C.c_void_p, C.c_int, C.c_void_p]
     L.mm_step.argtypes = [h, C.c_void_p, C.c_int, C.c_void_p]
+    L.mm_reset_seeded.argtypes = [h, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.mm_check_seeds.argtypes = [C.POINTER(MMConfig), C.c_int, C.c_void_p, C.c_void_p]
+    L.mm_eval_record.argtypes = [h, C.POINTER(MMEvalRecords), C.c_int, C.c_void_p]
     L.mm_step_host.argtypes = [h, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.mm_step_host_ragged.argtypes = [h, C.c_void_p, C.c_int] + [C.c_void_p] * 6
     L.mm_step_host_packed.argtypes = [h, C.c_void_p, C.c_int, C.POINTER(MMPackedHost)]

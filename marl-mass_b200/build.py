@@ -15,8 +15,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_build")
 LIB = os.path.join(OUT_DIR, "libmarl_mass_b200.so")
-SOURCES = ["merge_step.cu", "merge_step_occ4.cu", "merge_step_spec_mass.cu", "merge_step_spec_hss.cu", "merge_step_spec_mass4.cu", "merge_step_spec_hss4.cu", "merge_coop.cu", "merge_outputs.cu", "actor_sample.cu", "supervisor.cu", "learner.cu", "optim.cu", "capi.cu"]
+SOURCES = ["merge_step.cu", "merge_step_occ4.cu", "merge_step_spec_mass.cu", "merge_step_spec_hss.cu", "merge_step_spec_mass4.cu", "merge_step_spec_hss4.cu", "merge_coop.cu", "merge_outputs.cu", "actor_sample.cu", "supervisor.cu", "learner.cu", "optim.cu", "eval_record.cu", "capi.cu"]
 HEADERS = [os.path.join(CSRC, "mm_internal.h"), os.path.join(CSRC, "mm_device.cuh"), os.path.join(CSRC, "supervisor_core.h"),
+           os.path.join(CSRC, "spawn_core.h"),
            os.path.join(HERE, "..", "include", "marl_mass_b200.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",

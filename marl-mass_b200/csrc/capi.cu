@@ -13,8 +13,13 @@
 #include <vector>
 
 #include "mm_internal.h"
+#include "spawn_core.h"
 
 using namespace mm;
+
+static_assert(mmspawn::TRAFFIC_CAV == MM_TRAFFIC_CAV && mmspawn::TRAFFIC_MIXED == MM_TRAFFIC_MIXED &&
+              mmspawn::TRAFFIC_AV == MM_TRAFFIC_AV && mmspawn::TRAFFIC_HDV == MM_TRAFFIC_HDV &&
+              mmspawn::KIND_CAV == MM_KIND_CAV && mmspawn::KIND_HDV == MM_KIND_HDV, "spawn_core.h codes");
 
 namespace {
 
@@ -69,6 +74,9 @@ struct mm_env {
     uint8_t *n_veh_u8 = nullptr, *n_agents_u8 = nullptr;
     int64_t *chunk_base_dev = nullptr, *chunk_base_host = nullptr, *chunk_base_host_dev = nullptr;
     cudaEvent_t scan_done[MAX_HOST_CHUNKS]{};
+    // mm_reset_seeded, allocated on first use: the test seeds and num_CAV values of the envs
+    int64_t *seeds = nullptr;
+    int32_t *seed_num_cav = nullptr;
     size_t stats_rows = 0;
     uint64_t seed = 0;
     int64_t launches = 0;
@@ -408,6 +416,72 @@ int mm_reset(mm_env *env, uint64_t seed, const uint8_t *mask_dev, int num_cav, v
     o.obs_mask = mask_dev;
     launch_observe(o, stream);
     env->launches += 2;
+    CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int mm_check_seeds(const mm_config *cfg, int n_envs, const int64_t *seeds, const int32_t *num_cav) {
+    if (int rc = validate(cfg)) return rc;
+    if (n_envs < 1) return fail(MM_ERR_ARG, "n_envs must be >= 1");
+    if (!seeds) return fail(MM_ERR_ARG, "seeds is null");
+    mmspawn::MT19937 mt;
+    for (int e = 0; e < n_envs; ++e) {
+        char buf[200];
+        if (seeds[e] < 0 || seeds[e] > (int64_t)0xffffffffLL) {
+            snprintf(buf, sizeof buf, "seed %lld of env %d: a test seed must lie in [0, 2^32)", (long long)seeds[e], e);
+            return fail(MM_ERR_ARG, buf);
+        }
+        const int c = num_cav ? num_cav[e] : 0;
+        if (c < 0 || c > 11) {
+            snprintf(buf, sizeof buf, "num_CAV %d of env %d must be in 0..11", c, e);
+            return fail(MM_ERR_ARG, buf);
+        }
+        if (!mmspawn::spawn_fits((uint32_t)seeds[e], cfg->traffic_density, c, mt)) {
+            snprintf(buf, sizeof buf, "num_CAV %d of env %d (seed %lld): the reference's spawn raises or builds more than 11 "
+                                      "vehicles at traffic_density %d", c, e, (long long)seeds[e], cfg->traffic_density);
+            return fail(MM_ERR_ARG, buf);
+        }
+    }
+    return 0;
+}
+
+int mm_reset_seeded(mm_env *env, const int64_t *seeds, const int32_t *num_cav, void *stream) {
+    if (!env) return fail(MM_ERR_ARG, "env is null");
+    if (int rc = mm_check_seeds(&env->cfg, env->n_envs, seeds, num_cav)) return rc;
+    CUDA_OK(cudaSetDevice(env->device));
+    const size_t E = (size_t)env->n_envs;
+    int err = dev_alloc(env, &env->seeds, E, false);
+    if (num_cav) err |= dev_alloc(env, &env->seed_num_cav, E, false);
+    if (err) return err;
+    // what mm_set_state concludes from the scenes: every traffic_type but cav puts at least one HDV into every env
+    const bool any_hdv = env->cfg.traffic_type != MM_TRAFFIC_CAV;
+    if (env->hdv_possible != any_hdv) ++env->epoch;
+    env->hdv_possible = any_hdv;
+    env->last_stream = (cudaStream_t)stream;
+    CUDA_OK(cudaMemcpyAsync(env->seeds, seeds, E * sizeof(int64_t), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    if (num_cav)
+        CUDA_OK(cudaMemcpyAsync(env->seed_num_cav, num_cav, E * sizeof(int32_t), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    SeededResetParams r{env->st, env->cfg, env->seeds, num_cav ? env->seed_num_cav : nullptr, env->n_envs};
+    launch_seeded_reset(r, stream);
+    StepParams o = step_params(env, nullptr, 0, env->n_envs);
+    launch_observe(o, stream);
+    env->launches += 2;
+    CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int mm_eval_record(mm_env *env, const mm_eval_records *rec, int t, void *stream) {
+    if (!env) return fail(MM_ERR_ARG, "env is null");
+    if (!rec) return fail(MM_ERR_ARG, "records are null");
+    if (!rec->n_agents || !rec->active || !rec->rewards || !rec->steps || !rec->avg_speed_sum || !rec->traffic_speed_sum ||
+        !rec->min_headway || !rec->merge_percent || !rec->crashed)
+        return fail(MM_ERR_ARG, "mm_eval_record: every record array but vehicle_speed / vehicle_position is required");
+    if (rec->T < 1) return fail(MM_ERR_ARG, "mm_eval_record: T must be >= 1");
+    if (t < 0 || t >= rec->T) return fail(MM_ERR_ARG, "mm_eval_record: t must be in [0, T)");
+    CUDA_OK(cudaSetDevice(env->device));
+    env->last_stream = (cudaStream_t)stream;
+    launch_eval_record(env->st, env->out, env->n_envs, *rec, t, stream);
+    env->launches += 1;
     CUDA_OK(cudaGetLastError());
     return 0;
 }

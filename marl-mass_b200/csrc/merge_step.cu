@@ -24,6 +24,7 @@
 #include <math_constants.h>
 #include <cstdlib>
 #include "mm_internal.h"
+#include "spawn_core.h"
 
 // Other builds of the step kernel: a small translation unit defines one of the macros below and includes this file; the
 // kernel then lives in its own namespace and only its launcher is exported.
@@ -413,6 +414,41 @@ __global__ void __launch_bounds__(BLOCK, MM_MIN_BLOCKS) step_kernel(const __grid
 // ------------------------------------------------------------------------------------------------
 // device-side spawn (merge_env_v1.py:180-211, 265-364; abstract.py:176-199) with Philox4x32-10
 // ------------------------------------------------------------------------------------------------
+// The constructor writes of slot i of the env whose field base is g (Vehicle / ControlledVehicle / MDPLCVehicle /
+// IDMVehicle.__init__ at heading 0): every f64 field cleared, then position, speed, target speed, the IDM timer,
+// min_headway and cos(heading) = 1; returns the flags word.  kind MM_KIND_NONE leaves the slot empty with flags
+// `empty_flags`.  The two spawns differ only in what they leave where the reference has no value: reset_kernel writes
+// min_headway 4.5 into every slot and flags 0 into empty ones, mm_set_state of a spawn.py scene 0 for the HDVs and empty
+// slots and hl_action None (-1 on the host) into empty ones.
+__device__ __forceinline__ uint32_t construct_vehicle(double *g, int i, int kind, double x, double y, double speed,
+                                                      double min_headway, uint32_t empty_flags) {
+    uint32_t f = empty_flags;
+    double tspeed = 0, timer = 0;
+    if (kind != MM_KIND_NONE) {
+        const bool cav = kind == MM_KIND_CAV;
+        int lane = closest_lane(x, y, 0.0);
+        int sidx = 0;
+        if (cav) {
+            sidx = speed_to_index(speed);
+            tspeed = 10.0 + sidx * (30.0 - 10.0) / 4;
+        } else {
+            tspeed = speed;
+            timer = pymod_pos((x + y) * PI, 1.0);  // behavior.py:54
+        }
+        f = (uint32_t)kind | ((uint32_t)lane << FL_LANE_SHIFT) | ((uint32_t)lane << FL_TLANE_SHIFT) |
+            ((uint32_t)sidx << FL_SIDX_SHIFT) | ((uint32_t)A_NONE << FL_HL_SHIFT);
+    }
+    for (int fld = 0; fld < F_COUNT; ++fld) g[(fld * MAXV + i) * TILE] = 0.0;
+    g[(F_X * MAXV + i) * TILE] = x;
+    g[(F_Y * MAXV + i) * TILE] = y;
+    g[(F_V * MAXV + i) * TILE] = speed;
+    g[(F_TSPEED * MAXV + i) * TILE] = tspeed;
+    g[(F_TIMER * MAXV + i) * TILE] = timer;
+    g[(F_MINHW * MAXV + i) * TILE] = min_headway;
+    g[(F_COSH * MAXV + i) * TILE] = 1.0;            // heading 0
+    return f;
+}
+
 __global__ void __launch_bounds__(BLOCK) reset_kernel(const __grid_constant__ ResetParams p) {
     const int local = blockIdx.x * BLOCK + threadIdx.x;
     if (local >= p.env_count) return;
@@ -468,8 +504,8 @@ __global__ void __launch_bounds__(BLOCK) reset_kernel(const __grid_constant__ Re
     int mi = 0, ri = 0;
     double *g = p.st.f64 + f64_index(e, 0, 0);
     for (int i = 0; i < MAXV; ++i) {
-        uint32_t f = 0;
-        double x = 0, y = 0, speed = 0, tspeed = 0, timer = 0;
+        int kind = MM_KIND_NONE;
+        double x = 0, y = 0, speed = 0;
         if (i < n_veh) {
             bool cav = i < n_cav;
             bool on_main = cav ? (i < n_s_c) : (i - n_cav < n_s_h);
@@ -477,29 +513,32 @@ __global__ void __launch_bounds__(BLOCK) reset_kernel(const __grid_constant__ Re
             speed = rng.uniform() * 2 + 25;
             if (on_main) { x = 10.0 + 50.0 * main_slots[mi++] + noise; y = 0.0; }
             else { x = 5.0 + 50.0 * ramp_slots[ri++] + noise; y = 10.5; }
-            int lane = closest_lane(x, y, 0.0);
-            int sidx = 0;
-            if (cav) {
-                sidx = speed_to_index(speed);
-                tspeed = 10.0 + sidx * (30.0 - 10.0) / 4;
-            } else {
-                tspeed = speed;
-                timer = pymod_pos((x + y) * PI, 1.0);  // behavior.py:54
-            }
-            f = (uint32_t)(cav ? MM_KIND_CAV : MM_KIND_HDV) | ((uint32_t)lane << FL_LANE_SHIFT) |
-                ((uint32_t)lane << FL_TLANE_SHIFT) | ((uint32_t)sidx << FL_SIDX_SHIFT) | ((uint32_t)A_NONE << FL_HL_SHIFT);
+            kind = cav ? MM_KIND_CAV : MM_KIND_HDV;
         }
-        for (int fld = 0; fld < F_COUNT; ++fld) g[(fld * MAXV + i) * TILE] = 0.0;
-        g[(F_X * MAXV + i) * TILE] = x;
-        g[(F_Y * MAXV + i) * TILE] = y;
-        g[(F_V * MAXV + i) * TILE] = speed;
-        g[(F_TSPEED * MAXV + i) * TILE] = tspeed;
-        g[(F_TIMER * MAXV + i) * TILE] = timer;
-        g[(F_MINHW * MAXV + i) * TILE] = 180.0 / 40.0;  // safe_controller.py:56
-        g[(F_COSH * MAXV + i) * TILE] = 1.0;            // heading 0
-        p.st.flags[flags_index(e, i)] = f;
+        p.st.flags[flags_index(e, i)] = construct_vehicle(g, i, kind, x, y, speed, 180.0 / 40.0 /* safe_controller.py:56 */, 0u);
     }
     p.st.einfo[e] = (uint32_t)n_veh | ((uint32_t)n_cav << EI_NCAV_SHIFT) | ((uint32_t)n_m_c << EI_NMERGE_SHIFT);
+}
+
+// The reference's own scene for each env's test seed (spawn_core.h: its MT19937 draws), written as mm_set_state leaves
+// the state spawn.spawn_state builds for it: the same f64 fields (cold ones cleared), flags and einfo; the episode
+// counters are not touched (mm_set_state leaves them too).  Arguments checked by mm_reset_seeded: every scene fits.
+__global__ void __launch_bounds__(BLOCK) seeded_reset_kernel(const __grid_constant__ SeededResetParams p) {
+    const int e = blockIdx.x * BLOCK + threadIdx.x;
+    if (e >= p.n_envs) return;
+    mmspawn::MT19937 mt;
+    mmspawn::Scene sc;
+    mmspawn::spawn_scene((uint32_t)p.seeds[e], p.cfg.traffic_density, p.cfg.traffic_type, p.num_cav ? p.num_cav[e] : 0,
+                         sc, mt);
+    double *g = p.st.f64 + f64_index(e, 0, 0);
+    for (int i = 0; i < MAXV; ++i) {
+        const bool live = i < sc.n_veh;
+        const int kind = live ? sc.kind[i] : MM_KIND_NONE;
+        p.st.flags[flags_index(e, i)] = construct_vehicle(g, i, kind, live ? sc.x[i] : 0.0, live ? sc.y[i] : 0.0,
+                                                          live ? sc.speed[i] : 0.0, kind == MM_KIND_CAV ? 180.0 / 40.0 : 0.0,
+                                                          (uint32_t)A_NONE << FL_HL_SHIFT);
+    }
+    p.st.einfo[e] = (uint32_t)sc.n_veh | ((uint32_t)sc.n_cav << EI_NCAV_SHIFT) | ((uint32_t)sc.n_merge << EI_NMERGE_SHIFT);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -803,6 +842,12 @@ void launch_reset(const ResetParams &p, void *stream) {
     int grid = (p.env_count + BLOCK - 1) / BLOCK;
     if (grid <= 0) return;
     reset_kernel<<<grid, BLOCK, 0, (cudaStream_t)stream>>>(p);
+}
+
+void launch_seeded_reset(const SeededResetParams &p, void *stream) {
+    int grid = (p.n_envs + BLOCK - 1) / BLOCK;
+    if (grid <= 0) return;
+    seeded_reset_kernel<<<grid, BLOCK, 0, (cudaStream_t)stream>>>(p);
 }
 
 void launch_pack_state(const DevState &st, int n_envs, const double *f64_em, const int32_t *i32_em,

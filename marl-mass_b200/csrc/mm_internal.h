@@ -103,6 +103,14 @@ struct ResetParams {
     int n_envs, env_offset, env_count, num_cav, use_done;
 };
 
+struct SeededResetParams {
+    DevState st;
+    mm_config cfg;
+    const int64_t *seeds;    // [n_envs] in [0, 2^32), checked by mm_reset_seeded
+    const int32_t *num_cav;  // [n_envs] or null (0: drawn)
+    int n_envs;
+};
+
 // launchers (merge_step.cu)
 int launch_step(const StepParams &p, bool diag, void *stream);   // returns the MM_BUILD_* it launched
 // the same kernel compiled for 4 CTAs per SM (merge_step_occ4.cu): picked when that makes the grid a single wave
@@ -117,6 +125,9 @@ void launch_step_coop(const StepParams &p, bool diag, void *stream);
 unsigned long long step_variant_epoch();   // changes whenever set_step_variant was called
 void set_step_variant(int v);   // 0: automatic, 3 / 4: force the generic 3- or 4-CTAs-per-SM build, 5: automatic without the specialised builds
 void launch_reset(const ResetParams &p, void *stream);
+void launch_seeded_reset(const SeededResetParams &p, void *stream);   // the scenes of spawn.py (spawn_core.h)
+// evaluation records of policy step t (eval_record.cu); arguments already checked by mm_eval_record
+void launch_eval_record(const DevState &st, const DevOut &out, int n_envs, const mm_eval_records &r, int t, void *stream);
 // outputs kernel (merge_outputs.cu): observations, rewards, terminal flags, info scalars and statistics of the policy step
 // the physics kernel has just advanced (with_rewards), or the first observation after a (re)spawn / set_state (!with_rewards,
 // optionally only for envs whose p.obs_mask byte is set)

@@ -196,6 +196,21 @@ class MergeEnvBatched(object):
         v = self.buffers()
         return v["obs"], self.action_mask()
 
+    def reset_from_seeds_device(self, seeds, num_CAV=0, stream=None):
+        """The scenes of `reset_from_seeds`, built on the device (mm_reset_seeded: the reference's MT19937 draws per env,
+        one thread each) and left as `set_state` leaves them; nothing is synchronised.  num_CAV: one value or one per
+        seed.  Unlike `reset_from_seeds` it keeps no `spawn_rngs` (the single-env adapter continues that stream on the
+        host for the supervisors' draws).  Raises MMError, before anything is enqueued, for a seed outside [0, 2^32) or a
+        num_CAV for which the reference's spawn raises or builds more than 11 vehicles."""
+        self._apply_config()
+        seeds = np.ascontiguousarray(seeds, np.int64).reshape(-1)
+        assert len(seeds) == self.n_envs
+        nc = np.ascontiguousarray(np.broadcast_to(np.asarray(num_CAV, np.int32), (self.n_envs,)))
+        _lib.check(self._L.mm_reset_seeded(self._h, C.c_void_p(seeds.ctypes.data),
+                                           C.c_void_p(nc.ctypes.data if nc.any() else 0), self._stream_ptr(stream)))
+        v = self.buffers()
+        return v["obs"], self.action_mask()
+
     def action_mask(self):
         """[E, MAXV, 5] int32.  action_masking False: all ones, as the reference returns (abstract.py:207-209).
         True: `_get_available_actions` per agent (abstract.py:219-240), unpacked from the kernel's bitmask.
@@ -361,6 +376,10 @@ class MergeEnvBatched(object):
         self.set_state(st)
         v = self.buffers()
         return v["obs"], self.action_mask()
+
+    def eval_record(self, records, t, stream=None):
+        """mm_eval_record: the evaluation records (`_lib.MMEvalRecords`) of policy step t, taken on the device."""
+        _lib.check(self._L.mm_eval_record(self._h, C.byref(records), int(t), self._stream_ptr(stream)))
 
     def shield_diag(self):
         E = self.n_envs

@@ -93,3 +93,98 @@ def evaluation(action_fn, config, test_seeds, eval_episodes=None, is_train=True,
                 "min_headway": min_headway, "traffic_speeds": list(traffic_speed / steps),
                 "merge_percents": [float(m) for m in merge_percent]}
     return rewards, ([np.array(x) for x in v_speed], [np.array(x) for x in v_pos]), ext_info
+
+
+def crash_rate_ci95(crashes, episodes):
+    """Two-sided 95 % Clopper-Pearson interval of a binomial rate (crashes out of episodes)."""
+    from scipy.stats import beta
+    k, n = int(crashes), int(episodes)
+    lo = float(beta.ppf(0.025, k, n - k + 1)) if k > 0 else 0.0
+    hi = float(beta.ppf(0.975, k + 1, n - k)) if k < n else 1.0
+    return lo, hi
+
+
+def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, device=0, vehicle_records=False,
+                   batch=1 << 20):
+    """`evaluation` for many test seeds: the same episodes, bit for bit, for the same seeds and action function, with the
+    scenes spawned on the device (`reset_from_seeds_device`) and the records kept there (mm_eval_record) - no host
+    replay, no state copy and no synchronisation inside the step loop.
+
+    action_fn and the num_CAV rule (`eval_num_cav` by episode index when is_train) are `evaluation`'s.  Every batch of at
+    most `batch` envs (the last one, if shorter, on its own handle) runs exactly T = duration * policy_frequency policy
+    steps - every episode has ended by then, which is checked once at the end.  Returns a dict of numpy arrays over the
+    N episodes: rewards [N, T] f32 (0 after the episode's last step), steps [N], avg_speeds / traffic_speeds [N] (the
+    float64 sums over the episode's steps / steps, as `evaluation` forms them), crashed [N] bool, merge_percents [N],
+    min_headway [N] (per episode; `evaluation` reports the minimum over all of them), episode_reward [N] (float64 sum of
+    the row of rewards), n_agents [N] (at reset); with vehicle_records also vehicle_speed / vehicle_position
+    [N, T, 12] f64 (slots below n_agents, steps below steps; 0 elsewhere); and crash_rate with its 95 % Clopper-Pearson
+    interval crash_rate_ci95.  An env's index inside its batch keys the draws of a row-keyed action function (the fused
+    actor) and of the priority / dmc supervisors (Philox keyed by env): with those, results match `evaluation` and do not
+    depend on `batch` as long as all seeds fit in one batch."""
+    import torch
+    from . import _lib
+    seeds = np.asarray([int(s) for s in seeds.split(",")] if isinstance(seeds, str) else seeds, np.int64).reshape(-1)
+    n_ep = len(seeds) if eval_episodes is None else int(eval_episodes)
+    seeds = seeds[:n_ep]
+    batch = int(batch)
+    if n_ep < 1 or batch < 1:
+        raise ValueError("evaluate_seeds needs at least one seed and batch >= 1")
+    dev = torch.device("cuda", device)
+    env = None
+    res = None
+    for b0 in range(0, n_ep, batch):
+        n = min(batch, n_ep - b0)
+        if env is None or env.n_envs != n:
+            if env is not None:
+                env.close()
+            env = MergeEnvBatched(n, config, device=device)
+        T = env.T
+        if res is None:
+            td = env.config["traffic_density"]
+            num_cav = eval_num_cav(np.arange(n_ep), td) if is_train else np.zeros(n_ep, np.int64)
+            res = {"rewards": np.zeros((n_ep, T), np.float32), "steps": np.zeros(n_ep, np.int64),
+                   "avg_speed_sum": np.zeros(n_ep), "traffic_speed_sum": np.zeros(n_ep),
+                   "crashed": np.zeros(n_ep, bool), "merge_percents": np.zeros(n_ep), "min_headway": np.zeros(n_ep),
+                   "n_agents": np.zeros(n_ep, np.int32)}
+            if vehicle_records:
+                res["vehicle_speed"] = np.zeros((n_ep, T, MAXV))
+                res["vehicle_position"] = np.zeros((n_ep, T, MAXV))
+        env.reset_from_seeds_device(seeds[b0:b0 + n], num_CAV=num_cav[b0:b0 + n])
+        n_agents = env.buffers()["n_agents"].clone()
+        rec = {"active": torch.ones(n, dtype=torch.uint8, device=dev), "rewards": torch.zeros((n, T), device=dev),
+               "steps": torch.zeros(n, dtype=torch.int32, device=dev),
+               "avg_speed_sum": torch.zeros(n, dtype=torch.float64, device=dev),
+               "traffic_speed_sum": torch.zeros(n, dtype=torch.float64, device=dev),
+               "min_headway": torch.full((n,), float("inf"), device=dev), "merge_percent": torch.zeros(n, device=dev),
+               "crashed": torch.zeros(n, dtype=torch.uint8, device=dev)}
+        if vehicle_records:
+            rec["vehicle_speed"] = torch.zeros((n, T, MAXV), dtype=torch.float64, device=dev)
+            rec["vehicle_position"] = torch.zeros((n, T, MAXV), dtype=torch.float64, device=dev)
+        records = _lib.MMEvalRecords(T=T, n_agents=n_agents.data_ptr(), **{k: v.data_ptr() for k, v in rec.items()})
+        for t in range(T):
+            a = action_fn(env.obs_view(), n_agents).to(torch.int8)
+            env.step(a)
+            env.eval_record(records, t)
+        if rec["active"].any():     # the one synchronisation of the batch
+            raise RuntimeError("evaluate_seeds: %d episodes of seeds[%d:%d] had not ended after T = %d policy steps"
+                               % (int(rec["active"].sum()), b0, b0 + n, T))
+        sl = slice(b0, b0 + n)
+        res["rewards"][sl] = rec["rewards"].cpu().numpy()
+        res["steps"][sl] = rec["steps"].cpu().numpy()
+        res["avg_speed_sum"][sl] = rec["avg_speed_sum"].cpu().numpy()
+        res["traffic_speed_sum"][sl] = rec["traffic_speed_sum"].cpu().numpy()
+        res["crashed"][sl] = rec["crashed"].cpu().numpy() != 0
+        res["merge_percents"][sl] = rec["merge_percent"].cpu().numpy()
+        res["min_headway"][sl] = rec["min_headway"].cpu().numpy()
+        res["n_agents"][sl] = n_agents.cpu().numpy()
+        if vehicle_records:
+            res["vehicle_speed"][sl] = rec["vehicle_speed"].cpu().numpy()
+            res["vehicle_position"][sl] = rec["vehicle_position"].cpu().numpy()
+    env.close()
+    res["avg_speeds"] = res.pop("avg_speed_sum") / res["steps"]
+    res["traffic_speeds"] = res.pop("traffic_speed_sum") / res["steps"]
+    res["episode_reward"] = res["rewards"].astype(np.float64).sum(axis=1)
+    k = int(res["crashed"].sum())
+    res["crash_rate"] = k / n_ep
+    res["crash_rate_ci95"] = crash_rate_ci95(k, n_ep)
+    return res

@@ -51,10 +51,15 @@ def load_ini(path):
 
 
 def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch",
-          optimizer="torch"):
+          optimizer="torch", eval_seeds=0):
     """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`).
     optimizer: "torch" (clip_grad_norm_ + torch.optim.RMSprop, the default) or "cuda" (`rollout.DeviceRMSprop`: the same
-    step in one launch per minibatch)."""
+    step in one launch per minibatch).
+    eval_seeds: N > 0 also evaluates every eval point on the test seeds 0..N-1 (`evaluation.evaluate_seeds`, the
+    reference's protocol with the scenes spawned and the records kept on the device) and logs the evalN_* keys: episodes,
+    crash_rate with its 95 % Clopper-Pearson interval, mean episode reward, mean average speed, mean merge percent,
+    minimum headway and the wall time in seconds.  Its draws come from a counter of their own, so the other keys are
+    the same with and without it."""
     import torch
     from . import evaluation as ev
     from .env import DEFAULT_CONFIG, MergeEnvBatched
@@ -93,6 +98,11 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
         draws["n"] += 1
         return pol.sample_actions(obs, n_agents, seed=tr["torch_seed"] + 7919, step=draws["n"])
 
+    def act_seeds(obs, n_agents):
+        draws["seeds"] += 1
+        return pol.sample_actions(obs, n_agents, seed=tr["torch_seed"] + 7919, step=draws["seeds"])
+    draws["seeds"] = 0
+
     history = []
     for it in range(iterations):
         t0 = time.perf_counter()
@@ -113,6 +123,14 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
             rec.update({"eval_reward": float(np.mean([np.sum(r) for r in rewards])),       # run_mappo.py:303-306
                         "eval_avg_speed": float(np.mean(info["avg_speeds"])), "eval_crashes": int(np.sum(info["crash_count"])),
                         "eval_min_headway": info["min_headway"], "eval_merge_percent": float(np.mean(info["merge_percents"]))})
+            if eval_seeds > 0:
+                t3 = time.perf_counter()
+                r = ev.evaluate_seeds(act_seeds, env_cfg, np.arange(int(eval_seeds)), device=device)
+                rec.update({"evalN_episodes": int(eval_seeds), "evalN_crash_rate": r["crash_rate"],
+                            "evalN_crash_rate_ci95": list(r["crash_rate_ci95"]),
+                            "evalN_reward": float(np.mean(r["episode_reward"])), "evalN_avg_speed": float(np.mean(r["avg_speeds"])),
+                            "evalN_merge_percent": float(np.mean(r["merge_percents"])),
+                            "evalN_min_headway": float(np.min(r["min_headway"])), "evalN_s": time.perf_counter() - t3})
         if world > 1 and it == iterations - 1:      # the replicas must still hold identical networks
             flat = torch.cat([q.detach().reshape(-1) for m in pol.networks() for q in m.parameters()])
             hi, lo = flat.clone(), flat.clone()
@@ -139,8 +157,11 @@ def main():
                     help="PPO update: torch autograd or the on-device learner kernels")
     ap.add_argument("--optimizer", choices=("torch", "cuda"), default="torch",
                     help="gradient clipping + RMSprop step: torch ops or one device launch per minibatch")
+    ap.add_argument("--eval-seeds", type=int, default=0,
+                    help="N > 0: also evaluate on the test seeds 0..N-1 with the device-side protocol (evalN_* keys)")
     a = ap.parse_args()
-    train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl, optimizer=a.optimizer)
+    train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl, optimizer=a.optimizer,
+          eval_seeds=a.eval_seeds)
 
 
 if __name__ == "__main__":
