@@ -185,6 +185,38 @@ typedef struct {
 } mm_eval_records;
 int mm_eval_record(mm_env *env, const mm_eval_records *rec, int t, void *stream);
 
+/* Shield activity and control profiles of the evaluation's episodes (MDPLCVehicle.log_step, safe_controller.py:187-227:
+ * state_hist / action_hist with safe_diff and safe_status), reduced on the device from the per-sub-step shield record of
+ * a handle created with record_diag.  mm_eval_shield_record(env, rec, t) runs after the t-th mm_step(auto_reset = 0) and
+ * BEFORE mm_eval_record(t) (which clears active at done, so the terminal step is still counted), on every env whose
+ * active byte is set (`active` / `n_agents` are those of the mm_eval_records).  It visits sub-step s = 0, 1, 2 and, in
+ * each, vehicle slot i = 0..MM_MAXV-1, and where the shield ran (ran[e][s][i]) adds 1 to shield_solves, to shield_active
+ * when active != 0, to lane_change_vetoes when is_lc_safe == 0 (the counting rules of mm_stats), to shield_interventions
+ * when safe_acc != nom_acc or safe_steer != nom_steer; adds |safe_acc - nom_acc| (the float64 difference, then its
+ * absolute value: safe_diff["acceleration"]) to acc_correction_sum in that order; and keeps the running maxima of
+ * |safe_acc - nom_acc| and |safe_steer - nom_steer|.  Where a vehicle moved (moved[e][s][i]) and i < n_agents[e], it keeps
+ * the minimum applied acceleration (safe_acc) in min_agent_acc.  The caller initialises the records: counters, sum and
+ * maxima 0, min_agent_acc +inf.
+ * Control profiles: profile_slot (nullable, [n_envs]) maps an env to a profile row k >= 0, or -1 for none; a selected
+ * env copies its three sub-step rows of each non-null profile_* array, [K][3 T][MM_MAXV] at row 3 t + s, verbatim from
+ * the shield record while it is active (rows after its episode keep what the caller wrote).  k is not checked: the
+ * caller builds the map.  All pointers are DEVICE pointers, enqueued on `stream`.  Checked before any CUDA call:
+ * MM_ERR_ARG for null records / env / required pointers, T < 1 or t outside [0, T); MM_ERR_STATE for a handle created
+ * without record_diag. */
+typedef struct {
+    int32_t T;                          /* row capacity of the profiles: 3 T rows per profile */
+    const int32_t *n_agents;            /* [n_envs] agents at reset */
+    const uint8_t *active;              /* [n_envs] the active bytes of the mm_eval_records */
+    int32_t *shield_solves, *shield_active, *lane_change_vetoes, *shield_interventions;     /* [n_envs] */
+    double *acc_correction_sum, *acc_correction_max, *steer_correction_max, *min_agent_acc;  /* [n_envs] */
+    const int32_t *profile_slot;        /* nullable, [n_envs]: -1 or the profile row k */
+    /* nullable, [K][3 T][MM_MAXV] each: the planes of mm_shield_diag_host of the same names */
+    int32_t *profile_moved, *profile_ran, *profile_active, *profile_is_lc_safe, *profile_hl_action, *profile_lane;
+    double *profile_x, *profile_y, *profile_heading, *profile_speed, *profile_min_headway, *profile_safe_acc,
+           *profile_safe_steer, *profile_nom_acc, *profile_nom_steer;
+} mm_eval_shield_records;
+int mm_eval_shield_record(mm_env *env, const mm_eval_shield_records *rec, int t, void *stream);
+
 /* MergeEnv.step (merge_env_v1.py:126-166): actions_dev is [n_envs][MM_MAXV] int8 on the device
  * (NULL: use mm_buffers.actions).  auto_reset != 0 re-spawns finished envs after their outputs are written
  * (the obs of a finished env is then the first obs of its next episode, as MAPPO.interact does, mappo.py:133-135). */

@@ -113,6 +113,18 @@ class MMEvalRecords(C.Structure):
                                                               "vehicle_speed", "vehicle_position")]
 
 
+PROFILE_I = ("moved", "ran", "active", "is_lc_safe", "hl_action", "lane")
+PROFILE_F = ("x", "y", "heading", "speed", "min_headway", "safe_acc", "safe_steer", "nom_acc", "nom_steer")
+SHIELD_COUNTS = ("shield_solves", "shield_active", "lane_change_vetoes", "shield_interventions")
+SHIELD_F64 = ("acc_correction_sum", "acc_correction_max", "steer_correction_max", "min_agent_acc")
+
+
+class MMEvalShieldRecords(C.Structure):
+    """mm_eval_shield_records: per-episode shield records and optional control profiles (device pointers)"""
+    _fields_ = [("T", C.c_int32)] + [(k, C.c_void_p) for k in ("n_agents", "active") + SHIELD_COUNTS + SHIELD_F64 +
+                                     ("profile_slot",) + tuple("profile_" + f for f in PROFILE_I + PROFILE_F)]
+
+
 class MMError(RuntimeError):
     pass
 
@@ -124,7 +136,7 @@ EXPORTS = ("mm_create", "mm_destroy", "mm_set_config", "mm_num_envs", "mm_reset"
            "mm_step_host_ragged", "mm_step_host_packed", "mm_expand_obs_rows",
            "mm_buffers_get", "mm_get_state", "mm_set_state", "mm_get_shield_diag", "mm_stats", "mm_shield_qp", "mm_shield_query",
            "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_rmsprop_step", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
-           "mm_reset_seeded", "mm_check_seeds", "mm_eval_record", "mm_kernel_launches", "mm_last_error", "mm_version")
+           "mm_reset_seeded", "mm_check_seeds", "mm_eval_record", "mm_eval_shield_record", "mm_kernel_launches", "mm_last_error", "mm_version")
 
 
 def lib():
@@ -150,6 +162,7 @@ def lib():
     L.mm_reset_seeded.argtypes = [h, C.c_void_p, C.c_void_p, C.c_void_p]
     L.mm_check_seeds.argtypes = [C.POINTER(MMConfig), C.c_int, C.c_void_p, C.c_void_p]
     L.mm_eval_record.argtypes = [h, C.POINTER(MMEvalRecords), C.c_int, C.c_void_p]
+    L.mm_eval_shield_record.argtypes = [h, C.POINTER(MMEvalShieldRecords), C.c_int, C.c_void_p]
     L.mm_step_host.argtypes = [h, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.mm_step_host_ragged.argtypes = [h, C.c_void_p, C.c_int] + [C.c_void_p] * 6
     L.mm_step_host_packed.argtypes = [h, C.c_void_p, C.c_int, C.POINTER(MMPackedHost)]

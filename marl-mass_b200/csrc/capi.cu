@@ -486,6 +486,25 @@ int mm_eval_record(mm_env *env, const mm_eval_records *rec, int t, void *stream)
     return 0;
 }
 
+int mm_eval_shield_record(mm_env *env, const mm_eval_shield_records *rec, int t, void *stream) {
+    // the records first, so that a null handle can stand in for one in a test without a device
+    if (!rec) return fail(MM_ERR_ARG, "records are null");
+    if (!rec->n_agents || !rec->active || !rec->shield_solves || !rec->shield_active || !rec->lane_change_vetoes ||
+        !rec->shield_interventions || !rec->acc_correction_sum || !rec->acc_correction_max || !rec->steer_correction_max ||
+        !rec->min_agent_acc)
+        return fail(MM_ERR_ARG, "mm_eval_shield_record: every record array but profile_slot / profile_* is required");
+    if (rec->T < 1) return fail(MM_ERR_ARG, "mm_eval_shield_record: T must be >= 1");
+    if (t < 0 || t >= rec->T) return fail(MM_ERR_ARG, "mm_eval_shield_record: t must be in [0, T)");
+    if (!env) return fail(MM_ERR_ARG, "env is null");
+    if (!env->record_diag) return fail(MM_ERR_STATE, "handle was created without record_diag");
+    CUDA_OK(cudaSetDevice(env->device));
+    env->last_stream = (cudaStream_t)stream;
+    launch_eval_shield_record(env->out, env->n_envs, *rec, t, stream);
+    env->launches += 1;
+    CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
 int mm_step(mm_env *env, const int8_t *actions_dev, int auto_reset, void *stream) {
     if (!env) return fail(MM_ERR_ARG, "env is null");
     CUDA_OK(cudaSetDevice(env->device));

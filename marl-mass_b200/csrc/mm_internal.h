@@ -128,6 +128,9 @@ void launch_reset(const ResetParams &p, void *stream);
 void launch_seeded_reset(const SeededResetParams &p, void *stream);   // the scenes of spawn.py (spawn_core.h)
 // evaluation records of policy step t (eval_record.cu); arguments already checked by mm_eval_record
 void launch_eval_record(const DevState &st, const DevOut &out, int n_envs, const mm_eval_records &r, int t, void *stream);
+// shield records and control profiles of policy step t from the diagnostic record (eval_record.cu); checked by
+// mm_eval_shield_record
+void launch_eval_shield_record(const DevOut &out, int n_envs, const mm_eval_shield_records &r, int t, void *stream);
 // outputs kernel (merge_outputs.cu): observations, rewards, terminal flags, info scalars and statistics of the policy step
 // the physics kernel has just advanced (with_rewards), or the first observation after a (re)spawn / set_state (!with_rewards,
 // optionally only for envs whose p.obs_mask byte is set)

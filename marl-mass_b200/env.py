@@ -381,6 +381,11 @@ class MergeEnvBatched(object):
         """mm_eval_record: the evaluation records (`_lib.MMEvalRecords`) of policy step t, taken on the device."""
         _lib.check(self._L.mm_eval_record(self._h, C.byref(records), int(t), self._stream_ptr(stream)))
 
+    def eval_shield_record(self, records, t, stream=None):
+        """mm_eval_shield_record: the shield records and control profiles (`_lib.MMEvalShieldRecords`) of policy step t,
+        reduced on the device from the diagnostic record (needs record_diag).  Call it before `eval_record(t)`."""
+        _lib.check(self._L.mm_eval_shield_record(self._h, C.byref(records), int(t), self._stream_ptr(stream)))
+
     def shield_diag(self):
         E = self.n_envs
         d = {k: np.zeros((E, 3, MAXV), np.int32) for k in SH_I}

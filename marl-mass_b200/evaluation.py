@@ -7,6 +7,7 @@ The reference runs `eval_episodes` episodes one after the other on `env_eval`, e
 own for those seeds (host replay of its MT19937 draws, `spawn.py`), all envs step together until the last one is
 done, and each env's records stop at its own terminal step.  Same return structure, same keys.
 """
+import operator
 import time
 
 import numpy as np
@@ -105,7 +106,7 @@ def crash_rate_ci95(crashes, episodes):
 
 
 def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, device=0, vehicle_records=False,
-                   batch=1 << 20):
+                   batch=1 << 20, shield_records=False, control_profiles=None):
     """`evaluation` for many test seeds: the same episodes, bit for bit, for the same seeds and action function, with the
     scenes spawned on the device (`reset_from_seeds_device`) and the records kept there (mm_eval_record) - no host
     replay, no state copy and no synchronisation inside the step loop.
@@ -120,7 +121,18 @@ def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, 
     [N, T, 12] f64 (slots below n_agents, steps below steps; 0 elsewhere); and crash_rate with its 95 % Clopper-Pearson
     interval crash_rate_ci95.  An env's index inside its batch keys the draws of a row-keyed action function (the fused
     actor) and of the priority / dmc supervisors (Philox keyed by env): with those, results match `evaluation` and do not
-    depend on `batch` as long as all seeds fit in one batch."""
+    depend on `batch` as long as all seeds fit in one batch.
+
+    shield_records / control_profiles (a sequence of K distinct episode indices into the seeds) run the batches on handles
+    with the shield's diagnostic record (record_diag) and reduce it on the device after every step
+    (mm_eval_shield_record).  shield_records adds, per episode: shield_solves, shield_active, shield_interventions,
+    lane_change_vetoes [N] int64 and acc_correction_sum, acc_correction_max, steer_correction_max (|safe - nominal| of
+    the shielded actions) and min_agent_acc (the hardest applied acceleration of a controlled vehicle, +inf if none
+    moved) [N] f64, and intervention_rate (interventions over solves, 0 without solves).  control_profiles adds
+    control_profile_episodes [K] and control_profiles, a dict of the per-sub-step fields of log_step
+    (safe_controller.py:187-227) - moved, ran, active, is_lc_safe, hl_action, lane (int32) and x, y, heading, speed,
+    min_headway, safe_acc, safe_steer, nom_acc, nom_steer (f64) - each [K, 3 T, 12] with row 3 t + s for sub-step s of
+    policy step t, 0 after the episode."""
     import torch
     from . import _lib
     seeds = np.asarray([int(s) for s in seeds.split(",")] if isinstance(seeds, str) else seeds, np.int64).reshape(-1)
@@ -129,6 +141,14 @@ def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, 
     batch = int(batch)
     if n_ep < 1 or batch < 1:
         raise ValueError("evaluate_seeds needs at least one seed and batch >= 1")
+    profiles = None
+    if control_profiles is not None:
+        profiles = np.array([operator.index(i) for i in control_profiles], np.int64).reshape(-1)
+        if len(np.unique(profiles)) != len(profiles):
+            raise ValueError("evaluate_seeds: control_profiles holds an episode index more than once")
+        if len(profiles) and (profiles.min() < 0 or profiles.max() >= n_ep):
+            raise ValueError("evaluate_seeds: control_profiles must be episode indices in [0, %d)" % n_ep)
+    diag = bool(shield_records) or profiles is not None
     dev = torch.device("cuda", device)
     env = None
     res = None
@@ -137,7 +157,7 @@ def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, 
         if env is None or env.n_envs != n:
             if env is not None:
                 env.close()
-            env = MergeEnvBatched(n, config, device=device)
+            env = MergeEnvBatched(n, config, device=device, record_diag=diag)
         T = env.T
         if res is None:
             td = env.config["traffic_density"]
@@ -149,6 +169,14 @@ def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, 
             if vehicle_records:
                 res["vehicle_speed"] = np.zeros((n_ep, T, MAXV))
                 res["vehicle_position"] = np.zeros((n_ep, T, MAXV))
+            if diag:
+                sh = {k: torch.zeros(n_ep, dtype=torch.int32, device=dev) for k in _lib.SHIELD_COUNTS}
+                sh.update({k: torch.zeros(n_ep, dtype=torch.float64, device=dev) for k in _lib.SHIELD_F64})
+                sh["min_agent_acc"].fill_(float("inf"))
+            if profiles is not None:
+                prof = {k: torch.zeros((len(profiles), 3 * T, MAXV), dtype=torch.int32, device=dev) for k in _lib.PROFILE_I}
+                prof.update({k: torch.zeros((len(profiles), 3 * T, MAXV), dtype=torch.float64, device=dev)
+                             for k in _lib.PROFILE_F})
         env.reset_from_seeds_device(seeds[b0:b0 + n], num_CAV=num_cav[b0:b0 + n])
         n_agents = env.buffers()["n_agents"].clone()
         rec = {"active": torch.ones(n, dtype=torch.uint8, device=dev), "rewards": torch.zeros((n, T), device=dev),
@@ -161,9 +189,21 @@ def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, 
             rec["vehicle_speed"] = torch.zeros((n, T, MAXV), dtype=torch.float64, device=dev)
             rec["vehicle_position"] = torch.zeros((n, T, MAXV), dtype=torch.float64, device=dev)
         records = _lib.MMEvalRecords(T=T, n_agents=n_agents.data_ptr(), **{k: v.data_ptr() for k, v in rec.items()})
+        if diag:
+            ptrs = {k: v[b0:b0 + n].data_ptr() for k, v in sh.items()}
+            if profiles is not None:
+                slot = np.full(n, -1, np.int32)
+                mine = (profiles >= b0) & (profiles < b0 + n)
+                slot[profiles[mine] - b0] = np.nonzero(mine)[0]
+                slot_dev = torch.from_numpy(slot).to(dev)
+                ptrs["profile_slot"] = slot_dev.data_ptr()
+                ptrs.update({"profile_" + k: v.data_ptr() for k, v in prof.items()})
+            sh_records = _lib.MMEvalShieldRecords(T=T, n_agents=n_agents.data_ptr(), active=rec["active"].data_ptr(), **ptrs)
         for t in range(T):
             a = action_fn(env.obs_view(), n_agents).to(torch.int8)
             env.step(a)
+            if diag:
+                env.eval_shield_record(sh_records, t)
             env.eval_record(records, t)
         if rec["active"].any():     # the one synchronisation of the batch
             raise RuntimeError("evaluate_seeds: %d episodes of seeds[%d:%d] had not ended after T = %d policy steps"
@@ -181,6 +221,16 @@ def evaluate_seeds(action_fn, config, seeds, eval_episodes=None, is_train=True, 
             res["vehicle_speed"][sl] = rec["vehicle_speed"].cpu().numpy()
             res["vehicle_position"][sl] = rec["vehicle_position"].cpu().numpy()
     env.close()
+    if shield_records:
+        for k in _lib.SHIELD_COUNTS:
+            res[k] = sh[k].cpu().numpy().astype(np.int64)
+        for k in _lib.SHIELD_F64:
+            res[k] = sh[k].cpu().numpy()
+        solves = int(res["shield_solves"].sum())
+        res["intervention_rate"] = int(res["shield_interventions"].sum()) / solves if solves else 0.0
+    if profiles is not None:
+        res["control_profiles"] = {k: v.cpu().numpy() for k, v in prof.items()}
+        res["control_profile_episodes"] = profiles
     res["avg_speeds"] = res.pop("avg_speed_sum") / res["steps"]
     res["traffic_speeds"] = res.pop("traffic_speed_sum") / res["steps"]
     res["episode_reward"] = res["rewards"].astype(np.float64).sum(axis=1)

@@ -51,7 +51,7 @@ def load_ini(path):
 
 
 def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch",
-          optimizer="torch", eval_seeds=0):
+          optimizer="torch", eval_seeds=0, eval_shield=False):
     """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`).
     optimizer: "torch" (clip_grad_norm_ + torch.optim.RMSprop, the default) or "cuda" (`rollout.DeviceRMSprop`: the same
     step in one launch per minibatch).
@@ -59,7 +59,13 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
     reference's protocol with the scenes spawned and the records kept on the device) and logs the evalN_* keys: episodes,
     crash_rate with its 95 % Clopper-Pearson interval, mean episode reward, mean average speed, mean merge percent,
     minimum headway and the wall time in seconds.  Its draws come from a counter of their own, so the other keys are
-    the same with and without it."""
+    the same with and without it.
+    eval_shield: with eval_seeds, also record the shield's activity on those episodes (`evaluate_seeds(shield_records=True)`)
+    and log evalN_shield_intervention_rate (interventions over QP solves), evalN_lane_change_vetoes_per_episode,
+    evalN_min_agent_acc (the hardest applied acceleration of any controlled vehicle) and evalN_acc_correction_max (the
+    largest |safe - nominal| acceleration)."""
+    if eval_shield and not eval_seeds > 0:
+        raise ValueError("train: eval_shield records the shield on the eval_seeds episodes and needs eval_seeds > 0")
     import torch
     from . import evaluation as ev
     from .env import DEFAULT_CONFIG, MergeEnvBatched
@@ -125,7 +131,12 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
                         "eval_min_headway": info["min_headway"], "eval_merge_percent": float(np.mean(info["merge_percents"]))})
             if eval_seeds > 0:
                 t3 = time.perf_counter()
-                r = ev.evaluate_seeds(act_seeds, env_cfg, np.arange(int(eval_seeds)), device=device)
+                r = ev.evaluate_seeds(act_seeds, env_cfg, np.arange(int(eval_seeds)), device=device, shield_records=eval_shield)
+                if eval_shield:
+                    rec.update({"evalN_shield_intervention_rate": r["intervention_rate"],
+                                "evalN_lane_change_vetoes_per_episode": float(np.mean(r["lane_change_vetoes"])),
+                                "evalN_min_agent_acc": float(np.min(r["min_agent_acc"])),
+                                "evalN_acc_correction_max": float(np.max(r["acc_correction_max"]))})
                 rec.update({"evalN_episodes": int(eval_seeds), "evalN_crash_rate": r["crash_rate"],
                             "evalN_crash_rate_ci95": list(r["crash_rate_ci95"]),
                             "evalN_reward": float(np.mean(r["episode_reward"])), "evalN_avg_speed": float(np.mean(r["avg_speeds"])),
@@ -159,9 +170,11 @@ def main():
                     help="gradient clipping + RMSprop step: torch ops or one device launch per minibatch")
     ap.add_argument("--eval-seeds", type=int, default=0,
                     help="N > 0: also evaluate on the test seeds 0..N-1 with the device-side protocol (evalN_* keys)")
+    ap.add_argument("--eval-shield", action="store_true",
+                    help="with --eval-seeds: also log the shield's interventions, vetoes and corrections (evalN_shield_* keys)")
     a = ap.parse_args()
     train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl, optimizer=a.optimizer,
-          eval_seeds=a.eval_seeds)
+          eval_seeds=a.eval_seeds, eval_shield=a.eval_shield)
 
 
 if __name__ == "__main__":
