@@ -370,6 +370,27 @@ int mm_ppo_grads(int kind, const float *states, const int8_t *actions, const flo
                  const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
                  const mm_ppo_grads_out *grads, float *losses, void *stream);
 
+/* Statistics pass (forward only, the same forward arithmetic as the target and gradient passes): the standard PPO
+ * diagnostics of one network over the n listed rows, reduced into stats[MM_PPO_STATS_LEN] (f64, DEVICE pointer), written
+ * (not accumulated).  Per row, in f32 as the passes compute it:
+ *   ACTOR, SHARED  the entropy -sum_k p_k log p_k of the log-softmax (ENTROPY); with old_logp (nullable) the ratio
+ *                  r = exp(logp(a) - old_logp), k3 = (r - 1) - (logp(a) - old_logp) (K3), |r - 1| > clip (CLIPPED) and the
+ *                  range of r (RATIO_MIN, RATIO_MAX)
+ *   CRITIC, SHARED the value v = Q(s, one_hot(a)) (CRITIC) or V(s) (SHARED) against the return G: v, v^2, G, G^2 and
+ *                  (G - v)^2 (V, V2, G, G2, RES2; v^2, G^2 and (G - v)^2 squared in f64)
+ * N counts the rows.  Sums and counts combine across data-parallel shards with SUM, RATIO_MIN with MIN and RATIO_MAX with
+ * MAX.  Fields a kind has no term for are 0; where no ratio is formed (CRITIC, old_logp null, n = 0) RATIO_MIN = +inf and
+ * RATIO_MAX = -inf.  n = 0 (an empty shard) writes that empty value.  Deterministic: each thread sums its rows in f64 in a
+ * fixed order, each CTA writes one partial per field, a second kernel adds them in CTA order; no float atomics.  The
+ * partials share mm_ppo_grads' workspace, so calls on one device must be ordered with it (one stream).  Arguments are
+ * checked before any CUDA call (MM_ERR_ARG): kind, net, n >= 0, stats, and for n > 0 states, actions, idx and returns
+ * (CRITIC, SHARED); 0 < clip < 1 when old_logp is given. */
+enum { MM_PPO_STAT_N, MM_PPO_STAT_ENTROPY, MM_PPO_STAT_K3, MM_PPO_STAT_CLIPPED, MM_PPO_STAT_RATIO_MIN,
+       MM_PPO_STAT_RATIO_MAX, MM_PPO_STAT_V, MM_PPO_STAT_V2, MM_PPO_STAT_G, MM_PPO_STAT_G2, MM_PPO_STAT_RES2,
+       MM_PPO_STATS_LEN };
+int mm_ppo_stats(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                 const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net, double *stats, void *stream);
+
 /* Optimiser step of the learner on the device: for each group (one network), torch.nn.utils.clip_grad_norm_(params,
  * max_norm) followed by torch.optim.RMSprop(lr, alpha, eps).step() without momentum, centring or weight decay
  * (marl/mappo.py:88-90, marl/mappo_gi.py:150-156), in one launch with one CTA per group.  Per group:

@@ -1010,6 +1010,19 @@ int mm_ppo_grads(int kind, const float *states, const int8_t *actions, const flo
     return 0;
 }
 
+int mm_ppo_stats(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                 const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net, double *stats, void *stream) {
+    if (int rc = check_ppo_net(kind, net)) return rc;
+    if (n < 0) return fail(MM_ERR_ARG, "n must be >= 0");
+    if (!stats) return fail(MM_ERR_ARG, "stats is required");
+    if (n > 0 && (!states || !actions || !idx)) return fail(MM_ERR_ARG, "states, actions and idx are required");
+    if (n > 0 && kind != MM_PPO_ACTOR && !returns) return fail(MM_ERR_ARG, "returns are required for the value statistics");
+    if (old_logp && !(clip > 0.f && clip < 1.f)) return fail(MM_ERR_ARG, "clip must be in (0, 1)");
+    if (launch_ppo_stats(kind, states, actions, returns, old_logp, idx, n, clip, net, stats, stream))
+        return fail(MM_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
+    return 0;
+}
+
 int mm_rmsprop_step(const mm_opt_group *groups, int n_groups, void *stream) {
     if (!groups) return fail(MM_ERR_ARG, "groups is null");
     if (n_groups < 1 || n_groups > MM_OPT_MAX_GROUPS) return fail(MM_ERR_ARG, "n_groups must be in 1..MM_OPT_MAX_GROUPS (8)");

@@ -10,7 +10,10 @@
 //     forward with the same code as the target pass (so r == 1 exactly where the network equals its target), the per-row
 //     loss derivative and the backward, and accumulates the weight gradients of its tiles in registers;
 //   * ppo_reduce_kernel sums the CTA partials in CTA order and applies 1/N: no float atomics anywhere, two calls with
-//     the same inputs give bit-identical gradients.
+//     the same inputs give bit-identical gradients;
+//   * ppo_kernel<KIND, false, true> (the statistics pass, mm_ppo_stats) runs the same forward over listed rows and sums
+//     per-row diagnostics (entropy, ratio to old_logp, value against the return) in f64 per CTA, and
+//     ppo_stats_reduce_kernel adds the CTA partials in CTA order.
 //
 // Network kinds (torch Linear layout: weight [out][in], bias [out]):
 //   ACTOR   ActorNetwork   30 -> 128 -> 128 -> 5, log-softmax
@@ -199,11 +202,21 @@ __device__ __forceinline__ float ppo_row(float r, float adv, float clip, float &
     return d_r * r;
 }
 
-template <int KIND, bool GRAD>
+// statistics partials per CTA: the MM_PPO_STAT_* fields as f64, RATIO_MIN / RATIO_MAX included
+constexpr int NSTAT = MM_PPO_STATS_LEN;
+
+// The three passes over listed rows are one kernel, so that they run the same forward arithmetic:
+//   <KIND, false>        the target pass: writes the per-row constants (old_logp_out / q_target_out)
+//   <KIND, true>         the gradient pass: adds the loss and the backward, weight-gradient partials per CTA
+//   <KIND, false, true>  the statistics pass: reduces per-row diagnostics (entropy, ratio, value fit) into NSTAT f64
+//                        partials per CTA, written through `partials` (old_logp_in nullable: no ratio)
+// STATS is a trailing defaulted parameter so that the target and gradient passes compile exactly as they did without it.
+template <int KIND, bool GRAD, bool STATS = false>
 __global__ void __launch_bounds__(LT, 1)
 ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions, const float *__restrict__ returns,
            const float *__restrict__ old_logp_in, const float *__restrict__ q_target_in, const int64_t *__restrict__ idx, int64_t n,
            float clip, mm_ppo_net net, float *__restrict__ old_logp_out, float *__restrict__ q_target_out, float *__restrict__ partials) {
+    static_assert(!(GRAD && STATS), "one pass at a time");
     using L = LG<KIND>;
     constexpr int H1 = L::H1, IN2 = L::IN2, OUT3 = L::OUT3, SB = L::SB, S3 = L::S3, N2T = L::N2G / 8;
     extern __shared__ __align__(16) unsigned char lsm[];
@@ -256,6 +269,12 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
     float g2[N2T][4], g3[3][1][4], g1[4][4], g1x[1][4];
     zero(g2); zero(g3[0]); zero(g3[1]); zero(g3[2]); zero(g1); zero(g1x);
     float loss_a = 0.f, loss_c = 0.f;
+    // statistics pass: this thread's rows, in tile order (f64 sums, f32 ratio range)
+    double st[NSTAT];
+#pragma unroll
+    for (int f = 0; f < NSTAT; ++f) st[f] = 0.0;
+    float r_min = __int_as_float(0x7f800000), r_max = -__int_as_float(0x7f800000);
+    const bool with_ratio = STATS && KIND != MM_PPO_CRITIC && old_logp_in != nullptr;
 
     const int64_t n_tiles = (n + LROWS - 1) / LROWS;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -275,6 +294,10 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
                     rf[r] = src < 0 ? 0.f : returns[src];
                     rf[LROWS + r] = (src < 0 || KIND == MM_PPO_CRITIC) ? 0.f : old_logp_in[src];
                     rf[2 * LROWS + r] = (src < 0 || KIND != MM_PPO_ACTOR) ? 0.f : q_target_in[src];
+                }
+                if (STATS) {
+                    rf[r] = (src < 0 || KIND == MM_PPO_ACTOR) ? 0.f : returns[src];
+                    rf[LROWS + r] = (src < 0 || !with_ratio) ? 0.f : old_logp_in[src];
                 }
                 if (KIND == MM_PPO_CRITIC) {
 #pragma unroll
@@ -346,9 +369,24 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
 #pragma unroll
                     for (int k = 1; k < NA; ++k) za = k == a ? z[k] : za;
                     const float logp = (za - m) - logf(s);
-                    if (!GRAD) {
+                    if (!GRAD && !STATS) {
                         if (src >= 0) old_logp_out[src] = logp;
-                    } else if (src >= 0) {
+                    } else if (STATS && src >= 0) {
+                        // entropy -sum p_k log p_k of the full log-softmax; ratio, k3 and clipping against old_logp
+                        const float lse = logf(s);
+                        float pl = 0.f;
+#pragma unroll
+                        for (int k = 0; k < NA; ++k) pl += (e[k] / s) * ((z[k] - m) - lse);
+                        st[MM_PPO_STAT_ENTROPY] += (double)(-pl);
+                        if (with_ratio) {
+                            const float lr = logp - rf[LROWS + r];
+                            const float ratio = expf(lr);
+                            st[MM_PPO_STAT_K3] += (double)((ratio - 1.f) - lr);
+                            st[MM_PPO_STAT_CLIPPED] += fabsf(ratio - 1.f) > clip ? 1.0 : 0.0;
+                            r_min = fminf(r_min, ratio);
+                            r_max = fmaxf(r_max, ratio);
+                        }
+                    } else if (GRAD && src >= 0) {
                         const float adv = KIND == MM_PPO_ACTOR ? rf[r] - rf[2 * LROWS + r] : rf[r] - z[5];
                         const float ratio = expf(logp - rf[LROWS + r]);
                         float l;
@@ -360,14 +398,23 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
                 }
                 if (KIND != MM_PPO_ACTOR) {
                     constexpr int kv = KIND == MM_PPO_CRITIC ? 0 : 5;
-                    if (!GRAD) {
+                    if (!GRAD && !STATS) {
                         if (KIND == MM_PPO_CRITIC && src >= 0) q_target_out[src] = z[kv];
-                    } else if (src >= 0) {
+                    } else if (STATS && src >= 0) {
+                        // the value's fit to the return: v = Q(s, a) or V(s), G, and the residual G - v, in f32
+                        const float v = z[kv], gr = rf[r], res = gr - v;
+                        st[MM_PPO_STAT_V] += (double)v;
+                        st[MM_PPO_STAT_V2] += (double)v * (double)v;
+                        st[MM_PPO_STAT_G] += (double)gr;
+                        st[MM_PPO_STAT_G2] += (double)gr * (double)gr;
+                        st[MM_PPO_STAT_RES2] += (double)res * (double)res;
+                    } else if (GRAD && src >= 0) {
                         const float d = z[kv] - rf[r];
                         loss_c += d * d;
                         dz[kv] = 2.f * d;
                     }
                 }
+                if (STATS && src >= 0) st[MM_PPO_STAT_N] += 1.0;
                 if (GRAD) {
                     uint4 v;
                     v.x = h2u(__floats2half2_rn(dz[0], dz[1]));
@@ -424,6 +471,33 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
         if (H1 > 128) wgrad_gemm<1>(g1x, h2a, SB, 128 + (warp >> 2) * 16, xa, SX, (warp & 3) * 8, lane);
         __syncthreads();
     }
+    if (STATS) {
+        // warp butterfly, then the 8 warps in order by one thread per field (the dZ3 tile, unused here, holds the warps'
+        // sums): the CTA's partial has a fixed summation order
+        st[MM_PPO_STAT_RATIO_MIN] = (double)r_min;
+        st[MM_PPO_STAT_RATIO_MAX] = (double)r_max;
+#pragma unroll
+        for (int f = 0; f < NSTAT; ++f)
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const double x = __shfl_xor_sync(0xffffffffu, st[f], o);
+                st[f] = f == MM_PPO_STAT_RATIO_MIN ? fmin(st[f], x) : f == MM_PPO_STAT_RATIO_MAX ? fmax(st[f], x) : st[f] + x;
+            }
+        double *wsum = reinterpret_cast<double *>(dz3s);
+        if (lane == 0)
+#pragma unroll
+            for (int f = 0; f < NSTAT; ++f) wsum[warp * NSTAT + f] = st[f];
+        __syncthreads();
+        if (tid < NSTAT) {
+            double acc = wsum[tid];
+            for (int w = 1; w < LT / 32; ++w) {
+                const double x = wsum[w * NSTAT + tid];
+                acc = tid == MM_PPO_STAT_RATIO_MIN ? fmin(acc, x) : tid == MM_PPO_STAT_RATIO_MAX ? fmax(acc, x) : acc + x;
+            }
+            reinterpret_cast<double *>(partials)[(int64_t)blockIdx.x * NSTAT + tid] = acc;
+        }
+        return;
+    }
     if (!GRAD) return;
 
     // ---- this CTA's partial sums, each element written by exactly one thread
@@ -454,6 +528,20 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
         part[L::PL] = sa;
         part[L::PL + 1] = sc;
     }
+}
+
+// The statistics partials of n_parts CTAs combined in CTA order (sums; min / max for the ratio range) into stats.
+// n_parts = 0 writes the empty value: zeros, RATIO_MIN = +inf, RATIO_MAX = -inf.
+__global__ void ppo_stats_reduce_kernel(const double *__restrict__ partials, int n_parts, double *__restrict__ stats) {
+    const int f = threadIdx.x;
+    if (f >= NSTAT) return;
+    const double inf = __longlong_as_double(0x7ff0000000000000ll);
+    double acc = f == MM_PPO_STAT_RATIO_MIN ? inf : f == MM_PPO_STAT_RATIO_MAX ? -inf : 0.0;
+    for (int c = 0; c < n_parts; ++c) {
+        const double x = partials[(int64_t)c * NSTAT + f];
+        acc = f == MM_PPO_STAT_RATIO_MIN ? fmin(acc, x) : f == MM_PPO_STAT_RATIO_MAX ? fmax(acc, x) : acc + x;
+    }
+    stats[f] = acc;
 }
 
 // Sum of the CTA partials in CTA order, times 1/N, scattered into the torch parameters' layout.
@@ -499,14 +587,32 @@ int device_sms(int &dev, int &sms) {
     return cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess;
 }
 
-template <int KIND, bool GRAD>
+template <int KIND, bool GRAD, bool STATS = false>
 int prepare(int dev) {
     static bool ready[MM_MAX_DEVICES] = {};
     if (ready[dev]) return 0;
-    if (cudaFuncSetAttribute(ppo_kernel<KIND, GRAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG<KIND>::SMEM) != cudaSuccess)
+    if (cudaFuncSetAttribute(ppo_kernel<KIND, GRAD, STATS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LG<KIND>::SMEM) !=
+        cudaSuccess)
         return 1;
     ready[dev] = true;
     return 0;
+}
+
+// The partials workspace: sized once per device for the largest kind's gradient partials at one CTA per SM (the
+// statistics partials are far smaller), reused by every call; calls on one device are ordered on the caller's stream, as
+// the update loop issues them.  -> null when the allocation fails.
+float *workspace(int dev, int sms) {
+    std::lock_guard<std::mutex> lock(g_ws_mutex);
+    const size_t need = (size_t)sms * LG<MM_PPO_SHARED>::P;
+    static_assert(LG<MM_PPO_ACTOR>::P * sizeof(float) >= NSTAT * sizeof(double), "statistics partials fit the workspace");
+    if (g_ws[dev].floats < need) {
+        if (g_ws[dev].ptr) cudaFree(g_ws[dev].ptr);
+        g_ws[dev].ptr = nullptr;
+        g_ws[dev].floats = 0;
+        if (cudaMalloc(&g_ws[dev].ptr, need * sizeof(float)) != cudaSuccess) return nullptr;
+        g_ws[dev].floats = need;
+    }
+    return g_ws[dev].ptr;
 }
 
 template <int KIND>
@@ -527,28 +633,38 @@ int launch_grads_t(const float *states, const int8_t *actions, const float *retu
     int dev = 0, sms = 0;
     if (device_sms(dev, sms) || prepare<KIND, true>(dev)) return 1;
     const int64_t tiles = (n + LROWS - 1) / LROWS, grid = tiles < sms ? tiles : sms;
-    float *ws;
-    {
-        // the partials workspace: sized once per device for the largest kind at one CTA per SM, reused by every call (calls
-        // on one device are ordered on the caller's stream, as the update loop issues them)
-        std::lock_guard<std::mutex> lock(g_ws_mutex);
-        const size_t need = (size_t)sms * LG<MM_PPO_SHARED>::P;
-        if (g_ws[dev].floats < need) {
-            if (g_ws[dev].ptr) cudaFree(g_ws[dev].ptr);
-            g_ws[dev].ptr = nullptr;
-            g_ws[dev].floats = 0;
-            if (cudaMalloc(&g_ws[dev].ptr, need * sizeof(float)) != cudaSuccess) return 1;
-            g_ws[dev].floats = need;
-        }
-        ws = g_ws[dev].ptr;
-    }
+    float *ws = workspace(dev, sms);
+    if (!ws) return 1;
     ppo_kernel<KIND, true><<<(unsigned)grid, LT, LG<KIND>::SMEM, s>>>(states, actions, returns, old_logp, q_target, idx, n, clip, net,
                                                                        nullptr, nullptr, ws);
     ppo_reduce_kernel<KIND><<<(unsigned)((LG<KIND>::P + 255) / 256), 256, 0, s>>>(ws, (int)grid, 1.0f / (float)n, gr, losses);
     return cudaGetLastError() != cudaSuccess;
 }
 
+template <int KIND>
+int launch_stats_t(const float *states, const int8_t *actions, const float *returns, const float *old_logp, const int64_t *idx,
+                   int64_t n, float clip, const mm_ppo_net &net, double *stats, cudaStream_t s) {
+    int dev = 0, sms = 0;
+    if (device_sms(dev, sms) || prepare<KIND, false, true>(dev)) return 1;
+    const int64_t tiles = (n + LROWS - 1) / LROWS, grid = tiles < sms ? tiles : sms;
+    float *ws = workspace(dev, sms);
+    if (!ws) return 1;
+    if (grid > 0)
+        ppo_kernel<KIND, false, true><<<(unsigned)grid, LT, LG<KIND>::SMEM, s>>>(states, actions, returns, old_logp, nullptr, idx, n,
+                                                                              clip, net, nullptr, nullptr, ws);
+    ppo_stats_reduce_kernel<<<1, 32, 0, s>>>(reinterpret_cast<const double *>(ws), (int)grid, stats);
+    return cudaGetLastError() != cudaSuccess;
+}
+
 }  // namespace
+
+int launch_ppo_stats(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                     const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net, double *stats, void *stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (kind == MM_PPO_ACTOR) return launch_stats_t<MM_PPO_ACTOR>(states, actions, returns, old_logp, idx, n, clip, *net, stats, s);
+    if (kind == MM_PPO_CRITIC) return launch_stats_t<MM_PPO_CRITIC>(states, actions, returns, old_logp, idx, n, clip, *net, stats, s);
+    return launch_stats_t<MM_PPO_SHARED>(states, actions, returns, old_logp, idx, n, clip, *net, stats, s);
+}
 
 int launch_ppo_targets(int kind, const float *states, const int8_t *actions, const int64_t *idx, int64_t n, const mm_ppo_net *net,
                        float *old_logp, float *q_target, void *stream) {

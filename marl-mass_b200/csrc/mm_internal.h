@@ -178,6 +178,8 @@ int launch_ppo_targets(int kind, const float *states, const int8_t *actions, con
 int launch_ppo_grads(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
                      const float *q_target, const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net,
                      const mm_ppo_grads_out *grads, float *losses, void *stream);
+int launch_ppo_stats(int kind, const float *states, const int8_t *actions, const float *returns, const float *old_logp,
+                     const int64_t *idx, int64_t n, float clip, const mm_ppo_net *net, double *stats, void *stream);
 // clip_grad_norm_ + RMSprop, one CTA per group (optim.cu); arguments already checked by the C ABI
 int launch_rmsprop_step(const mm_opt_group *groups, int n_groups, void *stream);
 

@@ -1,7 +1,8 @@
 """Multi-GPU plumbing: env instances shard across ranks with no step-path traffic (SURVEY.md §8e).
 
-One process per GPU (torch.distributed, NCCL on GPUs / gloo in the CPU tests).  The only collective is the
-all-reduce of the episode-statistics vector: SUM for the counters, MIN for min_headway.
+One process per GPU (torch.distributed, NCCL on GPUs / gloo in the CPU tests).  The only collectives are the
+all-reduce of the episode-statistics vector (SUM for the counters, MIN for min_headway) and, with update statistics
+on, of the learner's PPO statistics vectors (SUM, MIN for the smallest ratio, MAX for the largest).
 """
 import os
 
@@ -66,6 +67,27 @@ def all_reduce_stats(stats, device=None):
     out = {k: float(v) for k, v in zip(SUM_KEYS, s.tolist())}
     out.update({k: float(v) for k, v in zip(MIN_KEYS, m.tolist())})
     return out
+
+
+def all_reduce_ppo_stats(v):
+    """Fold per-rank PPO statistics vectors (`rollout.ppo_stats`: f64 [..., PPO_STATS_LEN] on the device) into job totals:
+    SUM for the sums and counts, MIN for ratio_min, MAX for ratio_max (as a MIN of its negation).  Returns a new tensor;
+    no-op (the same tensor) without a process group."""
+    import torch
+    import torch.distributed as dist
+    from ._lib import PPO_STAT
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return v
+    lo, hi = PPO_STAT["ratio_min"], PPO_STAT["ratio_max"]
+    s = v.clone()
+    s[..., lo] = 0.0
+    s[..., hi] = 0.0
+    m = torch.stack([v[..., lo], -v[..., hi]], -1).contiguous()
+    dist.all_reduce(s, op=dist.ReduceOp.SUM)
+    dist.all_reduce(m, op=dist.ReduceOp.MIN)
+    s[..., lo] = m[..., 0]
+    s[..., hi] = -m[..., 1]
+    return s
 
 
 def summarize(stats):

@@ -20,6 +20,7 @@ import torch
 from torch import nn
 
 from . import _lib
+from . import dist as mmd
 from ._lib import MAXV, NA, NS
 
 
@@ -409,6 +410,93 @@ def shared_network_gradients(policy, S, A8, G, old_logp, idx, clip=0.2, losses=N
     return losses[0] + losses[1], losses[0], losses[1]
 
 
+# ---- PPO diagnostics of one network over listed rows (mm_ppo_stats), and their torch reference
+
+@torch.no_grad()
+def ppo_stats(net, S, A8, G, idx, old_logp=None, clip=0.2):
+    """Statistics pass of the learner (mm_ppo_stats) over the rows S[idx]: -> f64 device tensor [PPO_STATS_LEN] with the
+    fields of `_lib.PPO_STAT_FIELDS` (row count; entropy of the policy; with old_logp [rows] the sums of k3 =
+    (r - 1) - log r and of |r - 1| > clip and the range of r = exp(logp(a) - old_logp); sums of v, v^2, G, G^2 and
+    (G - v)^2 for the value Q(s, a) of a CriticNetwork or V(s) of the shared network).  `net` as for `ppo_targets`; G [rows]
+    the returns (may be None for an ActorNetwork).  Enqueued on the current stream, no synchronisation."""
+    _check_rows(S, A8, idx, G)
+    kind, params = _ppo_kind(net)
+    if old_logp is not None:
+        assert old_logp.dtype == torch.float32 and old_logp.is_contiguous() and old_logp.numel() == S.shape[0]
+    out = torch.empty(_lib.PPO_STATS_LEN, dtype=torch.float64, device=S.device)
+    _lib.check(_lib.lib().mm_ppo_stats(kind, _ptr(S), _ptr(A8), _ptr(G), _ptr(old_logp), _ptr(idx), C.c_int64(idx.numel()),
+                                       C.c_float(clip), C.byref(_ppo_net(params)), _ptr(out), _stream()))
+    return out
+
+
+@torch.no_grad()
+def _ppo_stats_torch(net, S, A8, G, idx, old_logp, clip):
+    """-> (statistics vector, log p(a) per row of idx or None); rows in the module's dtype, sums in float64"""
+    dt = next(net.parameters()).dtype
+    s = S[idx].to(dt)
+    onehot = torch.nn.functional.one_hot(A8[idx].long(), NA).to(dt)
+    lp_all = v = logp = None
+    if isinstance(net, ActorCriticNetwork):
+        hidden = net.trunk(s)
+        lp_all, v = net.policy_head(hidden), net.critic_linear(hidden)[:, 0]
+    elif isinstance(net, CriticNetwork):
+        v = net(s, onehot)[:, 0]
+    else:
+        lp_all = net(s)
+    K = _lib.PPO_STAT
+    out = torch.zeros(_lib.PPO_STATS_LEN, dtype=torch.float64, device=S.device)
+    out[K["n"]] = idx.numel()
+    out[K["ratio_min"]], out[K["ratio_max"]] = float("inf"), -float("inf")
+    if lp_all is not None:
+        logp = (lp_all * onehot).sum(1)            # as mappo_losses / shared_network_loss form it
+        out[K["entropy"]] = (-(lp_all.exp() * lp_all).sum(1)).double().sum()
+        if old_logp is not None and idx.numel():
+            lr = logp - old_logp[idx].to(dt)
+            r = torch.exp(lr)
+            out[K["k3"]] = ((r - 1) - lr).double().sum()
+            out[K["clipped"]] = ((r - 1).abs() > clip).double().sum()
+            out[K["ratio_min"]], out[K["ratio_max"]] = r.min().double(), r.max().double()
+    if v is not None:
+        g = G[idx].to(dt)
+        vd, gd, res = v.double(), g.double(), (g - v).double()
+        out[K["v"]], out[K["v2"]] = vd.sum(), (vd * vd).sum()
+        out[K["g"]], out[K["g2"]] = gd.sum(), (gd * gd).sum()
+        out[K["res2"]] = (res * res).sum()
+    return out, logp
+
+
+def ppo_stats_torch(net, S, A8, G, idx, old_logp=None, clip=0.2):
+    """`ppo_stats` from the torch modules: the per-row values in the module's dtype (float32: the numerics of the torch
+    update path), the sums in float64.  Any device, any float dtype of `net`."""
+    return _ppo_stats_torch(net, S, A8, G, idx, old_logp, clip)[0]
+
+
+def ppo_stats_keys(before, after):
+    """The diagnostics of one update from the statistics vectors (host sequences, all-reduced over ranks) of the pass over
+    every live row with the rollout networks (`before`, no ratio) and with the updated ones against the rollout policy's
+    log-probabilities (`after`).  Explained variance 1 - Var(G - v) / Var(G), advantage G - v of the rollout critic;
+    variances and the advantage's std are population moments."""
+    K = _lib.PPO_STAT
+    n = before[K["n"]]
+    if n <= 0:
+        nan = float("nan")
+        return dict.fromkeys(("approx_kl", "clip_fraction", "ratio_min", "ratio_max", "entropy_before", "entropy_after",
+                              "explained_variance_before", "explained_variance_after", "advantage_mean", "advantage_std"), nan)
+
+    def fit(v):
+        mean_res = (v[K["g"]] - v[K["v"]]) / n
+        var_res = v[K["res2"]] / n - mean_res * mean_res
+        var_g = v[K["g2"]] / n - (v[K["g"]] / n) ** 2
+        return mean_res, var_res, (1.0 - var_res / var_g) if var_g > 0 else float("nan")
+
+    adv_mean, adv_var, ev_before = fit(before)
+    return {"approx_kl": after[K["k3"]] / n, "clip_fraction": after[K["clipped"]] / n,
+            "ratio_min": after[K["ratio_min"]], "ratio_max": after[K["ratio_max"]],
+            "entropy_before": before[K["entropy"]] / n, "entropy_after": after[K["entropy"]] / n,
+            "explained_variance_before": ev_before, "explained_variance_after": fit(after)[2],
+            "advantage_mean": adv_mean, "advantage_std": max(adv_var, 0.0) ** 0.5}
+
+
 # ---- the optimiser step on the device (mm_rmsprop_step): clip_grad_norm_ + RMSprop, one launch for whole networks
 
 _MIRROR_COLS = {}
@@ -721,21 +809,27 @@ class BatchedMAPPORollout(object):
             q.grad.copy_(flat[o:o + q.numel()].view_as(q.grad))
             o += q.numel()
 
-    def update(self, minibatch=1 << 18, epochs=1, impl="torch"):
+    def update(self, minibatch=1 << 18, epochs=1, impl="torch", stats=False):
         """PPO-clip actor update and critic regression on the last rollout (mappo.py:161-206, `mappo_losses`), all
         agents at once, with the per-sample surrogate (the reference's [N] x [N, 1] product is an N x N table).
         Under torch.distributed every rank runs the same number of minibatches and the gradients are averaged.
-        impl: "torch" (autograd) or "cuda" (the learner kernels: `_update_cuda`)."""
+        impl: "torch" (autograd) or "cuda" (the learner kernels: `_update_cuda`).
+        stats: also measure what the update did (the keys of `ppo_stats_keys`): a statistics pass over every live row with
+        the rollout (target) networks before the first minibatch and one with the updated networks after the last, with
+        `ppo_stats_torch` (impl "torch") or `ppo_stats` (impl "cuda"), all-reduced over ranks and read in one host read.
+        The passes draw no random numbers and write no parameter: the update is the same with and without them."""
         if impl == "cuda":
-            return self._update_cuda(minibatch, epochs)
+            return self._update_cuda(minibatch, epochs, stats)
         assert impl == "torch", impl
+        batch = self._learner_batch() if stats else None
+        before = self._stats_begin("torch", batch) if stats else None
         b = self.buf
         live = b["live"].reshape(-1)
         idx = live.nonzero(as_tuple=False).squeeze(1)
         S = b["states"].reshape(-1, NS)
         A = torch.nn.functional.one_hot(b["actions"].reshape(-1), NA).float()
         G = b["returns"].reshape(-1, 1)
-        stats = {}
+        rec = {}
         n_max = torch.tensor([idx.numel()], device=self.dev)
         if self._world() > 1:
             import torch.distributed as dist
@@ -752,11 +846,13 @@ class BatchedMAPPORollout(object):
                 self.critic_opt.zero_grad(set_to_none=True)
                 critic_loss.backward()
                 self._optimizer_step([self.critic_opt], [self.critic])
-                stats = {"actor_loss": float(actor_loss.detach()), "critic_loss": float(critic_loss.detach()),
-                         "samples": int(idx.numel())}
+                rec = {"actor_loss": float(actor_loss.detach()), "critic_loss": float(critic_loss.detach()),
+                       "samples": int(idx.numel())}
+        if stats:
+            rec.update(self._stats_end("torch", batch, *before))
         self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
         self.critic_target.load_state_dict(self.critic.state_dict())
-        return stats
+        return rec
 
     def _learner_batch(self):
         """(live row list, states [rows, 30], actions int8 [rows], returns [rows], minibatch count) of the last rollout"""
@@ -774,16 +870,54 @@ class BatchedMAPPORollout(object):
             dist.all_reduce(n_max, op=dist.ReduceOp.MAX)
         return max(1, -(-int(n_max) // int(minibatch)))       # same count on every rank
 
-    def _update_cuda(self, minibatch, epochs):
+    def _stat_nets(self, target):
+        """(policy network, value network) of the statistics passes: the rollout's (the targets) or the updated ones"""
+        return (self.actor_target, self.critic_target) if target else (self.actor, self.critic)
+
+    def _stats_pass(self, impl, target, batch, old_logp):
+        """-> (statistics vector of the policy and value networks over every live row, the policy's log p(a) per row of
+        idx from the torch pass or None)"""
+        idx, S, A8, G = batch
+        pol, val = self._stat_nets(target)
+        if impl == "cuda":
+            v, logp = ppo_stats(pol, S, A8, G, idx, old_logp, self.clip_param), None
+        else:
+            v, logp = _ppo_stats_torch(pol, S, A8, G, idx, old_logp, self.clip_param)
+        if val is not pol:
+            vf = _lib.PPO_STAT["v"]
+            w = ppo_stats(val, S, A8, G, idx) if impl == "cuda" else _ppo_stats_torch(val, S, A8, G, idx, None, self.clip_param)[0]
+            v[vf:] = w[vf:]
+        return v, logp
+
+    @torch.no_grad()
+    def _stats_begin(self, impl, batch, old_logp=None):
+        """statistics pass with the rollout networks; -> (its vector, the rollout policy's log p(a) indexed like the
+        states: `old_logp` of the CUDA target pass, or from this pass)"""
+        before, logp = self._stats_pass(impl, True, batch, None)
+        if old_logp is None:
+            idx, S = batch[0], batch[1]
+            old_logp = torch.zeros(S.shape[0], dtype=logp.dtype, device=S.device)
+            old_logp[idx] = logp
+        return before, old_logp
+
+    @torch.no_grad()
+    def _stats_end(self, impl, batch, before, old_logp):
+        """statistics pass with the updated networks against the rollout policy, all-reduce, one host read -> the keys"""
+        after, _ = self._stats_pass(impl, False, batch, old_logp)
+        b, a = mmd.all_reduce_ppo_stats(torch.stack([before, after])).tolist()
+        return ppo_stats_keys(b, a)
+
+    def _update_cuda(self, minibatch, epochs, stats=False):
         """`update` with the learner kernels: one target pass (old log-probabilities and Q_target of every live sample,
         the target networks do not change within an update), then per minibatch one gradient pass (mappo_gradients) in
         place of the two backward passes; then all-reduce, gradient clipping and the RMSprop steps as in the torch path
         (with optimizer="cuda" one launch steps both networks).  The losses stay on the device until the one read at the
         end."""
-        idx, S, A8, G = self._learner_batch()
+        batch = idx, S, A8, G = self._learner_batch()
         n_mb = self._minibatch_count(idx, minibatch)
         old_logp = ppo_targets(self.actor_target, S, A8, idx)
         q_target = ppo_targets(self.critic_target, S, A8, idx)
+        before = self._stats_begin("cuda", batch, old_logp) if stats else None
         losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
         for _ in range(epochs):
             perm = idx[torch.randperm(idx.numel(), device=self.dev)]
@@ -791,9 +925,12 @@ class BatchedMAPPORollout(object):
                 mappo_gradients(self.actor, self.critic, S, A8, G, old_logp, q_target, j, self.clip_param, losses=losses)
                 self._optimizer_step([self.actor_opt, self.critic_opt], [self.actor, self.critic])
         a_loss, c_loss = losses.tolist()
+        rec = {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
+        if stats:
+            rec.update(self._stats_end("cuda", batch, *before))
         self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
         self.critic_target.load_state_dict(self.critic.state_dict())
-        return {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
+        return rec
 
 
 class BatchedMAPPOGIRollout(BatchedMAPPORollout):
@@ -846,24 +983,30 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
     def networks(self):
         return [self.policy, self.policy_target]
 
+    def _stat_nets(self, target):
+        net = self.policy_target if target else self.policy
+        return net, net
+
     def sample_actions(self, obs, n_agents, seed, step):
         if self.fused:
             return policy_sample(self.policy, obs.contiguous(), n_agents, seed=seed, step=step)
         return self.act_torch(obs, n_agents)[0]
 
-    def update(self, minibatch=1 << 18, epochs=1, impl="torch"):
+    def update(self, minibatch=1 << 18, epochs=1, impl="torch", stats=False):
         """One pass of `MAPPO_GI.train` (shared branch, mappo_gi.py:307-349) over the last rollout, all agents at once;
         under torch.distributed the gradients are averaged over the ranks.  impl: "torch" (autograd) or "cuda" (the
-        learner kernels)."""
+        learner kernels).  stats: as for `BatchedMAPPORollout.update`, with the shared network as policy and value."""
         if impl == "cuda":
-            return self._update_cuda(minibatch, epochs)
+            return self._update_cuda(minibatch, epochs, stats)
         assert impl == "torch", impl
+        batch = self._learner_batch() if stats else None
+        before = self._stats_begin("torch", batch) if stats else None
         b = self.buf
         idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
         S = b["states"].reshape(-1, NS)
         A = torch.nn.functional.one_hot(b["actions"].reshape(-1), NA).float()
         G = b["returns"].reshape(-1, 1)
-        stats = {}
+        rec = {}
         n_max = torch.tensor([idx.numel()], device=self.dev)
         if self._world() > 1:
             import torch.distributed as dist
@@ -876,17 +1019,20 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
                 self.policy_opt.zero_grad(set_to_none=True)
                 loss.backward()
                 self._optimizer_step([self.policy_opt], [self.policy])
-                stats = {"actor_loss": float(a_loss.detach()), "critic_loss": float(c_loss.detach()),
-                         "samples": int(idx.numel())}
+                rec = {"actor_loss": float(a_loss.detach()), "critic_loss": float(c_loss.detach()),
+                       "samples": int(idx.numel())}
+        if stats:
+            rec.update(self._stats_end("torch", batch, *before))
         self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
-        return stats
+        return rec
 
-    def _update_cuda(self, minibatch, epochs):
+    def _update_cuda(self, minibatch, epochs, stats=False):
         """`update` with the learner kernels: one target pass, one gradient pass per minibatch
         (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step (optimizer="cuda": one launch)."""
-        idx, S, A8, G = self._learner_batch()
+        batch = idx, S, A8, G = self._learner_batch()
         n_mb = self._minibatch_count(idx, minibatch)
         old_logp = ppo_targets(self.policy_target, S, A8, idx)
+        before = self._stats_begin("cuda", batch, old_logp) if stats else None
         losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
         for _ in range(epochs):
             perm = idx[torch.randperm(idx.numel(), device=self.dev)]
@@ -894,5 +1040,8 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
                 shared_network_gradients(self.policy, S, A8, G, old_logp, j, self.clip_param, losses=losses)
                 self._optimizer_step([self.policy_opt], [self.policy])
         a_loss, c_loss = losses.tolist()
+        rec = {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
+        if stats:
+            rec.update(self._stats_end("cuda", batch, *before))
         self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
-        return {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
+        return rec

@@ -51,7 +51,7 @@ def load_ini(path):
 
 
 def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch",
-          optimizer="torch", eval_seeds=0, eval_shield=False):
+          optimizer="torch", eval_seeds=0, eval_shield=False, update_stats=False):
     """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`).
     optimizer: "torch" (clip_grad_norm_ + torch.optim.RMSprop, the default) or "cuda" (`rollout.DeviceRMSprop`: the same
     step in one launch per minibatch).
@@ -63,7 +63,11 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
     eval_shield: with eval_seeds, also record the shield's activity on those episodes (`evaluate_seeds(shield_records=True)`)
     and log evalN_shield_intervention_rate (interventions over QP solves), evalN_lane_change_vetoes_per_episode,
     evalN_min_agent_acc (the hardest applied acceleration of any controlled vehicle) and evalN_acc_correction_max (the
-    largest |safe - nominal| acceleration)."""
+    largest |safe - nominal| acceleration).
+    update_stats: also measure every update (`update(stats=True)`, with either update_impl) and log the keys of
+    `rollout.ppo_stats_keys` with an update_ prefix: update_approx_kl, update_clip_fraction, update_ratio_min /
+    update_ratio_max, update_entropy_before / _after, update_explained_variance_before / _after, update_advantage_mean and
+    update_advantage_std.  The update and every other key are the same with and without it."""
     if eval_shield and not eval_seeds > 0:
         raise ValueError("train: eval_shield records the shield on the eval_seeds episodes and needs eval_seeds > 0")
     import torch
@@ -86,6 +90,10 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
         # with n_s = 30).  Rejected before anything is built (a 25-column state would otherwise be fed to 30 inputs).
         raise ValueError("train: env id %r is not covered by the batched learner (n_s = 30 env id merge-multi-agent-v1 only)"
                          % (env_cfg.get("env_name"),))
+    if not isinstance(update_stats, bool):
+        raise ValueError("train: update_stats must be True or False, got %r" % (update_stats,))
+    if update_stats and update_impl not in ("torch", "cuda"):
+        raise ValueError("train: update_stats measures the 'torch' or 'cuda' update, got update_impl %r" % (update_impl,))
     env = MergeEnvBatched(n_envs, dict(DEFAULT_CONFIG, **env_cfg), device=device)
     # rank-distinct spawn stream; its first observation goes to the rollout so that collect() does not re-spawn the
     # scenes with the (rank-independent) config seed
@@ -116,7 +124,8 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
         pol.collect()
         torch.cuda.synchronize(device)
         t1 = time.perf_counter()
-        up = pol.update(minibatch=minibatch, impl=update_impl)
+        up = pol.update(minibatch=minibatch, impl=update_impl, stats=update_stats)
+        up = {(k if k in ("actor_loss", "critic_loss", "samples") else "update_" + k): v for k, v in up.items()}
         torch.cuda.synchronize(device)
         t2 = time.perf_counter()
         s = mmd.all_reduce_stats(env.stats())
@@ -172,9 +181,12 @@ def main():
                     help="N > 0: also evaluate on the test seeds 0..N-1 with the device-side protocol (evalN_* keys)")
     ap.add_argument("--eval-shield", action="store_true",
                     help="with --eval-seeds: also log the shield's interventions, vetoes and corrections (evalN_shield_* keys)")
+    ap.add_argument("--update-stats", action="store_true",
+                    help="also log what each update did: KL to the rollout policy, clip fraction, ratio range, entropy, "
+                         "explained variance, advantage mean / std (update_* keys)")
     a = ap.parse_args()
     train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl, optimizer=a.optimizer,
-          eval_seeds=a.eval_seeds, eval_shield=a.eval_shield)
+          eval_seeds=a.eval_seeds, eval_shield=a.eval_shield, update_stats=a.update_stats)
 
 
 if __name__ == "__main__":
