@@ -332,6 +332,19 @@ int mm_set_actor_impl(int impl);
 int mm_discounted_returns(const float *rewards, const uint8_t *dones, const float *final_value, float gamma, int T,
                           int64_t n_cols, int cols_per_env, float *out, void *stream);
 
+/* mm_lambda_returns: the lambda-return (GAE(lambda) return) of every (env, agent) column of a rollout, in the same kernel as
+ * mm_discounted_returns.  Per column, from t = T - 1 down to 0, with run = v_next = final_value[c] (nullable: 0):
+ *   if dones[t][c / cols_per_env]: run = v_next = 0
+ *   run = (lambda * run + (1 - lambda) * v_next) * gamma + rewards[t][c];  out[t][c] = run;  v_next = values[t][c]
+ * each product and sum rounded to float32 separately (never fused).  values [T][n_cols] f32 = V(s_t) of the networks that
+ * collected the rollout; nullable when lambda == 1, which gives mm_discounted_returns' output bit for bit (with values as
+ * well, as long as they are finite where they are read; up to the sign of a zero).  values[t][c] is read only where step
+ * t - 1 did not end the episode.  lambda = 0 gives the one-step targets r_t + gamma (1 - d_t) V(s_{t+1}).  DEVICE
+ * pointers; arguments are checked before any CUDA call (MM_ERR_ARG): rewards, dones and out required, 0 <= lambda <= 1,
+ * finite gamma, values required when lambda < 1, the rollout shape as for mm_discounted_returns. */
+int mm_lambda_returns(const float *rewards, const uint8_t *dones, const float *values, const float *final_value, float gamma,
+                      float lambda, int T, int64_t n_cols, int cols_per_env, float *out, void *stream);
+
 /* On-device PPO learner: the networks of one MAPPO / MAPPO_GI update with the per-sample PPO-clip surrogate and the MSE
  * value loss (marl/mappo.py:161-206, marl/mappo_gi.py:307-349; rollout.mappo_losses / shared_network_loss with
  * pairwise=False, critic_loss="mse").  Network kinds, parameters as torch.nn.Linear lays them out (weight [out][in]):
@@ -350,7 +363,8 @@ typedef struct { float *w1, *b1, *w2, *b2, *w3, *b3, *w4, *b4; } mm_ppo_grads_ou
 
 /* Target pass (forward only), once per update with the TARGET networks: for every listed row, old_logp[row] = log p(a)
  * (MM_PPO_ACTOR, MM_PPO_SHARED) or q_target[row] = Q(s, one_hot(a)) (MM_PPO_CRITIC); outputs are indexed like states.
- * Replaces the no-grad half of MAPPO.train (mappo.py:170-183) and MAPPO_GI.train (mappo_gi.py:307-320), which torch
+ * MM_PPO_SHARED with a non-null q_target also writes q_target[row] = V(s) from the same forward (the values of the
+ * rollout for mm_lambda_returns); MM_PPO_ACTOR ignores q_target.  Rows not listed are not written.  Replaces the no-grad half of MAPPO.train (mappo.py:170-183) and MAPPO_GI.train (mappo_gi.py:307-320), which torch
  * recomputes for every minibatch. */
 int mm_ppo_targets(int kind, const float *states, const int8_t *actions, const int64_t *idx, int64_t n, const mm_ppo_net *net,
                    float *old_logp, float *q_target, void *stream);

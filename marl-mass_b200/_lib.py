@@ -139,7 +139,7 @@ SUPERVISOR_DRAWS = 32     # MM_SUPERVISOR_DRAWS
 EXPORTS = ("mm_create", "mm_destroy", "mm_set_config", "mm_num_envs", "mm_reset", "mm_step", "mm_step_host",
            "mm_step_host_ragged", "mm_step_host_packed", "mm_expand_obs_rows",
            "mm_buffers_get", "mm_get_state", "mm_set_state", "mm_get_shield_diag", "mm_stats", "mm_shield_qp", "mm_shield_query",
-           "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_ppo_stats", "mm_rmsprop_step", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
+           "mm_actor_sample", "mm_actor_sample_mlp", "mm_set_actor_impl", "mm_set_step_variant", "mm_step_build", "mm_abi_version", "mm_discounted_returns", "mm_lambda_returns", "mm_ppo_targets", "mm_ppo_grads", "mm_ppo_stats", "mm_rmsprop_step", "mm_supervise", "mm_set_supervisor_draws", "mm_supervisor_draws_used",
            "mm_reset_seeded", "mm_check_seeds", "mm_eval_record", "mm_eval_shield_record", "mm_kernel_launches", "mm_last_error", "mm_version")
 
 
@@ -187,6 +187,8 @@ def lib():
     L.mm_step_build.argtypes = [h]
     L.mm_discounted_returns.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int, C.c_int64, C.c_int,
                                         C.c_void_p, C.c_void_p]
+    L.mm_lambda_returns.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_int, C.c_int64,
+                                    C.c_int, C.c_void_p, C.c_void_p]
     L.mm_ppo_targets.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(MMPpoNet), C.c_void_p,
                                  C.c_void_p, C.c_void_p]
     L.mm_ppo_grads.argtypes = [C.c_int] + [C.c_void_p] * 6 + [C.c_int64, C.c_float, C.POINTER(MMPpoNet), C.POINTER(MMPpoGrads),

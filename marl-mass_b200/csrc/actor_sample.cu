@@ -601,32 +601,43 @@ int launch_actor_mlp(const float *obs, const int32_t *n_agents, int64_t n_rows, 
     return 2;
 }
 
-// R_t = r_t + gamma * R_{t+1}, restarted after a terminal step: MAPPO._discount_reward (marl/mappo.py:364-370) for every
-// (env, agent) column of a rollout at once.  rewards / out [T][n_cols], dones [T][n_cols / cols_per_env] (1 where step t
-// ended the episode of that env), final_value [n_cols] (critic bootstrap; ignored where the last step was terminal).
+// The lambda-return R_t = r_t + gamma * (lambda R_{t+1} + (1 - lambda) V_{t+1}), restarted after a terminal step, for every
+// (env, agent) column of a rollout at once.  rewards / values / out [T][n_cols], dones [T][n_cols / cols_per_env] (1 where
+// step t ended the episode of that env), final_value [n_cols] (R and V after the last step; ignored where the last step was
+// terminal).  values == nullptr is lambda = 1, the discounted return of MAPPO._discount_reward (marl/mappo.py:364-370):
+// run = run * gamma + r, the expression mm_discounted_returns has always computed.  With values the mix is rounded
+// product by product (__fmul_rn / __fadd_rn, never contracted whatever -fmad says), so lambda = 1 gives
+// 1 * run + 0 * v == run and the same bits as without values (up to the sign of a zero run); values[t][c] is read only
+// when step t - 1 did not end the episode, and a non-finite value there would turn 0 * v into NaN.
 __global__ void __launch_bounds__(256) discounted_returns_kernel(const float *__restrict__ rewards,
                                                                  const uint8_t *__restrict__ dones,
-                                                                 const float *__restrict__ final_value, float gamma, int T,
-                                                                 int64_t n_cols, int cols_per_env, float *__restrict__ out) {
+                                                                 const float *__restrict__ values,
+                                                                 const float *__restrict__ final_value, float gamma, float lambda,
+                                                                 int T, int64_t n_cols, int cols_per_env, float *__restrict__ out) {
     const int64_t n_env = n_cols / cols_per_env;
+    const float one_minus_lambda = __fsub_rn(1.f, lambda);
     for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n_cols; c += (int64_t)gridDim.x * blockDim.x) {
         const int64_t e = c / cols_per_env;
-        float run = final_value ? final_value[c] : 0.f;
+        float run = final_value ? final_value[c] : 0.f, v_next = run;
         for (int t = T - 1; t >= 0; --t) {
-            if (dones[(int64_t)t * n_env + e]) run = 0.f;
+            if (dones[(int64_t)t * n_env + e]) run = v_next = 0.f;
+            if (values) {
+                run = __fadd_rn(__fmul_rn(lambda, run), __fmul_rn(one_minus_lambda, v_next));
+                v_next = values[(int64_t)t * n_cols + c];
+            }
             run = run * gamma + rewards[(int64_t)t * n_cols + c];
             out[(int64_t)t * n_cols + c] = run;
         }
     }
 }
 
-int launch_discounted_returns(const float *rewards, const uint8_t *dones, const float *final_value, float gamma, int T,
-                              int64_t n_cols, int cols_per_env, float *out, void *stream) {
+int launch_discounted_returns(const float *rewards, const uint8_t *dones, const float *values, const float *final_value,
+                              float gamma, float lambda, int T, int64_t n_cols, int cols_per_env, float *out, void *stream) {
     if (n_cols <= 0 || T <= 0) return 0;
     int64_t blocks = (n_cols + 255) / 256;
     if (blocks > 148 * 8) blocks = 148 * 8;
-    discounted_returns_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(rewards, dones, final_value, gamma, T, n_cols,
-                                                                               cols_per_env, out);
+    discounted_returns_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(rewards, dones, values, final_value, gamma,
+                                                                               lambda, T, n_cols, cols_per_env, out);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

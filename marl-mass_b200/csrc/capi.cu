@@ -967,7 +967,20 @@ int mm_discounted_returns(const float *rewards, const uint8_t *dones, const floa
     if (!rewards || !dones || !out) return fail(MM_ERR_ARG, "null argument");
     if (T < 0 || n_cols < 0 || cols_per_env <= 0 || n_cols % cols_per_env != 0)
         return fail(MM_ERR_ARG, "bad rollout shape");
-    if (launch_discounted_returns(rewards, dones, final_value, gamma, T, n_cols, cols_per_env, out, stream))
+    if (launch_discounted_returns(rewards, dones, nullptr, final_value, gamma, 1.f, T, n_cols, cols_per_env, out, stream))
+        return fail(MM_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
+    return 0;
+}
+
+int mm_lambda_returns(const float *rewards, const uint8_t *dones, const float *values, const float *final_value, float gamma,
+                      float lambda, int T, int64_t n_cols, int cols_per_env, float *out, void *stream) {
+    if (!rewards || !dones || !out) return fail(MM_ERR_ARG, "rewards, dones and out are required");
+    if (T < 0 || n_cols < 0 || cols_per_env <= 0 || n_cols % cols_per_env != 0)
+        return fail(MM_ERR_ARG, "bad rollout shape");
+    if (!(lambda >= 0.f && lambda <= 1.f)) return fail(MM_ERR_ARG, "lambda must be in [0, 1]");
+    if (!std::isfinite(gamma)) return fail(MM_ERR_ARG, "gamma must be finite");
+    if (lambda < 1.f && !values) return fail(MM_ERR_ARG, "values are required for lambda < 1");
+    if (launch_discounted_returns(rewards, dones, values, final_value, gamma, lambda, T, n_cols, cols_per_env, out, stream))
         return fail(MM_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
     return 0;
 }

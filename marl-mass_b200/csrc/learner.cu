@@ -206,7 +206,8 @@ __device__ __forceinline__ float ppo_row(float r, float adv, float clip, float &
 constexpr int NSTAT = MM_PPO_STATS_LEN;
 
 // The three passes over listed rows are one kernel, so that they run the same forward arithmetic:
-//   <KIND, false>        the target pass: writes the per-row constants (old_logp_out / q_target_out)
+//   <KIND, false>        the target pass: writes the per-row constants (old_logp_out / q_target_out; the shared network
+//                        writes V(s) to q_target_out when it is non-null)
 //   <KIND, true>         the gradient pass: adds the loss and the backward, weight-gradient partials per CTA
 //   <KIND, false, true>  the statistics pass: reduces per-row diagnostics (entropy, ratio, value fit) into NSTAT f64
 //                        partials per CTA, written through `partials` (old_logp_in nullable: no ratio)
@@ -399,7 +400,7 @@ ppo_kernel(const float *__restrict__ states, const int8_t *__restrict__ actions,
                 if (KIND != MM_PPO_ACTOR) {
                     constexpr int kv = KIND == MM_PPO_CRITIC ? 0 : 5;
                     if (!GRAD && !STATS) {
-                        if (KIND == MM_PPO_CRITIC && src >= 0) q_target_out[src] = z[kv];
+                        if ((KIND == MM_PPO_CRITIC || q_target_out != nullptr) && src >= 0) q_target_out[src] = z[kv];
                     } else if (STATS && src >= 0) {
                         // the value's fit to the return: v = Q(s, a) or V(s), G, and the residual G - v, in f32
                         const float v = z[kv], gr = rf[r], res = gr - v;

@@ -169,8 +169,8 @@ int launch_actor_mlp(const float *obs, const int32_t *n_agents, int64_t n_rows, 
                      const float *w2, const float *b2, const float *w3, const float *b3, const float *wv, const float *bv,
                      uint64_t seed, uint64_t step, const uint8_t *mask_bits, int8_t *actions, float *logp_all, float *logp_sel,
                      float *values, float *obs_copy, uint8_t *live_out, void *stream);
-int launch_discounted_returns(const float *rewards, const uint8_t *dones, const float *final_value, float gamma, int T,
-                              int64_t n_cols, int cols_per_env, float *out, void *stream);
+int launch_discounted_returns(const float *rewards, const uint8_t *dones, const float *values, const float *final_value,
+                              float gamma, float lambda, int T, int64_t n_cols, int cols_per_env, float *out, void *stream);
 
 // on-device PPO learner (learner.cu); arguments already checked by the C ABI
 int launch_ppo_targets(int kind, const float *states, const int8_t *actions, const int64_t *idx, int64_t n, const mm_ppo_net *net,

@@ -174,6 +174,42 @@ def discounted_returns(rewards, dones, final_value, gamma):
     return out
 
 
+def lambda_returns(rewards, dones, values, final_value, gamma, lam):
+    """GAE(lambda) returns R_t = r_t + gamma * (lam * R_{t+1} + (1 - lam) * V_{t+1}), restarted after a terminal step, one
+    CUDA kernel for the whole rollout (mm_lambda_returns, the kernel of `discounted_returns`).  lam = 1 gives
+    `discounted_returns` bit for bit; lam = 0 the one-step targets r_t + gamma (1 - d_t) V_{t+1}.
+
+    rewards, values [T, E, A] f32 cuda (values: V(s_t) of the networks that collected the rollout, finite wherever a
+    recursion reads them - rows of an agent that does not exist are best zero), dones [T, E], final_value [E, A] or None
+    (R and V after the last step)."""
+    T, E, A = rewards.shape
+    rewards = rewards.contiguous().float()
+    values = values.contiguous().float()
+    d8 = (dones != 0).to(torch.uint8).contiguous()
+    assert rewards.is_cuda and d8.shape == (T, E) and values.shape == rewards.shape and values.device == rewards.device
+    fv = None if final_value is None else final_value.contiguous().float()
+    out = torch.empty_like(rewards)
+    _lib.check(_lib.lib().mm_lambda_returns(_ptr(rewards), _ptr(d8), _ptr(values), _ptr(fv), C.c_float(gamma), C.c_float(lam),
+                                            T, C.c_int64(E * A), A, _ptr(out), _stream()))
+    return out
+
+
+def check_gae_lambda(gae_lambda):
+    """None, or the GAE lambda as a float in [0, 1]; anything else (a non-number, a bool, NaN, out of range) raises
+    ValueError.  A string (an ini value) is parsed as a number."""
+    if gae_lambda is None:
+        return None
+    x = gae_lambda
+    if isinstance(x, str):
+        try:
+            x = float(x)
+        except ValueError:
+            x = None
+    if isinstance(x, bool) or not isinstance(x, (int, float, np.integer, np.floating)) or not 0.0 <= float(x) <= 1.0:
+        raise ValueError("gae_lambda must be None or a number in [0, 1], got %r" % (gae_lambda,))
+    return float(x)
+
+
 _ACTOR_IMPLS = {"tcgen05": 0, "mma": 1}
 
 
@@ -331,20 +367,24 @@ def _check_rows(S, A8, idx, G=None):
 
 
 @torch.no_grad()
-def ppo_targets(net, S, A8, idx, out=None):
+def ppo_targets(net, S, A8, idx, out=None, value_out=None):
     """Target pass of one update (mm_ppo_targets): for the rows listed in idx, the target log-probability of the taken
     action (`net` an ActorNetwork or the shared ActorCriticNetwork) or Q_target(s, one_hot(a)) (`net` a CriticNetwork).
     S [rows, 30] f32, A8 [rows] int8 (the rollout buffer as collected), idx int64 [n]; -> out [rows] f32, indexed like
-    S (rows not listed are left as they are)."""
+    S (rows not listed are left as they are).  value_out [rows] f32 (shared network only): also V(s) from the same
+    forward, indexed the same way."""
     rows = _check_rows(S, A8, idx)
     kind, params = _ppo_kind(net)
     out = torch.empty(rows, dtype=torch.float32, device=S.device) if out is None else out
     assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == rows
+    if value_out is not None:
+        assert kind == _lib.PPO_SHARED, "value_out is the shared network's V(s)"
+        assert value_out.dtype == torch.float32 and value_out.is_contiguous() and value_out.numel() == rows
     if idx.numel() == 0:
         return out
     crit = kind == _lib.PPO_CRITIC
     _lib.check(_lib.lib().mm_ppo_targets(kind, _ptr(S), _ptr(A8), _ptr(idx), C.c_int64(idx.numel()), C.byref(_ppo_net(params)),
-                                         _ptr(None if crit else out), _ptr(out if crit else None), _stream()))
+                                         _ptr(None if crit else out), _ptr(out if crit else value_out), _stream()))
     return out
 
 
@@ -647,15 +687,19 @@ def _check_record_slots(rows, obs_copy, live_out):
 class BatchedMAPPORollout(object):
     def __init__(self, env, actor=None, critic=None, roll_out_n_steps=100, reward_gamma=0.99, reward_scale=20.0,
                  reward_type="regionalR", clip_param=0.2, actor_lr=5e-4, critic_lr=5e-4, max_grad_norm=5.0, seed=0,
-                 fused=True, obs=None, reset_seed=None, optimizer="torch"):
+                 fused=True, obs=None, reset_seed=None, optimizer="torch", gae_lambda=None):
         """obs: the observation of an env the caller has already reset (train.py resets with a rank-distinct spawn
         seed and hands its first observation over).  Without it the first collect() spawns the scenes itself with
         `reset_seed` (default: derived from `seed`, which the data-parallel driver makes rank-distinct) - never with the
         env's config seed, which is the same on every rank and would make the shards replicas of one another.
         optimizer: "torch" (torch.optim.RMSprop after clip_grad_norm_, the default) or "cuda" (`DeviceRMSprop`: the same
-        step as one launch per minibatch, with either update impl)."""
+        step as one launch per minibatch, with either update impl).
+        gae_lambda: None (the default: the Monte-Carlo returns of the reference) or a number in [0, 1]: update() trains on
+        the lambda-returns (`lambda_returns`, stored as buf["lambda_returns"]) with the values of the networks that
+        collected the rollout, the target networks at the start of the update.  1 gives the same returns bit for bit."""
         if optimizer not in ("torch", "cuda"):
             raise ValueError("optimizer must be 'torch' or 'cuda', got %r" % (optimizer,))
+        self.gae_lambda = check_gae_lambda(gae_lambda)
         self.env = env
         dev = torch.device("cuda", env.device)
         self.actor = (actor or ActorNetwork()).to(dev)
@@ -738,7 +782,7 @@ class BatchedMAPPORollout(object):
         # bootstrap where the last step did not end the episode (mappo.py:148-150)
         final_value = self._final_value(self.obs, v["n_agents"])
         returns = discounted_returns(R, D, final_value, self.gamma)
-        self.buf = dict(states=S, actions=A, returns=returns, live=L, dones=D, rewards=R)
+        self.buf = dict(states=S, actions=A, returns=returns, live=L, dones=D, rewards=R, final_value=final_value)
         return self.buf
 
     def _final_value(self, obs, n_agents):
@@ -817,10 +861,15 @@ class BatchedMAPPORollout(object):
         stats: also measure what the update did (the keys of `ppo_stats_keys`): a statistics pass over every live row with
         the rollout (target) networks before the first minibatch and one with the updated networks after the last, with
         `ppo_stats_torch` (impl "torch") or `ppo_stats` (impl "cuda"), all-reduced over ranks and read in one host read.
-        The passes draw no random numbers and write no parameter: the update is the same with and without them."""
+        The passes draw no random numbers and write no parameter: the update is the same with and without them.
+        With gae_lambda set, the returns G of everything above (advantage, critic target, statistics) are the
+        lambda-returns: Q_target(s_t, a_t) over every live row (one no-grad critic_target forward with impl "torch", the
+        target pass's q_target with impl "cuda") into `lambda_returns` before the first minibatch."""
         if impl == "cuda":
             return self._update_cuda(minibatch, epochs, stats)
         assert impl == "torch", impl
+        if self.gae_lambda is not None:
+            self._set_lambda_returns(self._rollout_values_torch())
         batch = self._learner_batch() if stats else None
         before = self._stats_begin("torch", batch) if stats else None
         b = self.buf
@@ -828,7 +877,7 @@ class BatchedMAPPORollout(object):
         idx = live.nonzero(as_tuple=False).squeeze(1)
         S = b["states"].reshape(-1, NS)
         A = torch.nn.functional.one_hot(b["actions"].reshape(-1), NA).float()
-        G = b["returns"].reshape(-1, 1)
+        G = self._returns().reshape(-1, 1)
         rec = {}
         n_max = torch.tensor([idx.numel()], device=self.dev)
         if self._world() > 1:
@@ -854,14 +903,40 @@ class BatchedMAPPORollout(object):
         self.critic_target.load_state_dict(self.critic.state_dict())
         return rec
 
-    def _learner_batch(self):
-        """(live row list, states [rows, 30], actions int8 [rows], returns [rows], minibatch count) of the last rollout"""
+    def _learner_batch(self, with_returns=True):
+        """(live row list, states [rows, 30], actions int8 [rows], returns [rows] or None) of the last rollout"""
         b = self.buf
         idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
         S = b["states"].reshape(-1, NS)
         A8 = b["actions"].reshape(-1).to(torch.int8)
-        G = b["returns"].reshape(-1).contiguous()
+        G = self._returns().reshape(-1).contiguous() if with_returns else None
         return idx, S, A8, G
+
+    def _returns(self):
+        """the returns the update trains on: the lambda-returns with gae_lambda set, else the discounted returns"""
+        return self.buf["returns"] if self.gae_lambda is None else self.buf["lambda_returns"]
+
+    def _set_lambda_returns(self, values):
+        """buf["lambda_returns"] from the rollout's values [rows] (zero on the rows of agents that do not exist);
+        -> the lambda-returns as [rows]"""
+        b = self.buf
+        R = b["rewards"]
+        b["lambda_returns"] = lambda_returns(R, b["dones"], values.view(R.shape), b["final_value"], self.gamma, self.gae_lambda)
+        return b["lambda_returns"].view(-1)
+
+    @torch.no_grad()
+    def _rollout_values_torch(self):
+        """the rollout's values of every live row from one no-grad forward of the target network(s), zero elsewhere:
+        [rows] f32"""
+        b = self.buf
+        idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
+        v = torch.zeros(b["live"].numel(), device=self.dev)
+        v[idx] = self._target_values(b["states"].reshape(-1, NS)[idx], b["actions"].reshape(-1)[idx])
+        return v
+
+    def _target_values(self, S, A):
+        """Q_target(s, a) of the rows S [n, 30], A [n] (MAPPO's value of the rollout) -> [n]"""
+        return self.critic_target(S, torch.nn.functional.one_hot(A, NA).float())[:, 0]
 
     def _minibatch_count(self, idx, minibatch):
         n_max = torch.tensor([idx.numel()], device=self.dev)
@@ -912,11 +987,15 @@ class BatchedMAPPORollout(object):
         the target networks do not change within an update), then per minibatch one gradient pass (mappo_gradients) in
         place of the two backward passes; then all-reduce, gradient clipping and the RMSprop steps as in the torch path
         (with optimizer="cuda" one launch steps both networks).  The losses stay on the device until the one read at the
-        end."""
-        batch = idx, S, A8, G = self._learner_batch()
+        end.  With gae_lambda the target pass's q_target (zero-filled first: it writes live rows only) is the rollout's
+        values of the lambda-returns."""
+        gae = self.gae_lambda is not None
+        batch = idx, S, A8, G = self._learner_batch(with_returns=not gae)
         n_mb = self._minibatch_count(idx, minibatch)
         old_logp = ppo_targets(self.actor_target, S, A8, idx)
-        q_target = ppo_targets(self.critic_target, S, A8, idx)
+        q_target = ppo_targets(self.critic_target, S, A8, idx, out=torch.zeros(S.shape[0], device=self.dev) if gae else None)
+        if gae:
+            batch = idx, S, A8, G = idx, S, A8, self._set_lambda_returns(q_target)
         before = self._stats_begin("cuda", batch, old_logp) if stats else None
         losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
         for _ in range(epochs):
@@ -944,6 +1023,7 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
     the three first-layer blocks as one 30 -> 160 layer); other sizes run as torch layers."""
 
     def __init__(self, env, policy=None, hidden_size=128, **kw):
+        check_gae_lambda(kw.get("gae_lambda"))     # refused before anything is built, as in the base class
         net = policy or ActorCriticNetwork(NS, NA, hidden_size, 1, state_split=True)
         kw["fused"] = bool(kw.get("fused", True)) and net.state_split and net.fc2.in_features == 160 and \
             net.fc2.out_features == 128
@@ -987,6 +1067,10 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
         net = self.policy_target if target else self.policy
         return net, net
 
+    def _target_values(self, S, A):
+        """V_target(s) of the rows S [n, 30] (the value of the rollout of MAPPO_GI) -> [n]"""
+        return self.policy_target(S, out_type="v")[:, 0]
+
     def sample_actions(self, obs, n_agents, seed, step):
         if self.fused:
             return policy_sample(self.policy, obs.contiguous(), n_agents, seed=seed, step=step)
@@ -995,17 +1079,21 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
     def update(self, minibatch=1 << 18, epochs=1, impl="torch", stats=False):
         """One pass of `MAPPO_GI.train` (shared branch, mappo_gi.py:307-349) over the last rollout, all agents at once;
         under torch.distributed the gradients are averaged over the ranks.  impl: "torch" (autograd) or "cuda" (the
-        learner kernels).  stats: as for `BatchedMAPPORollout.update`, with the shared network as policy and value."""
+        learner kernels).  stats: as for `BatchedMAPPORollout.update`, with the shared network as policy and value.
+        gae_lambda: the lambda-returns with V_target(s_t) of every live row (a no-grad policy_target forward with impl
+        "torch", the V(s) output of the shared target pass with impl "cuda")."""
         if impl == "cuda":
             return self._update_cuda(minibatch, epochs, stats)
         assert impl == "torch", impl
+        if self.gae_lambda is not None:
+            self._set_lambda_returns(self._rollout_values_torch())
         batch = self._learner_batch() if stats else None
         before = self._stats_begin("torch", batch) if stats else None
         b = self.buf
         idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
         S = b["states"].reshape(-1, NS)
         A = torch.nn.functional.one_hot(b["actions"].reshape(-1), NA).float()
-        G = b["returns"].reshape(-1, 1)
+        G = self._returns().reshape(-1, 1)
         rec = {}
         n_max = torch.tensor([idx.numel()], device=self.dev)
         if self._world() > 1:
@@ -1028,10 +1116,15 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
 
     def _update_cuda(self, minibatch, epochs, stats=False):
         """`update` with the learner kernels: one target pass, one gradient pass per minibatch
-        (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step (optimizer="cuda": one launch)."""
-        batch = idx, S, A8, G = self._learner_batch()
+        (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step (optimizer="cuda": one launch).
+        With gae_lambda the same target pass also writes V_target(s) (into a zero-filled buffer) for the lambda-returns."""
+        gae = self.gae_lambda is not None
+        batch = idx, S, A8, G = self._learner_batch(with_returns=not gae)
         n_mb = self._minibatch_count(idx, minibatch)
-        old_logp = ppo_targets(self.policy_target, S, A8, idx)
+        values = torch.zeros(S.shape[0], device=self.dev) if gae else None
+        old_logp = ppo_targets(self.policy_target, S, A8, idx, value_out=values)
+        if gae:
+            batch = idx, S, A8, G = idx, S, A8, self._set_lambda_returns(values)
         before = self._stats_begin("cuda", batch, old_logp) if stats else None
         losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
         for _ in range(epochs):

@@ -46,12 +46,14 @@ def load_ini(path):
              "eval_episodes": c.getint(T, "EVAL_EPISODES", fallback=20), "torch_seed": c.getint(M, "torch_seed", fallback=0),
              # run_mappo.py:126,232: shared_network selects MAPPO_GI with its one ActorCriticNetwork
              "shared_network": c.getboolean(M, "shared_network", fallback=False),
-             "critic_hidden_size": c.getint(M, "critic_hidden_size", fallback=128)}
+             "critic_hidden_size": c.getint(M, "critic_hidden_size", fallback=128),
+             # not a key of the reference: the GAE lambda of the returns (None: its Monte-Carlo returns), checked by train()
+             "gae_lambda": c.get(M, "gae_lambda", fallback=None)}
     return env_cfg, rollout_kw, train
 
 
 def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, minibatch=1 << 18, log=print, update_impl="torch",
-          optimizer="torch", eval_seeds=0, eval_shield=False, update_stats=False):
+          optimizer="torch", eval_seeds=0, eval_shield=False, update_stats=False, gae_lambda=None):
     """update_impl: "torch" (autograd, the default) or "cuda" (the on-device learner, `update(impl="cuda")`).
     optimizer: "torch" (clip_grad_norm_ + torch.optim.RMSprop, the default) or "cuda" (`rollout.DeviceRMSprop`: the same
     step in one launch per minibatch).
@@ -67,13 +69,16 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
     update_stats: also measure every update (`update(stats=True)`, with either update_impl) and log the keys of
     `rollout.ppo_stats_keys` with an update_ prefix: update_approx_kl, update_clip_fraction, update_ratio_min /
     update_ratio_max, update_entropy_before / _after, update_explained_variance_before / _after, update_advantage_mean and
-    update_advantage_std.  The update and every other key are the same with and without it."""
+    update_advantage_std.  The update and every other key are the same with and without it.
+    gae_lambda: a number in [0, 1] trains on GAE(lambda) returns (`BatchedMAPPORollout(gae_lambda=...)`, with either
+    update_impl); None takes MODEL_CONFIG.gae_lambda from the ini, and without that key the returns are the reference's
+    Monte-Carlo returns.  A non-number, NaN or a value outside [0, 1] is refused before anything is built."""
     if eval_shield and not eval_seeds > 0:
         raise ValueError("train: eval_shield records the shield on the eval_seeds episodes and needs eval_seeds > 0")
     import torch
     from . import evaluation as ev
     from .env import DEFAULT_CONFIG, MergeEnvBatched
-    from .rollout import BatchedMAPPOGIRollout, BatchedMAPPORollout
+    from .rollout import BatchedMAPPOGIRollout, BatchedMAPPORollout, check_gae_lambda
     import torch.distributed as dist
     from . import dist as mmd
     env_cfg, rollout_kw, tr = load_ini(config) if isinstance(config, str) else config
@@ -94,15 +99,21 @@ def train(config, n_envs=4096, iterations=30, device=0, eval_interval=10, miniba
         raise ValueError("train: update_stats must be True or False, got %r" % (update_stats,))
     if update_stats and update_impl not in ("torch", "cuda"):
         raise ValueError("train: update_stats measures the 'torch' or 'cuda' update, got update_impl %r" % (update_impl,))
+    try:
+        gae_lambda = check_gae_lambda(tr.get("gae_lambda") if gae_lambda is None else gae_lambda)
+    except ValueError as e:
+        raise ValueError("train: %s" % e) from None
     env = MergeEnvBatched(n_envs, dict(DEFAULT_CONFIG, **env_cfg), device=device)
     # rank-distinct spawn stream; its first observation goes to the rollout so that collect() does not re-spawn the
     # scenes with the (rank-independent) config seed
     obs0, _ = env.reset(seed=mmd.rank_seed(env_cfg["seed"], rank) if world > 1 else env_cfg["seed"])
     if tr.get("shared_network"):
         pol = BatchedMAPPOGIRollout(env, hidden_size=tr.get("critic_hidden_size", 128),
-                                    seed=tr["torch_seed"] + 104729 * rank, obs=obs0, optimizer=optimizer, **rollout_kw)
+                                    seed=tr["torch_seed"] + 104729 * rank, obs=obs0, optimizer=optimizer, gae_lambda=gae_lambda,
+                                    **rollout_kw)
     else:
-        pol = BatchedMAPPORollout(env, seed=tr["torch_seed"] + 104729 * rank, obs=obs0, optimizer=optimizer, **rollout_kw)
+        pol = BatchedMAPPORollout(env, seed=tr["torch_seed"] + 104729 * rank, obs=obs0, optimizer=optimizer,
+                                  gae_lambda=gae_lambda, **rollout_kw)
     pol.sync_parameters()
     if rank != 0:
         log = lambda *_: None
@@ -184,9 +195,12 @@ def main():
     ap.add_argument("--update-stats", action="store_true",
                     help="also log what each update did: KL to the rollout policy, clip fraction, ratio range, entropy, "
                          "explained variance, advantage mean / std (update_* keys)")
+    ap.add_argument("--gae-lambda", type=float, default=None,
+                    help="train on GAE(lambda) returns with this lambda in [0, 1] (default: MODEL_CONFIG.gae_lambda of the "
+                         "ini, else the Monte-Carlo returns)")
     a = ap.parse_args()
     train(a.config, a.envs, a.iterations, a.device, a.eval_interval, update_impl=a.update_impl, optimizer=a.optimizer,
-          eval_seeds=a.eval_seeds, eval_shield=a.eval_shield, update_stats=a.update_stats)
+          eval_seeds=a.eval_seeds, eval_shield=a.eval_shield, update_stats=a.update_stats, gae_lambda=a.gae_lambda)
 
 
 if __name__ == "__main__":
