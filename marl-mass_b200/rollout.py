@@ -685,10 +685,30 @@ def _check_record_slots(rows, obs_copy, live_out):
 
 
 class BatchedMAPPORollout(object):
-    def __init__(self, env, actor=None, critic=None, roll_out_n_steps=100, reward_gamma=0.99, reward_scale=20.0,
-                 reward_type="regionalR", clip_param=0.2, actor_lr=5e-4, critic_lr=5e-4, max_grad_norm=5.0, seed=0,
-                 fused=True, obs=None, reset_seed=None, optimizer="torch", gae_lambda=None):
-        """obs: the observation of an env the caller has already reset (train.py resets with a rank-distinct spawn
+    """`MAPPO` (marl/mappo.py) on every env of a `MergeEnvBatched`: an actor and a critic network (Model_common.py), their
+    target networks and one RMSprop optimiser each.  `collect`, `update` and the acting methods are written once for both
+    learners; what MAPPO_GI does differently is in the small methods `BatchedMAPPOGIRollout` overrides (`_sampler`,
+    `_learners`, `_kernel_targets`, `_kernel_gradients`, `_autograd_gradients` and the value / statistics networks)."""
+
+    def __init__(self, env, actor=None, critic=None, actor_lr=5e-4, critic_lr=5e-4, **kw):
+        """actor, critic: the networks to train (default: new ones); actor_lr, critic_lr: their RMSprop learning rates
+        (mappo.py:88-90).  Every other argument is the rollout's, see `_setup`."""
+        self._setup(env, **kw)
+        self.actor = (actor or ActorNetwork()).to(self.dev)
+        self.critic = (critic or CriticNetwork()).to(self.dev)
+        self.actor_target = ActorNetwork().to(self.dev)
+        self.critic_target = CriticNetwork().to(self.dev)
+        self.actor_target.load_state_dict(self.actor.state_dict())
+        self.critic_target.load_state_dict(self.critic.state_dict())
+        self.actor_opt = self._make_optimizer(self.actor, actor_lr)
+        self.critic_opt = self._make_optimizer(self.critic, critic_lr)
+
+    def _setup(self, env, roll_out_n_steps=100, reward_gamma=0.99, reward_scale=20.0, reward_type="regionalR",
+               clip_param=0.2, max_grad_norm=5.0, seed=0, fused=True, obs=None, reset_seed=None, optimizer="torch",
+               gae_lambda=None):
+        """What both learners share; the arguments are checked before anything touches the env or the GPU.
+
+        obs: the observation of an env the caller has already reset (train.py resets with a rank-distinct spawn
         seed and hands its first observation over).  Without it the first collect() spawns the scenes itself with
         `reset_seed` (default: derived from `seed`, which the data-parallel driver makes rank-distinct) - never with the
         env's config seed, which is the same on every rank and would make the shards replicas of one another.
@@ -701,47 +721,44 @@ class BatchedMAPPORollout(object):
             raise ValueError("optimizer must be 'torch' or 'cuda', got %r" % (optimizer,))
         self.gae_lambda = check_gae_lambda(gae_lambda)
         self.env = env
-        dev = torch.device("cuda", env.device)
-        self.actor = (actor or ActorNetwork()).to(dev)
-        self.critic = (critic or CriticNetwork()).to(dev)
-        self.actor_target = ActorNetwork().to(dev)
-        self.critic_target = CriticNetwork().to(dev)
-        self.actor_target.load_state_dict(self.actor.state_dict())
-        self.critic_target.load_state_dict(self.critic.state_dict())
+        self.dev = torch.device("cuda", env.device)
         self.T = int(roll_out_n_steps)
         self.gamma, self.reward_scale, self.reward_type = float(reward_gamma), float(reward_scale), reward_type
         self.clip_param, self.max_grad_norm = clip_param, max_grad_norm
         self.optimizer = optimizer
-        self.actor_opt = self._make_optimizer(self.actor, actor_lr)    # mappo.py:88-90
-        self.critic_opt = self._make_optimizer(self.critic, critic_lr)
-        self.dev = dev
         self.obs = obs
         self.reset_seed = (0x5EED0000 + int(seed)) if reset_seed is None else int(reset_seed)
-        E = env.n_envs
-        self._slot = torch.arange(MAXV, device=dev)[None, :]
+        self._slot = torch.arange(MAXV, device=self.dev)[None, :]
         self.buf = None
-        self.E = E
+        self.E = env.n_envs
         self.seed, self._draws = int(seed), 0
         self.fused = bool(fused)
+
+    def _sampler(self):
+        """(the network that draws the actions, its fused draw: `actor_sample` or `policy_sample`)"""
+        return self.actor, actor_sample
 
     @torch.no_grad()
     def act_fused(self, obs, n_agents):
         """The draw of `act_torch` through the fused CUDA kernel (TF32 actor + inverse-CDF sampling, one launch)."""
+        net, sample = self._sampler()
         self._draws += 1
-        a = actor_sample(self.actor, obs, n_agents, seed=self.seed, step=self._draws)
+        a = sample(net, obs, n_agents, seed=self.seed, step=self._draws)
         return a, self._slot < n_agents[:, None]
 
     @torch.no_grad()
     def _record_act(self, obs, n_agents, a_slot, s_slot, l_slot):
+        net, sample = self._sampler()
         self._draws += 1
-        return actor_sample(self.actor, obs, n_agents, seed=self.seed, step=self._draws, out_actions=a_slot, obs_copy=s_slot,
-                            live_out=l_slot)
+        return sample(net, obs, n_agents, seed=self.seed, step=self._draws, out_actions=a_slot, obs_copy=s_slot,
+                      live_out=l_slot)
 
     @torch.no_grad()
     def act_torch(self, obs, n_agents):
-        """Plain torch fp32 actor + torch.multinomial: the numerics reference of `act_fused`."""
-        logp = self.actor(obs.reshape(-1, NS))                               # [E*12, 5]
-        a = torch.multinomial(logp.exp(), 1).view(obs.shape[0], MAXV)           # exploration_action, mappo.py:225-230
+        """Plain torch fp32 policy + torch.multinomial (exploration_action, mappo.py:225-230, mappo_gi.py:368-373): the
+        numerics reference of `act_fused`."""
+        logp = self._sampler()[0](obs.reshape(-1, NS))                          # [E*12, 5]
+        a = torch.multinomial(logp.exp(), 1).view(obs.shape[0], MAXV)
         live = self._slot < n_agents[:, None]
         return torch.where(live, a, torch.ones_like(a)).to(torch.int8), live
 
@@ -854,54 +871,86 @@ class BatchedMAPPORollout(object):
             o += q.numel()
 
     def update(self, minibatch=1 << 18, epochs=1, impl="torch", stats=False):
-        """PPO-clip actor update and critic regression on the last rollout (mappo.py:161-206, `mappo_losses`), all
-        agents at once, with the per-sample surrogate (the reference's [N] x [N, 1] product is an N x N table).
-        Under torch.distributed every rank runs the same number of minibatches and the gradients are averaged.
-        impl: "torch" (autograd) or "cuda" (the learner kernels: `_update_cuda`).
+        """One PPO update on the last rollout, all agents at once, with the per-sample surrogate (the reference's [N] x
+        [N, 1] product is an N x N table): MAPPO's PPO-clip actor update and critic regression (mappo.py:161-206,
+        `mappo_losses`), or MAPPO_GI's summed loss of the shared network (mappo_gi.py:307-349, `shared_network_loss`).
+        `epochs` passes over the live rows in random minibatches (one torch.randperm per epoch, the only random draw of an
+        update), an optimiser step after each; then the target networks take the updated parameters.  Under
+        torch.distributed every rank runs the same number of minibatches and the gradients are averaged.
+        impl: "torch" (autograd) or "cuda" (the learner kernels: one target pass over every live row - the target networks
+        do not change within an update - then one gradient pass per minibatch).
+        -> {"actor_loss", "critic_loss": the last minibatch's (0 with epochs=0), "samples"}; the losses stay on the device
+        until one host read at the end.
         stats: also measure what the update did (the keys of `ppo_stats_keys`): a statistics pass over every live row with
         the rollout (target) networks before the first minibatch and one with the updated networks after the last, with
         `ppo_stats_torch` (impl "torch") or `ppo_stats` (impl "cuda"), all-reduced over ranks and read in one host read.
         The passes draw no random numbers and write no parameter: the update is the same with and without them.
         With gae_lambda set, the returns G of everything above (advantage, critic target, statistics) are the
-        lambda-returns: Q_target(s_t, a_t) over every live row (one no-grad critic_target forward with impl "torch", the
-        target pass's q_target with impl "cuda") into `lambda_returns` before the first minibatch."""
+        lambda-returns, from the rollout's values of every live row (MAPPO: Q_target(s, a), MAPPO_GI: V_target(s); one
+        no-grad target forward with impl "torch", the target pass with impl "cuda") before the first minibatch."""
+        assert impl in ("torch", "cuda"), impl
+        gae = self.gae_lambda is not None
+        batch = idx, S, A8, G = self._learner_batch(with_returns=not gae)
+        n_mb = self._minibatch_count(idx, minibatch)
+        targets = old_logp = None
         if impl == "cuda":
-            return self._update_cuda(minibatch, epochs, stats)
-        assert impl == "torch", impl
-        if self.gae_lambda is not None:
-            self._set_lambda_returns(self._rollout_values_torch())
-        batch = self._learner_batch() if stats else None
-        before = self._stats_begin("torch", batch) if stats else None
-        b = self.buf
-        live = b["live"].reshape(-1)
-        idx = live.nonzero(as_tuple=False).squeeze(1)
-        S = b["states"].reshape(-1, NS)
-        A = torch.nn.functional.one_hot(b["actions"].reshape(-1), NA).float()
-        G = self._returns().reshape(-1, 1)
-        rec = {}
-        n_max = torch.tensor([idx.numel()], device=self.dev)
-        if self._world() > 1:
-            import torch.distributed as dist
-            dist.all_reduce(n_max, op=dist.ReduceOp.MAX)
-        n_mb = max(1, -(-int(n_max) // int(minibatch)))       # same count on every rank
+            targets, values = self._kernel_targets(batch, gae)
+            old_logp = targets[0]
+        elif gae:
+            values = self._rollout_values_torch()
+        if gae:
+            batch = idx, S, A8, G = idx, S, A8, self._set_lambda_returns(values)
+        before = self._stats_begin(impl, batch, old_logp) if stats else None
+        nets, _, opts = zip(*self._learners())
+        losses = torch.zeros(2, device=self.dev)       # written by the learner kernels
+        last = losses.unbind()                        # (actor_loss, critic_loss) of the last minibatch; 0 with epochs=0
+        codes = torch.arange(NA, dtype=torch.int8, device=self.dev)
         for _ in range(epochs):
             perm = idx[torch.randperm(idx.numel(), device=self.dev)]
             for j in torch.tensor_split(perm, n_mb):
-                actor_loss, critic_loss = mappo_losses(self.actor, self.actor_target, self.critic, self.critic_target,
-                                                       S[j], A[j], G[j], self.clip_param)
-                self.actor_opt.zero_grad(set_to_none=True)
-                actor_loss.backward()
-                self._optimizer_step([self.actor_opt], [self.actor])
-                self.critic_opt.zero_grad(set_to_none=True)
-                critic_loss.backward()
-                self._optimizer_step([self.critic_opt], [self.critic])
-                rec = {"actor_loss": float(actor_loss.detach()), "critic_loss": float(critic_loss.detach()),
-                       "samples": int(idx.numel())}
+                if impl == "cuda":
+                    last = self._kernel_gradients(batch, j, targets, losses)
+                else:       # one-hot actions as (a == k): 0 / 1 exactly, in fewer launches than one_hot(...).float()
+                    last = self._autograd_gradients(S[j], (A8[j, None] == codes).float(), G[j, None])
+                self._optimizer_step(opts, nets)
+        a_loss, c_loss = torch.stack(last).tolist()
+        rec = {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
         if stats:
-            rec.update(self._stats_end("torch", batch, *before))
-        self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
-        self.critic_target.load_state_dict(self.critic.state_dict())
+            rec.update(self._stats_end(impl, batch, *before))
+        for net, target, _ in self._learners():
+            target.load_state_dict(net.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
         return rec
+
+    def _learners(self):
+        """(network, its target network, its optimiser) of every network the update trains"""
+        return [(self.actor, self.actor_target, self.actor_opt), (self.critic, self.critic_target, self.critic_opt)]
+
+    def _kernel_targets(self, batch, gae):
+        """Target pass of the CUDA update -> (the fixed arguments of `_kernel_gradients`, old_logp first; the rollout's
+        values for the lambda-returns with gae, else None).  MAPPO: old_logp and q_target; with gae q_target is
+        zero-filled first (the pass writes live rows only) and is also the values."""
+        idx, S, A8, _ = batch
+        old_logp = ppo_targets(self.actor_target, S, A8, idx)
+        q_target = ppo_targets(self.critic_target, S, A8, idx, out=torch.zeros(S.shape[0], device=self.dev) if gae else None)
+        return (old_logp, q_target), (q_target if gae else None)
+
+    def _kernel_gradients(self, batch, j, targets, losses):
+        """.grad of every trained parameter for the rows j by the learner kernels -> (actor_loss, critic_loss) device
+        scalars, views of `losses`"""
+        _, S, A8, G = batch
+        return mappo_gradients(self.actor, self.critic, S, A8, G, *targets, j, self.clip_param, losses=losses)
+
+    def _autograd_gradients(self, s, onehot, g):
+        """.grad of every trained parameter for the rows s [n, 30], one-hot actions [n, 5], returns g [n, 1] by autograd
+        -> (actor_loss, critic_loss) device scalars.  The two losses share no parameters, so the backward order does not
+        matter."""
+        actor_loss, critic_loss = mappo_losses(self.actor, self.actor_target, self.critic, self.critic_target, s, onehot, g,
+                                               self.clip_param)
+        self.actor_opt.zero_grad(set_to_none=True)
+        self.critic_opt.zero_grad(set_to_none=True)
+        actor_loss.backward()
+        critic_loss.backward()
+        return actor_loss.detach(), critic_loss.detach()
 
     def _learner_batch(self, with_returns=True):
         """(live row list, states [rows, 30], actions int8 [rows], returns [rows] or None) of the last rollout"""
@@ -939,11 +988,14 @@ class BatchedMAPPORollout(object):
         return self.critic_target(S, torch.nn.functional.one_hot(A, NA).float())[:, 0]
 
     def _minibatch_count(self, idx, minibatch):
-        n_max = torch.tensor([idx.numel()], device=self.dev)
+        """minibatches per epoch, the same on every rank (those of the largest shard); one process needs no device copy"""
+        n = idx.numel()
         if self._world() > 1:
             import torch.distributed as dist
+            n_max = torch.tensor([n], device=self.dev)
             dist.all_reduce(n_max, op=dist.ReduceOp.MAX)
-        return max(1, -(-int(n_max) // int(minibatch)))       # same count on every rank
+            n = int(n_max)
+        return max(1, -(-n // int(minibatch)))
 
     def _stat_nets(self, target):
         """(policy network, value network) of the statistics passes: the rollout's (the targets) or the updated ones"""
@@ -982,78 +1034,32 @@ class BatchedMAPPORollout(object):
         b, a = mmd.all_reduce_ppo_stats(torch.stack([before, after])).tolist()
         return ppo_stats_keys(b, a)
 
-    def _update_cuda(self, minibatch, epochs, stats=False):
-        """`update` with the learner kernels: one target pass (old log-probabilities and Q_target of every live sample,
-        the target networks do not change within an update), then per minibatch one gradient pass (mappo_gradients) in
-        place of the two backward passes; then all-reduce, gradient clipping and the RMSprop steps as in the torch path
-        (with optimizer="cuda" one launch steps both networks).  The losses stay on the device until the one read at the
-        end.  With gae_lambda the target pass's q_target (zero-filled first: it writes live rows only) is the rollout's
-        values of the lambda-returns."""
-        gae = self.gae_lambda is not None
-        batch = idx, S, A8, G = self._learner_batch(with_returns=not gae)
-        n_mb = self._minibatch_count(idx, minibatch)
-        old_logp = ppo_targets(self.actor_target, S, A8, idx)
-        q_target = ppo_targets(self.critic_target, S, A8, idx, out=torch.zeros(S.shape[0], device=self.dev) if gae else None)
-        if gae:
-            batch = idx, S, A8, G = idx, S, A8, self._set_lambda_returns(q_target)
-        before = self._stats_begin("cuda", batch, old_logp) if stats else None
-        losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
-        for _ in range(epochs):
-            perm = idx[torch.randperm(idx.numel(), device=self.dev)]
-            for j in torch.tensor_split(perm, n_mb):
-                mappo_gradients(self.actor, self.critic, S, A8, G, old_logp, q_target, j, self.clip_param, losses=losses)
-                self._optimizer_step([self.actor_opt, self.critic_opt], [self.actor, self.critic])
-        a_loss, c_loss = losses.tolist()
-        rec = {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
-        if stats:
-            rec.update(self._stats_end("cuda", batch, *before))
-        self.actor_target.load_state_dict(self.actor.state_dict())     # TARGET_TAU = 1.0 in every shipped ini
-        self.critic_target.load_state_dict(self.critic.state_dict())
-        return rec
-
 
 class BatchedMAPPOGIRollout(BatchedMAPPORollout):
     """`MAPPO_GI` with `shared_network = True` (marl/mappo_gi.py; the 6 `*-shared*.ini` configs, run_mappo.py:232-277):
     ONE ActorCriticNetwork (Model_gi.py:137-220, state_split) gives the action distribution and the state value, one
     RMSprop optimiser at `actor_lr` (mappo_gi.py:150-156) steps the summed loss (`shared_network_loss`), the bootstrap
-    value is V(final state) (mappo_gi.py:396-404).  Rollout, reward selection, scaling and returns are the base class's.
+    value is V(final state) (mappo_gi.py:396-404).  Rollout, reward selection, scaling, returns and the update loop are
+    the base class's; this class supplies the shared network to them.  It builds none of MAPPO's networks.
     As in the reference the policy is evaluated WITHOUT an action mask everywhere (`self.policy(state)`,
     mappo_gi.py:309,359): `action_masking` only changes what env.reset / step report.  With the reference's hidden size
     (128) the action draw and the bootstrap value come from the fused kernel (`policy_sample`: mm_actor_sample_mlp with
     the three first-layer blocks as one 30 -> 160 layer); other sizes run as torch layers."""
 
-    def __init__(self, env, policy=None, hidden_size=128, **kw):
-        check_gae_lambda(kw.get("gae_lambda"))     # refused before anything is built, as in the base class
+    def __init__(self, env, policy=None, hidden_size=128, actor_lr=5e-4, critic_lr=None, **kw):
+        """policy: the shared network to train (default: a new one of `hidden_size`); actor_lr: its learning rate.
+        critic_lr is accepted, as the ini files carry it, and unused: the reference's MAPPO_GI has no critic optimiser.
+        Every other argument is the rollout's, see `BatchedMAPPORollout._setup`."""
+        self._setup(env, **kw)
         net = policy or ActorCriticNetwork(NS, NA, hidden_size, 1, state_split=True)
-        kw["fused"] = bool(kw.get("fused", True)) and net.state_split and net.fc2.in_features == 160 and \
-            net.fc2.out_features == 128
-        dev = torch.device("cuda", env.device)
-        super().__init__(env, **kw)
-        self.policy = net.to(dev)
-        self.policy_target = ActorCriticNetwork(NS, NA, hidden_size, 1, state_split=self.policy.state_split).to(dev)
+        self.fused = self.fused and net.state_split and net.fc2.in_features == 160 and net.fc2.out_features == 128
+        self.policy = net.to(self.dev)
+        self.policy_target = ActorCriticNetwork(NS, NA, hidden_size, 1, state_split=self.policy.state_split).to(self.dev)
         self.policy_target.load_state_dict(self.policy.state_dict())
-        self.policy_opt = self._make_optimizer(self.policy, self.actor_opt.param_groups[0]["lr"], shared_network=self.policy)
-        self.actor = self.critic = self.actor_target = self.critic_target = None     # not part of this learner
-        self.actor_opt = self.critic_opt = None
+        self.policy_opt = self._make_optimizer(self.policy, actor_lr, shared_network=self.policy)
 
-    @torch.no_grad()
-    def act_torch(self, obs, n_agents):
-        logp = self.policy(obs.reshape(-1, NS))
-        a = torch.multinomial(logp.exp(), 1).view(obs.shape[0], MAXV)           # exploration_action, mappo_gi.py:368-373
-        live = self._slot < n_agents[:, None]
-        return torch.where(live, a, torch.ones_like(a)).to(torch.int8), live
-
-    @torch.no_grad()
-    def act_fused(self, obs, n_agents):
-        self._draws += 1
-        a = policy_sample(self.policy, obs, n_agents, seed=self.seed, step=self._draws)
-        return a, self._slot < n_agents[:, None]
-
-    @torch.no_grad()
-    def _record_act(self, obs, n_agents, a_slot, s_slot, l_slot):
-        self._draws += 1
-        return policy_sample(self.policy, obs, n_agents, seed=self.seed, step=self._draws, out_actions=a_slot, obs_copy=s_slot,
-                             live_out=l_slot)
+    def _sampler(self):
+        return self.policy, policy_sample
 
     def _final_value(self, obs, n_agents):
         if self.fused:     # V(s) from the same kernel family: critic_linear as a sixth output column
@@ -1076,65 +1082,22 @@ class BatchedMAPPOGIRollout(BatchedMAPPORollout):
             return policy_sample(self.policy, obs.contiguous(), n_agents, seed=seed, step=step)
         return self.act_torch(obs, n_agents)[0]
 
-    def update(self, minibatch=1 << 18, epochs=1, impl="torch", stats=False):
-        """One pass of `MAPPO_GI.train` (shared branch, mappo_gi.py:307-349) over the last rollout, all agents at once;
-        under torch.distributed the gradients are averaged over the ranks.  impl: "torch" (autograd) or "cuda" (the
-        learner kernels).  stats: as for `BatchedMAPPORollout.update`, with the shared network as policy and value.
-        gae_lambda: the lambda-returns with V_target(s_t) of every live row (a no-grad policy_target forward with impl
-        "torch", the V(s) output of the shared target pass with impl "cuda")."""
-        if impl == "cuda":
-            return self._update_cuda(minibatch, epochs, stats)
-        assert impl == "torch", impl
-        if self.gae_lambda is not None:
-            self._set_lambda_returns(self._rollout_values_torch())
-        batch = self._learner_batch() if stats else None
-        before = self._stats_begin("torch", batch) if stats else None
-        b = self.buf
-        idx = b["live"].reshape(-1).nonzero(as_tuple=False).squeeze(1)
-        S = b["states"].reshape(-1, NS)
-        A = torch.nn.functional.one_hot(b["actions"].reshape(-1), NA).float()
-        G = self._returns().reshape(-1, 1)
-        rec = {}
-        n_max = torch.tensor([idx.numel()], device=self.dev)
-        if self._world() > 1:
-            import torch.distributed as dist
-            dist.all_reduce(n_max, op=dist.ReduceOp.MAX)
-        n_mb = max(1, -(-int(n_max) // int(minibatch)))       # same count on every rank
-        for _ in range(epochs):
-            perm = idx[torch.randperm(idx.numel(), device=self.dev)]
-            for j in torch.tensor_split(perm, n_mb):
-                loss, a_loss, c_loss = shared_network_loss(self.policy, self.policy_target, S[j], A[j], G[j], self.clip_param)
-                self.policy_opt.zero_grad(set_to_none=True)
-                loss.backward()
-                self._optimizer_step([self.policy_opt], [self.policy])
-                rec = {"actor_loss": float(a_loss.detach()), "critic_loss": float(c_loss.detach()),
-                       "samples": int(idx.numel())}
-        if stats:
-            rec.update(self._stats_end("torch", batch, *before))
-        self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
-        return rec
+    def _learners(self):
+        return [(self.policy, self.policy_target, self.policy_opt)]
 
-    def _update_cuda(self, minibatch, epochs, stats=False):
-        """`update` with the learner kernels: one target pass, one gradient pass per minibatch
-        (shared_network_gradients), the torch path's all-reduce, clipping and RMSprop step (optimizer="cuda": one launch).
-        With gae_lambda the same target pass also writes V_target(s) (into a zero-filled buffer) for the lambda-returns."""
-        gae = self.gae_lambda is not None
-        batch = idx, S, A8, G = self._learner_batch(with_returns=not gae)
-        n_mb = self._minibatch_count(idx, minibatch)
+    def _kernel_targets(self, batch, gae):
+        """MAPPO_GI: old_logp of the shared target pass, which with gae also writes V_target(s) (into a zero-filled
+        buffer), the values"""
+        idx, S, A8, _ = batch
         values = torch.zeros(S.shape[0], device=self.dev) if gae else None
-        old_logp = ppo_targets(self.policy_target, S, A8, idx, value_out=values)
-        if gae:
-            batch = idx, S, A8, G = idx, S, A8, self._set_lambda_returns(values)
-        before = self._stats_begin("cuda", batch, old_logp) if stats else None
-        losses = torch.zeros(2, dtype=torch.float32, device=self.dev)
-        for _ in range(epochs):
-            perm = idx[torch.randperm(idx.numel(), device=self.dev)]
-            for j in torch.tensor_split(perm, n_mb):
-                shared_network_gradients(self.policy, S, A8, G, old_logp, j, self.clip_param, losses=losses)
-                self._optimizer_step([self.policy_opt], [self.policy])
-        a_loss, c_loss = losses.tolist()
-        rec = {"actor_loss": a_loss, "critic_loss": c_loss, "samples": int(idx.numel())}
-        if stats:
-            rec.update(self._stats_end("cuda", batch, *before))
-        self.policy_target.load_state_dict(self.policy.state_dict())   # TARGET_TAU = 1.0 in every shipped ini
-        return rec
+        return (ppo_targets(self.policy_target, S, A8, idx, value_out=values),), values
+
+    def _kernel_gradients(self, batch, j, targets, losses):
+        _, S, A8, G = batch
+        return shared_network_gradients(self.policy, S, A8, G, *targets, j, self.clip_param, losses=losses)[1:]
+
+    def _autograd_gradients(self, s, onehot, g):
+        loss, actor_loss, critic_loss = shared_network_loss(self.policy, self.policy_target, s, onehot, g, self.clip_param)
+        self.policy_opt.zero_grad(set_to_none=True)
+        loss.backward()
+        return actor_loss.detach(), critic_loss.detach()
